@@ -2,7 +2,7 @@
 """Headline benchmark: S4G (PN2_CLS) inference scenes/s on B200 — BASELINE.json config[1]:
 batch 64 synthetic single-view tabletop clouds at the reference's num_points (25 600) per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (the whole PN2_CLS forward: FPS, ball query, fused SA / FP / head
 MLP chains) over one batch.  `value` = scenes/s with the inputs already resident in HBM, timed with
@@ -11,6 +11,9 @@ CUDA events on the launching stream (per-step event pairs, L2 flushed between st
 the clouds, forward, device -> pinned host copy of the four prediction tensors, every step (the public call takes
 the pinned result buffers — `model(batch, host_out=...)` — so each head's copy overlaps the next head's compute).
 Weak scaling: each rank owns its own 64 scenes, no collective on the data path (SURVEY.md §8e).
+`--steps` sets the number of timed steps of the device-resident and the end-to-end loops.  `--dump-outputs DIR` writes the
+predictions of the last device-resident step (rank 0) as DIR/<name>.npy in float32: inputs and weights are seeded, so
+two builds can be compared output for output.
 
 `--impl reference` times the reference model on the box's HOST cores: the UNMODIFIED reference python modules
 (staged under baseline/_ref; the bit-identical oracle restatement when they are not staged) on the C restatement of
@@ -55,6 +58,7 @@ METRIC = "S4G scenes/sec (PN2_CLS inference, 25600 points/scene)"
 UNIT = "scenes/s"
 NUM_POINTS = 25600
 L2_FLUSH_BYTES = 256 << 20
+DUMP_BYTES = 60_000_000  # array data written by --dump-outputs: under 64 MB with the .npy headers
 
 
 def load_peaks():
@@ -87,6 +91,21 @@ def seeded_model():
 def synthetic_scenes(batch, first_seed):
     from tests.inputs import tabletop_scene
     return torch.from_numpy(np.stack([tabletop_scene(first_seed + i, NUM_POINTS) for i in range(batch)]))
+
+
+def dump_outputs(preds, out_dir, budget=DUMP_BYTES):
+    """Writes each (B, C, N) prediction tensor as out_dir/<name>.npy in float32.  When they hold more than `budget`
+    bytes, every tensor keeps the same points: a sorted sample drawn from a fixed seed, so dumps stay comparable."""
+    n = next(iter(preds.values())).shape[-1]
+    total = 4 * sum(v.numel() for v in preds.values())
+    keep = None
+    if total > budget:
+        keep = torch.from_numpy(np.sort(np.random.default_rng(0).choice(n, n * budget // total, replace=False)))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in preds.items():
+        if keep is not None:
+            v = v.index_select(-1, keep.to(v.device))
+        np.save(os.path.join(out_dir, name + ".npy"), v.detach().float().cpu().numpy())
 
 
 class ClockSampler:
@@ -247,9 +266,9 @@ def run_reference(args, rank, world):
         for i in range(args.warmup + args.steps):
             t0 = time.perf_counter()
             if model is not None:
-                model({"scene_points": scenes})
+                out = model({"scene_points": scenes})
             else:
-                model_cpu.pointnet2_forward(scenes, sd, model_cpu.PN2_CLS_CONFIG)
+                out = model_cpu.pointnet2_forward(scenes, sd, model_cpu.PN2_CLS_CONFIG)
             dt = time.perf_counter() - t0
             if i >= args.warmup:
                 times.append(dt)
@@ -269,6 +288,8 @@ def run_reference(args, rank, world):
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        dump_outputs(out, args.dump_outputs)
 
 
 TRAFFIC_FILE = "profiles/r02/ncu_launches.json"
@@ -399,7 +420,10 @@ def main():
     ap.add_argument("--no-reference-cuda", action="store_true")
     ap.add_argument("--mlp-backend", default="tcgen05", choices=["tcgen05", "tf32", "torch"])
     ap.add_argument("--no-fp-split", action="store_true", help="A/B: interpolate-then-conv at the finest propagation level")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's predictions to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -450,7 +474,7 @@ def main():
         t = StageTimer()
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
-        eng.forward(scenes, timer=t)
+        step_out = eng.forward(scenes, timer=t)
         b.record()
         timers.append(t)
         step_events.append((a, b))
@@ -493,18 +517,20 @@ def main():
     if args.mlp_backend == "tcgen05":
         out16 = {k: torch.empty(v.shape, dtype=torch.bfloat16).pin_memory() for k, v in out_host.items()}
         ts = []
-        for i in range(3 + max(args.steps // 2, 3)):
+        for i in range(args.warmup + args.steps):
             torch.cuda.synchronize()
             t0 = time.perf_counter()
             x = host_scenes.to(dev, non_blocking=True)
             with torch.no_grad():
                 net({"scene_points": x}, host_out=out16)
             torch.cuda.synchronize()
-            if i >= 3:
+            if i >= args.warmup:
                 ts.append(1e3 * (time.perf_counter() - t0))
         e2e16_local = sum(ts) / len(ts)
     time.sleep(0.05)
     clocks.__exit__(None, None, None)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(step_out, args.dump_outputs)
 
     # ---------------- reduce over ranks (max time) ----------------
     if world > 1:

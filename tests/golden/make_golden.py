@@ -72,6 +72,12 @@ def sha(t):
     return hashlib.sha256(np.ascontiguousarray(t.numpy() if torch.is_tensor(t) else t).tobytes()).hexdigest()
 
 
+def array_digest(t):
+    """SHA-256 over dtype, shape and bytes: how a fixture stores seeded weights that its test rebuilds."""
+    a = np.ascontiguousarray(t.numpy() if torch.is_tensor(t) else t)
+    return hashlib.sha256(("%s %s " % (a.dtype, a.shape)).encode() + a.tobytes()).hexdigest()
+
+
 def run_pair(PointNet2, cfg, points):
     torch.manual_seed(0)
     ref_model = seed_reference_weights(PointNet2(**cfg)).eval()

@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, HERE)
-from make_golden import import_reference, seed_reference_weights  # noqa: E402
+from make_golden import array_digest, import_reference, seed_reference_weights  # noqa: E402
 
 import_reference()
 from grasp_proposal.network_models.models.PointNet2_local import PointNet2, PointNet2Loss, PointNet2Metric  # noqa: E402
@@ -42,7 +42,9 @@ labels = {"scored_grasp_labels": torch.from_numpy(rs.randint(0, 3, (2, n_frames,
           "best_frame_t": torch.from_numpy(rs.rand(2, 3, n_frames).astype(np.float32))}
 loss = PointNet2Loss()(out_given, labels)
 metric = PointNet2Metric()(out_given, labels)
-fix.update({"sd/" + k: v.numpy() for k, v in net.state_dict().items()})
+# the model's weights as digests (keeps the file under 1 MB): tests/test_pn2_local.py rebuilds them from the same seeds
+fix["sd_keys"] = np.array(list(net.state_dict()))
+fix["sd_sha256"] = np.array([array_digest(v) for v in net.state_dict().values()])
 fix.update({"self/" + k: v.numpy() for k, v in out_self.items()})
 fix.update({"given/" + k: v.numpy() for k, v in out_given.items()})
 fix.update({"label/" + k: v.numpy() for k, v in labels.items()})

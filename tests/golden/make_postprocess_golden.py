@@ -17,6 +17,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 REF = "/root/reference/inference/grasp_proposal"
+# torch's CPU softmax rounds the last bit of some elements differently with the number of threads that share the work:
+# the golden is written, and tests/test_oracle_cpu.py checks it, with this many
+TORCH_THREADS = 8
 
 
 def cut(path, cls, names):
@@ -38,6 +41,7 @@ def cut(path, cls, names):
 
 def main():
     from oracle import model_cpu
+    torch.set_num_threads(TORCH_THREADS)
     gd = cut(os.path.join(REF, "grasp_detector.py"), "GraspDetector", {"orthogonalization", "post_processing"})
     cc = cut(os.path.join(REF, "cloud_processor", "view_collision_checker.py"), "CloudCollisionChecker", {"view_non_collision"})
     mu = cut(os.path.join(REF, "utils", "math_utils.py"), None, {"torch_batch_transformation_inv"})

@@ -146,14 +146,22 @@ def test_post_processing_invariants():
 
 def test_post_processing_pinned_to_reference_code():
     """oracle/model_cpu.py vs outputs of the reference's OWN post_processing / view_non_collision / importance
-    sampling code (cut out of /root/reference and executed by tests/golden/make_postprocess_golden.py)."""
+    sampling code (cut out of the reference project's source by tests/golden/make_postprocess_golden.py).  Torch's CPU
+    softmax rounds the last bit of some elements differently with the number of threads that share the work, so the
+    oracle runs with the thread count the golden was written with."""
     import os
+    from tests.golden.make_postprocess_golden import TORCH_THREADS
     g = np.load(os.path.join(os.path.dirname(__file__), "golden", "postprocess_ref.npz"))
     preds = {k: torch.from_numpy(g[k]) for k in ("score", "frame_R", "frame_t")}
-    for tag in ("a", "b"):
-        thr, vthr = g[f"post_{tag}/thr"]
-        poses, scores = model_cpu.post_processing(g["points"], preds, float(thr), float(vthr))
-        assert np.array_equal(poses, g[f"post_{tag}/poses"]) and np.array_equal(scores, g[f"post_{tag}/scores"])
+    threads = torch.get_num_threads()
+    torch.set_num_threads(TORCH_THREADS)
+    try:
+        for tag in ("a", "b"):
+            thr, vthr = g[f"post_{tag}/thr"]
+            poses, scores = model_cpu.post_processing(g["points"], preds, float(thr), float(vthr))
+            assert np.array_equal(poses, g[f"post_{tag}/poses"]) and np.array_equal(scores, g[f"post_{tag}/scores"])
+    finally:
+        torch.set_num_threads(threads)
     ok, _ = model_cpu.collision_filter(g["coll/poses"], g["coll/cloud"])
     assert np.array_equal(ok, np.nonzero(g["coll/ok"])[0])
     assert np.array_equal(model_cpu.importance_sampling(g["samp/scores"], g["samp/u"]), g["samp/picked"])

@@ -30,11 +30,25 @@ def _sub(gold, prefix):
     return {k[len(prefix):]: torch.from_numpy(v) for k, v in gold.items() if k.startswith(prefix)}
 
 
+def _reference_weights(gold):
+    """The reference model's seeded weights: the fixture stores their digests, the generator's seeding rebuilds them."""
+    from s4g_release_b200.network_models.models.PointNet2_local import PointNet2
+    from tests.golden.make_golden import array_digest, seed_reference_weights
+    torch.manual_seed(0)
+    net = seed_reference_weights(PointNet2(**CFG))
+    torch.nn.init.normal_(net.t_logit.weight, std=0.05)
+    sd = net.state_dict()
+    assert list(sd) == list(gold["sd_keys"])
+    for (k, v), want in zip(sd.items(), gold["sd_sha256"]):
+        assert array_digest(v) == want, k
+    return sd
+
+
 def test_module_surface_and_seeded_init(gold):
     from s4g_release_b200.network_models.models.PointNet2_local import PointNet2
     torch.manual_seed(0)
     sd = PointNet2(**CFG).state_dict()
-    ref = _sub(gold, "sd/")
+    ref = _reference_weights(gold)
     assert list(sd) == list(ref) and all(sd[k].shape == ref[k].shape for k in sd)
     # same parameter creation order => identical default init under the same seed (BN / t_logit were re-seeded later)
     for k in ("sa_modules.0.mlp.0.conv.weight", "fp_modules.3.mlp.2.conv.weight", "mlp_grasp_eval.0.conv.weight",
@@ -71,7 +85,7 @@ def test_forward_on_the_sm100a_operators(gold):
     """both branches of the grasp-evaluation head on the GPU operators, incl. the in-place update of the caller's frames"""
     from s4g_release_b200.network_models.models.PointNet2_local import PointNet2
     net = PointNet2(**CFG)
-    net.load_state_dict(_sub(gold, "sd/"), strict=True)
+    net.load_state_dict(_reference_weights(gold), strict=True)
     net = net.cuda().eval()
     pts = torch.from_numpy(gold["points"]).cuda()
     frames = torch.from_numpy(gold["frames"]).cuda()

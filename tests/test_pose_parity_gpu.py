@@ -13,7 +13,8 @@ weights are not in the checkout (tests/conditioned.py explains both):
                 stress case with real decisions (thousands of points above the 0.7 threshold).  Anything but IEEE fp32
                 moves its outputs visibly, INCLUDING THE UNMODIFIED REFERENCE: on this GPU torch runs the reference's
                 cuDNN convolutions in TF32 by default.  That deviation (reference model + reference CUDA kernels, TF32 on,
-                vs the fp32 oracle) is measured in the same test and is the yardstick: the TF32 tight-parity mode must
+                vs the fp32 oracle) is measured in the same test when the reference is staged, else read from
+                tests/golden/reference_tf32_floor.json, and is the yardstick: the TF32 tight-parity mode must
                 stay within 2x of it, the bf16 throughput path within 16x (8x coarser mantissa, 21 layers) on the mean
                 errors, and no decision may flip outside the error band of its own score.
 
@@ -47,6 +48,7 @@ BOUNDS_SEEDED = {
 # conditioned weights: bounds as multiples of the reference's own TF32 deviation (+ a small absolute floor)
 MEAN_KEYS = {"score_abs_err_mean": 1e-4, "rot_err_deg_mean": 0.05, "translation_err_mm_mean": 0.05}
 FLOOR_FACTOR = {"tf32": 2.0, "tcgen05": 16.0}
+REFERENCE_TF32_FLOOR = os.path.join(os.path.dirname(__file__), "golden", "reference_tf32_floor.json")
 
 
 @pytest.fixture(scope="module")
@@ -142,12 +144,14 @@ def test_seeded_weights_absolute_bounds(scenes, nets, oracle_out, backend):
 def test_conditioned_weights_against_the_reference_tf32_yardstick(scenes, nets, oracle_out):
     want = oracle_out["conditioned"]
     ref_tf32 = _reference_tf32_out(nets["conditioned"], scenes)
-    if ref_tf32 is None:
-        pytest.skip("baseline/_ref or oracle/_ref not staged: no reference-TF32 yardstick")
-    floor = _worst(scenes, want, ref_tf32)
-    _report("conditioned/reference_cudnn_tf32", floor)
+    if ref_tf32 is None:  # the reference is not staged: its deviation as measured when it was (same scenes and weights)
+        floor = json.load(open(REFERENCE_TF32_FLOOR))["worst"]
+    else:
+        floor = _worst(scenes, want, ref_tf32)
+        _report("conditioned/reference_cudnn_tf32", floor)
     print("conditioned reference(TF32 default)", json.dumps(floor))
-    assert floor["n_above_threshold_ref"] >= 200, "the conditioned weights must produce real candidates"
+    n_above = min(int((pose_parity.expected_score(o["score"]) > 0.7).sum()) for o in want)
+    assert n_above >= 200, "the conditioned weights must produce real candidates"
     for backend in ("tf32", "tcgen05"):
         worst = _worst(scenes, want, _gpu_out(nets["conditioned"], scenes, backend))
         _report("conditioned/" + backend, worst)
