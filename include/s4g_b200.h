@@ -263,6 +263,18 @@ int s4g_interp_concat_act_bf16(const void* sparse, const int* index, const float
 /* gather_points for xyz with int32 indices (functions.py:10-25): (B,3,N),(B,M) -> (B,3,M). */
 int s4g_gather_xyz_f32_i32(const float* xyz, const int* index, int B, int N, int M, float* out, void* stream);
 
+/* The max over the neighbours of a GLOBAL set-abstraction level (num_centroids = 0: one group of all N points centred
+ * at the origin, PointNetSAModule.forward, modules.py:93-98 + :106 torch.max(new_feature, 3)).  The fused path runs the
+ * group through the gathered max-pool chain as P partial groups; this reduces the P partial rows of each scene:
+ * in [B*P][C] bf16 -> out [B][C] bf16 (C % 8 == 0).  Exact: max ignores order and repeated rows. */
+int s4g_rows_segment_max_bf16(const void* in, int B, int P, int C, void* out, void* stream);
+
+/* Zero-neighbour feature propagation (PointnetFPModule.forward, modules.py:131-134: sparse_feature.expand + channel
+ * concat, broadcast first): sparse [B][C2] bf16, dense [B*Nq][C1] bf16 (NULL when C1 == 0) -> out [B*Nq][C2+C1] bf16.
+ * C2, C1 multiples of 8. */
+int s4g_broadcast_concat_bf16(const void* sparse, const void* dense, int B, int Nq, int C2, int C1, void* out,
+                              void* stream);
+
 /* Fused shared-MLP chain on tcgen05 tensor cores (csrc/mlp_chain.cu): replaces
  * SharedMLP / Conv1d / Conv2d (nn_utils/mlp.py:95-106, nn_utils/conv.py:30-36,70-76) with eval-mode
  * BatchNorm folded in, and around it the grouping + max-pool of PointNetSAModule.forward

@@ -153,7 +153,93 @@ gather_xyz_kernel(const float* __restrict__ xyz, const int* __restrict__ index, 
   O[2 * M + m] = __ldg(X + 2 * N + j);
 }
 
+// Global set-abstraction level (num_centroids = 0, modules.py:93-98): the gathered max-pool chain pools a scene's N
+// points as P partial groups; this kernel reduces the P partial rows of each scene.  Max is exact and ignores order and
+// repeated rows, so the result equals the one N-wide group of the reference bit for bit.  One lane per 16-byte piece
+// (8 channels) of a row; the 8 warps of a block split the rows and meet in shared memory.
+constexpr int kSegWarps = 8;
+
+__device__ __forceinline__ uint32_t max_bf16x2(uint32_t a, uint32_t b) {
+  uint32_t r;
+  asm("max.bf16x2 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b));
+  return r;
+}
+
+__device__ __forceinline__ uint4 max_bf16x8(uint4 a, uint4 b) {
+  return make_uint4(max_bf16x2(a.x, b.x), max_bf16x2(a.y, b.y), max_bf16x2(a.z, b.z), max_bf16x2(a.w, b.w));
+}
+
+__global__ void __launch_bounds__(32 * kSegWarps)
+rows_segment_max_kernel(const uint4* __restrict__ in, int P, int C8, uint4* __restrict__ out) {
+  __shared__ uint4 s_part[kSegWarps][32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int b = blockIdx.y;
+  const int c = blockIdx.x * 32 + lane;
+  const uint32_t ninf = 0xff80ff80u;  // bf16 -inf pair
+  uint4 m = make_uint4(ninf, ninf, ninf, ninf);
+  if (c < C8) {
+    const uint4* src = in + (size_t)b * P * C8 + c;
+#pragma unroll 4
+    for (int r = warp; r < P; r += kSegWarps) m = max_bf16x8(m, __ldg(src + (size_t)r * C8));
+  }
+  s_part[warp][lane] = m;
+  __syncthreads();
+  if (warp == 0 && c < C8) {
+#pragma unroll
+    for (int w = 1; w < kSegWarps; ++w) m = max_bf16x8(m, s_part[w][lane]);
+    out[(size_t)b * C8 + c] = m;
+  }
+}
+
+// Broadcast feature propagation (num_fp_neighbours = 0, modules.py:131-134): the single global feature of a scene is
+// repeated on every dense row, followed by the dense skip feature — [broadcast | skip], the reference's order.  One
+// thread per 16-byte piece of an output row.
+__global__ void __launch_bounds__(256)
+broadcast_concat_kernel(const uint4* __restrict__ sparse, const uint4* __restrict__ dense, int Nq, int C2_8, int C1_8,
+                        uint4* __restrict__ out) {
+  const int b = blockIdx.y;
+  const int w8 = C2_8 + C1_8;
+  const int n = Nq * w8;
+  uint4* O = out + (size_t)b * n;
+  for (int i = blockIdx.x * 256 + threadIdx.x; i < n; i += gridDim.x * 256) {
+    const int q = i / w8, c = i - q * w8;
+    O[i] = c < C2_8 ? __ldg(sparse + (size_t)b * C2_8 + c) : __ldg(dense + ((size_t)b * Nq + q) * C1_8 + (c - C2_8));
+  }
+}
+
 }  // namespace s4g
+
+extern "C" int s4g_rows_segment_max_bf16(const void* in, int B, int P, int C, void* out, void* stream) {
+  S4G_CHECK_ARG(in && out, "rows_segment_max: null pointer");
+  S4G_CHECK_ARG(B >= 0 && B <= 65535 && P > 0 && C > 0 && C % 8 == 0, "rows_segment_max: bad shape (C %% 8 == 0)");
+  S4G_CHECK_ARG(((uintptr_t)in & 15) == 0 && ((uintptr_t)out & 15) == 0, "rows_segment_max: rows must be 16-byte aligned");
+  if (B == 0) return S4G_OK;
+  const int C8 = C / 8;
+  const dim3 grid((unsigned)((C8 + 31) / 32), (unsigned)B);
+  s4g::rows_segment_max_kernel<<<grid, 32 * s4g::kSegWarps, 0, (cudaStream_t)stream>>>(
+      reinterpret_cast<const uint4*>(in), P, C8, reinterpret_cast<uint4*>(out));
+  S4G_LAUNCH_CHECK("rows_segment_max");
+  return S4G_OK;
+}
+
+extern "C" int s4g_broadcast_concat_bf16(const void* sparse, const void* dense, int B, int Nq, int C2, int C1, void* out,
+                                         void* stream) {
+  S4G_CHECK_ARG(sparse && out, "broadcast_concat: null pointer");
+  S4G_CHECK_ARG(C2 > 0 && C2 % 8 == 0 && C1 >= 0 && C1 % 8 == 0, "broadcast_concat: channel counts must be multiples of 8");
+  S4G_CHECK_ARG(C1 == 0 || dense != nullptr, "broadcast_concat: dense feature missing");
+  S4G_CHECK_ARG(B >= 0 && B <= 65535 && Nq > 0 && (long long)Nq * ((C2 + C1) / 8) < (1ll << 31),
+                "broadcast_concat: bad shape");
+  S4G_CHECK_ARG(((uintptr_t)sparse & 15) == 0 && ((uintptr_t)out & 15) == 0 && ((uintptr_t)dense & 15) == 0,
+                "broadcast_concat: feature rows must be 16-byte aligned");
+  if (B == 0) return S4G_OK;
+  const long long pieces = (long long)Nq * ((C2 + C1) / 8);
+  const dim3 grid((unsigned)std::min<long long>((pieces + 255) / 256, 1024), (unsigned)B);
+  s4g::broadcast_concat_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(
+      reinterpret_cast<const uint4*>(sparse), reinterpret_cast<const uint4*>(dense), Nq, C2 / 8, C1 / 8,
+      reinterpret_cast<uint4*>(out));
+  S4G_LAUNCH_CHECK("broadcast_concat");
+  return S4G_OK;
+}
 
 extern "C" int s4g_three_nn_weights_f32_i32(const float* query, const float* key, int B, int Nq, int Nk, int* index,
                                             float* weight, void* stream) {

@@ -18,12 +18,25 @@ scale/shift (reference nn_utils/conv.py:70-76 → y = relu(W'x + b')).
 import json
 import os
 
+import numpy as np
 import torch
 
 from ._lib import check, lib, ptr, stream_ptr
 from .chain import IN_GATHER, IN_ROWS, OUT_LOGITS, OUT_MAXPOOL, OUT_ROWS, MlpChain
 
 BN_EPS = 1e-5
+GLOBAL_GROUPS = (8, 16, 32, 64)  # the max-pool group sizes the chain planner accepts
+
+
+def global_group_table(n):
+    """Neighbour table of a global set-abstraction level over n points (num_centroids = 0: one group of the whole cloud,
+    pointnet2_utils/modules.py:93-98).  The gathered max-pool chain pools groups of 8 / 16 / 32 / 64 rows, so the cloud
+    is cut into P = ceil(n / g) partial groups of g rows — g the smallest such size >= n, else 64 — and the last group is
+    padded with index j % n, a real point of the same scene.  The partial maxima are reduced afterwards; max ignores
+    order and repeated rows, so the result is that of one n-wide group.  -> (g, P, int32 indices [P * g])."""
+    g = next((k for k in GLOBAL_GROUPS if k >= n), GLOBAL_GROUPS[-1])
+    p = -(-n // g)
+    return g, p, np.arange(p * g, dtype=np.int32) % n
 
 
 class StageTimer:
@@ -176,6 +189,11 @@ class FusedPointNet2:
         if self.device.type != "cuda":
             raise RuntimeError("FusedPointNet2 needs the model on a CUDA device (there is no CPU path)")
         self.mlp_backend = mlp_backend
+        # a last level with one global group (num_centroids = 0) and the broadcast propagation level it pairs with
+        # (num_fp_neighbours[0] = 0); PointNet2.fusable(allow_global=True) admits only that pairing
+        self.global_level = self.cfg["num_centroids"][-1] == 0
+        self._global_tables = {}  # (B, N) -> (g, neighbour table (B,P,g) int32, zero centroids (B,3,P))
+        self._global_chains = {}  # g -> max-pool chain of the global level
         self.sa = [_fold_mlp(m.mlp) for m in model.sa_modules]
         self.fp = [_fold_mlp(m.mlp) for m in model.fp_modules]
         heads = []
@@ -278,12 +296,15 @@ class FusedPointNet2:
 
     def _build_chains(self):
         cfg = self.cfg
-        self.sa_chains = []
+        self.sa_chains = []  # the sampled levels
         feat_c = 0
-        for i, layers in enumerate(self.sa):
+        for i, layers in enumerate(self.sa[:len(self.sa) - self.global_level]):
             self.sa_chains.append(self._make_chain([(w, b, True) for w, b in layers], IN_GATHER, feat_c, OUT_MAXPOOL,
                                                    group=cfg["num_neighbours"][i]))
             feat_c = layers[-1][0].shape[0]
+        self._global_feat_c = feat_c
+        if self.global_level and self.sa_chains:  # the global level's cloud size is the previous level's centroid count
+            self._global_chain(global_group_table(cfg["num_centroids"][-2])[0])
         # Propagation levels WITHOUT a skip feature (the finest one of PN2_CLS: 25 600 queries from 5 120 keys): the first
         # conv commutes with the interpolation — W (sum_k w_k f_k) + b = sum_k w_k (W f_k + b), the weights sum to one —
         # so it runs on the sparse rows (5x fewer), the interpolation kernel gathers the 256-wide pre-activations
@@ -291,7 +312,9 @@ class FusedPointNet2:
         self.fp_pre, self.fp_chains = [], []
         skip_c = [0] + [layers[-1][0].shape[0] for layers in self.sa]
         for i, layers in enumerate(self.fp):
-            if self.fp_linear_split and skip_c[-2 - i] == 0 and len(layers) > 1 and layers[0][0].shape[0] <= 512:
+            broadcast = i == 0 and self.global_level
+            if (self.fp_linear_split and not broadcast and skip_c[-2 - i] == 0 and len(layers) > 1
+                    and layers[0][0].shape[0] <= 512):
                 w0, b0 = layers[0]
                 self.fp_pre.append(self._make_chain([(w0, b0, False)], IN_ROWS, 0, OUT_ROWS))
                 self.fp_chains.append(self._row_chains(layers[1:]))
@@ -302,6 +325,25 @@ class FusedPointNet2:
         for k, (layers, w, b) in enumerate(self.heads):
             self.head_chains.append(self._make_chain([(lw, lb, True) for lw, lb in layers] + [(w, b, False)], IN_ROWS, 0,
                                                      OUT_LOGITS, sigmoid=(k == 3)))
+
+    def _global_chain(self, g):
+        """The global level's max-pool chain for groups of g rows (g follows the cloud size, see global_group_table)."""
+        if g not in self._global_chains:
+            self._global_chains[g] = self._make_chain([(w, b, True) for w, b in self.sa[-1]], IN_GATHER,
+                                                      self._global_feat_c, OUT_MAXPOOL, group=g)
+        return self._global_chains[g]
+
+    def _global_group(self, B, n):
+        """(g, neighbour table (B,P,g) int32, zero centroids (B,3,P) fp32) of a global level over n points; built once
+        per shape from the host, so a forward launches nothing for them.  With zero centroids the chain's relative
+        coordinates x - 0 are the absolute coordinates the reference concatenates (modules.py:97-98)."""
+        key = (B, n)
+        if key not in self._global_tables:
+            g, p, idx = global_group_table(n)
+            nbr = np.ascontiguousarray(np.broadcast_to(idx.reshape(1, p, g), (B, p, g)))
+            self._global_tables[key] = (g, torch.from_numpy(nbr).to(self.device),
+                                        torch.from_numpy(np.zeros((B, 3, p), np.float32)).to(self.device))
+        return self._global_tables[key]
 
     def tolerance(self):
         """Max abs error of the head outputs relative to max(|ref|, 1) against the fp32 oracle."""
@@ -450,6 +492,37 @@ class FusedPointNet2:
               "interp_concat")
         return out
 
+    @staticmethod
+    def rows_segment_max(rows, B):
+        """bf16 [B*P, C] -> [B, C]: the max over each scene's P rows."""
+        C = rows.shape[1]
+        out = torch.empty((B, C), dtype=torch.bfloat16, device=rows.device)
+        check(lib.s4g_rows_segment_max_bf16(ptr(rows), B, rows.shape[0] // B, C, ptr(out), stream_ptr(rows.device)),
+              "rows_segment_max")
+        return out
+
+    @staticmethod
+    def broadcast_concat(sparse, dense, B, Nq):
+        """sparse bf16 [B, C2], dense bf16 [B*Nq, C1] or None -> [B*Nq, C2 + C1] rows [sparse | dense]."""
+        C2 = sparse.shape[1]
+        C1 = dense.shape[1] if dense is not None else 0
+        out = torch.empty((B * Nq, C2 + C1), dtype=torch.bfloat16, device=sparse.device)
+        check(lib.s4g_broadcast_concat_bf16(ptr(sparse), ptr(dense) if dense is not None else None, B, Nq, C2, C1,
+                                            ptr(out), stream_ptr(sparse.device)), "broadcast_concat")
+        return out
+
+    def _side_three_nn(self, pending, early_nn, device):
+        """Issues a propagation level's 3-NN search on the side stream once ``pending``'s ready event has fired."""
+        dense_p, sparse_p, ready, fp_level = pending
+        if self._geom_stream is None:
+            self._geom_stream = torch.cuda.Stream(device=device)
+        self._geom_stream.wait_event(ready)
+        with torch.cuda.stream(self._geom_stream):
+            found = self.three_nn_weights(dense_p, sparse_p)
+            done = torch.cuda.Event()
+            done.record()
+        early_nn[fp_level] = (found, done)
+
     def _forward_tcgen05(self, points, return_trace, timer=None, host_out=None):
         cfg = self.cfg
         xyz = points.float().contiguous()
@@ -462,7 +535,7 @@ class FusedPointNet2:
         # beside the sampling of level i + 1 (submitted after it: the sampler's CTAs are placed first): 0.54 + 0.37 ms
         # alone, 0.56 ms together at 64 scenes (profiles/r01/overlap_probe.txt).  A stage timer then sees only the
         # main stream's wait in "fpK.three_nn".
-        n_sa = len(self.sa_chains)
+        n_sa = len(self.sa)  # a global level (last, no sampler) has no entry in sa_chains
         overlap = self.overlap_geometry
         main = torch.cuda.current_stream()
         pending, early_nn = None, {}
@@ -490,15 +563,7 @@ class FusedPointNet2:
                     grid_done = torch.cuda.Event()
                     grid_done.record()
             if pending is not None:
-                dense_p, sparse_p, ready, fp_level = pending
-                if self._geom_stream is None:
-                    self._geom_stream = torch.cuda.Stream(device=xyz.device)
-                self._geom_stream.wait_event(ready)
-                with torch.cuda.stream(self._geom_stream):
-                    found = self.three_nn_weights(dense_p, sparse_p)
-                    done = torch.cuda.Event()
-                    done.record()
-                early_nn[fp_level] = (found, done)
+                self._side_three_nn(pending, early_nn, xyz.device)
                 pending = None
             try:
                 with _sec(timer, "sa%d.gather_xyz" % i):
@@ -528,9 +593,30 @@ class FusedPointNet2:
             if return_trace:
                 trace["fps"].append(idx)
                 trace["ball"].append(nbr)
+        if self.global_level:
+            i = n_sa - 1
+            if pending is not None:  # the search below the last sampled level runs beside the global pool
+                self._side_three_nn(pending, early_nn, xyz.device)
+                pending = None
+            g, nbr, ctr = self._global_group(B, xyz.shape[2])
+            with _sec(timer, "sa%d.mlp" % i):
+                part = self._global_chain(g).run_gather(feat, xyz, ctr, nbr)  # [B*P, C]: one max per partial group
+            with _sec(timer, "sa%d.pool" % i):
+                feat = self.rows_segment_max(part, B)
+            xyz = ctr[:, :, :1]  # the reference's zero centroid (B,3,1)
+            lv_xyz.append(xyz)
+            lv_feat.append(feat)
         sparse_xyz, sparse = xyz, feat
         for i, chains in enumerate(self.fp_chains):
             dense_xyz, dense = lv_xyz[-2 - i], lv_feat[-2 - i]
+            if i == 0 and self.global_level:
+                with _sec(timer, "fp0.broadcast"):
+                    x = self.broadcast_concat(sparse, dense, B, dense_xyz.shape[2])
+                with _sec(timer, "fp0.mlp"):
+                    for ch in chains:
+                        x = ch.run_rows(x)
+                sparse_xyz, sparse = dense_xyz, x
+                continue
             with _sec(timer, "fp%d.three_nn" % i):
                 if i in early_nn:
                     (idx3, w), done = early_nn.pop(i)
@@ -605,6 +691,13 @@ class FusedPointNet2:
             lv_xyz, lv_feat = [xyz], [None]
             trace = {"fps": [], "ball": []}
             for i, layers in enumerate(self.sa):
+                if cfg["num_centroids"][i] == 0:  # global level: the same partial groups as the fused path
+                    g, nbr, ctr = self._global_group(xyz.shape[0], xyz.shape[2])
+                    feat = self._sa_torch(xyz, feat, ctr, nbr, layers).amax(dim=1, keepdim=True)  # (B,1,C)
+                    xyz = ctr[:, :, :1]
+                    lv_xyz.append(xyz)
+                    lv_feat.append(feat)
+                    continue
                 idx = self.fps(xyz, cfg["num_centroids"][i])
                 new_xyz = torch.gather(xyz, 2, idx.long().unsqueeze(1).expand(-1, 3, -1)).contiguous()
                 nbr = self.ball_query(xyz, new_xyz, cfg["radius"][i], cfg["num_neighbours"][i])
@@ -618,7 +711,11 @@ class FusedPointNet2:
             sparse_xyz, sparse = xyz, feat
             for i, layers in enumerate(self.fp):
                 dense_xyz, dense = lv_xyz[-2 - i], lv_feat[-2 - i]
-                sparse = self._fp_torch(dense_xyz, sparse_xyz, dense, sparse, layers)
+                if i == 0 and self.global_level:  # broadcast propagation, [global | skip] (modules.py:131-134)
+                    x = sparse.expand(-1, dense_xyz.shape[2], -1)
+                    sparse = self._mlp(x if dense is None else torch.cat([x, dense], dim=-1), layers)
+                else:
+                    sparse = self._fp_torch(dense_xyz, sparse_xyz, dense, sparse, layers)
                 sparse_xyz = dense_xyz
             outs = []
             for layers, w, b in self.heads:

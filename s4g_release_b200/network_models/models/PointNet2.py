@@ -4,7 +4,8 @@ Same encoder / decoder as PointNet2_tcls.PointNet2 (so the same sm_100a operator
 global set-abstraction level, the same fused engine); the heads differ: ``frame_R`` is a 6-D rotation representation
 turned into a matrix by ``toRotMatrix`` (functions/functions.py:179-190), ``frame_t`` is a 3-D offset ADDED to the
 input points, the score key is ``scene_score_logits``, and ``t_logit`` starts at zero (:150-152).  The reference's
-default configuration (4 levels, the last one a global group with num_centroids = 0) runs on the module path.
+default configuration (4 levels, the last one a global group with num_centroids = 0) runs on the module path unless the
+fused engine is asked for with ``fused=True``.
 """
 import torch
 import torch.nn as nn
@@ -27,10 +28,9 @@ class PointNet2(_tcls.PointNet2):
         nn.init.zeros_(self.t_logit.bias)
 
     def forward(self, data_batch, fused=None):
+        """``fused`` routes as PointNet2_tcls.PointNet2.forward (an unsupported configuration with fused=True raises)."""
         points = data_batch["scene_points"]
-        if fused is None:
-            fused = (not self.training) and (not torch.is_grad_enabled()) and points.is_cuda and self.fusable()
-        raw = self.fused_engine().forward(points) if fused else self.forward_modules(points)
+        raw = super().forward(data_batch, fused=fused)
         return {"scene_score_logits": raw["score"], "frame_R": toRotMatrix(raw["frame_R"]),
                 "frame_t": points + raw["frame_t"], "movable_logits": raw["movable_logits"]}
 

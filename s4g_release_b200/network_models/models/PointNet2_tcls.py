@@ -10,7 +10,8 @@ Two execution paths share the parameters:
   * module path (``self.training`` or autograd enabled): the nn.Module stack of pointnet2_utils.modules on
     the sm_100a ops — used for training and as the drop-in;
   * fused path (eval + no_grad on CUDA): ``engine.FusedPointNet2`` runs the whole forward with the
-    hand-written kernels (geometry in fp32, MLP chains on tcgen05 tensor cores).
+    hand-written kernels (geometry in fp32, MLP chains on tcgen05 tensor cores).  A configuration whose last level is
+    one global group (this class's default arguments) runs on it only when asked, ``forward(..., fused=True)``.
 """
 import torch
 import torch.nn as nn
@@ -114,16 +115,23 @@ class PointNet2(nn.Module):
         }
 
     # ------------------------------------------------------------------ fused (inference) path
-    def fusable(self):
+    def fusable(self, allow_global=False):
         """Whether the fused engine has a plan for this configuration (engine.py / csrc/chain_plan.cu): every level
-        samples centroids (no global num_centroids = 0 level), neighbourhoods of 8 / 16 / 32 / 64 points, 3-NN
-        propagation, hidden widths that are multiples of 16 and <= 512 inside a chain (a FP chain is cut after a
-        wider layer, so only its LAST layer may be), at most 16 logits per head.  Anything else — e.g. this class's own
-        default constructor arguments — runs on the module path, like the reference."""
+        samples centroids, neighbourhoods of 8 / 16 / 32 / 64 points, 3-NN propagation, hidden widths that are multiples
+        of 16 and <= 512 inside a chain (a FP chain is cut after a wider layer, so only its LAST layer may be), at most
+        16 logits per head.
+
+        ``allow_global=True`` also admits a LAST set-abstraction level with one global group (num_centroids = 0,
+        num_neighbours = -1) paired with a first propagation level that broadcasts its feature (num_fp_neighbours[0]
+        = 0) — e.g. this class's own default constructor arguments.  ``forward(fused=True)`` accepts those; the
+        automatic route (``fused=None``) uses the default answer and runs them on the module path, like the reference."""
         c = self.config
-        if not all(n > 0 for n in c["num_centroids"]) or not all(k in (8, 16, 32, 64) for k in c["num_neighbours"]):
+        cent, nbrs, fp_nbrs = c["num_centroids"], c["num_neighbours"], c["num_fp_neighbours"]
+        if allow_global and cent[-1] == 0 and nbrs[-1] < 0 and fp_nbrs[0] == 0:
+            cent, nbrs, fp_nbrs = cent[:-1], nbrs[:-1], fp_nbrs[1:]  # the rules below cover the remaining levels
+        if not all(n > 0 for n in cent) or not all(k in (8, 16, 32, 64) for k in nbrs):
             return False
-        if not all(k == 3 for k in c["num_fp_neighbours"]):
+        if not all(k == 3 for k in fp_nbrs):
             return False
         widths_ok = lambda chans: all(w % 16 == 0 and w >= 16 for w in chans)
         for chans in c["sa_channels"]:
@@ -192,13 +200,15 @@ class PointNet2(nn.Module):
         return clone
 
     def forward(self, data_batch, fused=None, host_out=None):
-        """``host_out`` (fused path only): dict of pinned host tensors that receive the predictions while the later
+        """``fused``: None = the fused engine in eval + no_grad on CUDA when ``fusable()``, else the module path;
+        True = the fused engine (also for a global last level, ``fusable(allow_global=True)``); False = the module path.
+        ``host_out`` (fused path only): dict of pinned host tensors that receive the predictions while the later
         heads are still computing (engine.FusedPointNet2.forward)."""
         points = data_batch["scene_points"]
         if fused is None:
             fused = (not self.training) and (not torch.is_grad_enabled()) and points.is_cuda and self.fusable()
         if fused:
-            if not self.fusable():
+            if not self.fusable(allow_global=True):
                 raise RuntimeError("the fused engine has no plan for this configuration (see PointNet2.fusable); "
                                    "call with fused=False for the module path")
             return self.fused_engine().forward(points, host_out=host_out)
