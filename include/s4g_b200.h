@@ -198,6 +198,24 @@ int s4g_train_bn_bwd_reduce_bf16(const void* dz, const uint8_t* arg, int K, cons
 int s4g_train_bn_bwd_apply_bf16(const void* dz, const uint8_t* arg, int K, const void* y, const float* scale,
                                 const float* shift, const float* ka, const float* kb, const float* kc, long long P, int C,
                                 int relu, unsigned seed, float drop_p, void* dy, void* stream);
+/* The max over a GLOBAL set-abstraction level's one group per scene (num_centroids = 0, modules.py:93-98 + the torch.max of
+ * :106): z = relu(y * scale + shift) over the N rows of each of the B scenes (y [B*N][C], any N >= 1), reduced per scene
+ * and channel: out [B][C] bf16, arg [B][C] int32 = the row inside the scene of the FIRST maximum (like torch.max), ymax
+ * (may be NULL) [B][C] bf16 = y at that row.  work: B*C 64-bit words of scratch.  The partial maxima of the CTAs are
+ * merged with 64-bit atomicMax on (value, first row) keys: the result does not depend on their order. */
+int s4g_train_bn_act_segmax_bf16(const void* y, const float* scale, const float* shift, void* out, int* arg, void* ymax,
+                                 unsigned long long* work, int B, long long N, int C, int relu, void* stream);
+/* The two BatchNorm-backward passes of such a block: the pooled gradient dz [P/N][C] routed to row arg[b][c] (int32, from
+ * s4g_train_bn_act_segmax_bf16) of scene b; otherwise as s4g_train_bn_bwd_reduce_bf16 / _apply_bf16 (no dropout). */
+int s4g_train_bn_bwd_reduce_seg_bf16(const void* dz, const int* arg, long long N, const void* y, const float* scale,
+                                     const float* shift, long long P, int C, int relu, double* sums2c, void* stream);
+int s4g_train_bn_bwd_apply_seg_bf16(const void* dz, const int* arg, long long N, const void* y, const float* scale,
+                                    const float* shift, const float* ka, const float* kb, const float* kc, long long P, int C,
+                                    int relu, void* dy, void* stream);
+/* The backward of a broadcast propagation level (num_fp_neighbours = 0, modules.py:131-134 expand) for its global input:
+ * out[b][c] += sum_n dz[b*Nq + n][c] for c < C2 (dz rows ld wide, bf16; out fp32 [B][C2]).  Fixed summation order, no
+ * atomics: the same bits on every run. */
+int s4g_train_rows_segment_sum_bf16(const void* dz, long long ld, int B, long long Nq, int C2, float* out, void* stream);
 /* QueryGrouper.forward (pointnet2_utils/modules.py:37-54) in the row layout: out row (b, m, k) =
  * [feat[b*N + nbr[b][m][k]][0..Cf) | xyz[b][:, nbr] - ctr[b][:, m] | 0 x 5]  (width Cf + 8; the weight columns are
  * re-ordered to match by the caller).  feat may be NULL when Cf == 0. */

@@ -76,7 +76,11 @@ _SIGNATURES = {
     "s4g_train_bn_act_maxpool_bf16": ([_vp, _vp, _vp, _vp, _vp, _vp, _ll, _i, _i, _i, _vp], _i),
     "s4g_train_bn_bwd_reduce_bf16": ([_vp, _vp, _i, _vp, _vp, _vp, _ll, _i, _i, ctypes.c_uint, _f, _vp, _vp], _i),
     "s4g_train_bn_bwd_apply_bf16": ([_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _i, _i, ctypes.c_uint, _f, _vp, _vp], _i),
-    "s4g_train_group_rows_bf16": ([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp], _i),
+    "s4g_train_bn_act_segmax_bf16": ([_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _ll, _i, _i, _vp], _i),
+    "s4g_train_bn_bwd_reduce_seg_bf16": ([_vp, _vp, _ll, _vp, _vp, _vp, _ll, _i, _i, _vp, _vp], _i),
+    "s4g_train_bn_bwd_apply_seg_bf16": ([_vp, _vp, _ll, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _i, _i, _vp, _vp], _i),
+    "s4g_train_rows_segment_sum_bf16": ([_vp, _ll, _i, _ll, _i, _vp, _vp], _i),
+    "s4g_train_group_rows_bf16":([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp], _i),
     "s4g_train_group_rows_bwd": ([_vp, _ll, _vp, _i, _i, _i, _i, _i, _vp, _vp], _i),
     "s4g_train_interp_rows_bwd": ([_vp, _ll, _vp, _vp, _i, _i, _i, _i, _vp, _vp], _i),
     "s4g_train_relu_mask_rows_bf16": ([_vp, _vp, _vp, _vp, _ll, _i, _vp, _vp], _i),

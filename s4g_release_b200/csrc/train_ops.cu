@@ -179,6 +179,148 @@ bn_act_maxpool_kernel(const __nv_bfloat16* __restrict__ y, const float* __restri
   reinterpret_cast<uint2*>(arg + g * C)[piece] = packed;
 }
 
+// ---------------------------------------------------------------------------------------------- global max-pool
+// bn_act followed by the max over ALL N rows of each scene: the one group of a global set-abstraction level
+// (num_centroids = 0, modules.py:93-98 + the torch.max of :106).  N is any size, so a scene's rows are split across
+// CTAs (grid = chunks x B).  Per channel the result is carried as one 64-bit key, (fp32 activation in an order-preserving
+// encoding) << 32 | ~row: the largest key is the largest activation at its FIRST row, the torch.max rule of
+// bn_act_maxpool_kernel.  A thread keeps its running maximum as (value, row), the CTA merges its threads' keys with
+// shared-memory atomicMax and the CTAs theirs with global atomicMax: a maximum does not depend on the order of the
+// merges, so the result is the same bits on every run.  bn_act_segmax_finish_kernel then decodes the keys.
+constexpr int kSegRows = 512;  // rows per CTA
+
+__device__ __forceinline__ unsigned long long seg_key(float t, unsigned row) {
+  const unsigned u = __float_as_uint(t);
+  const unsigned o = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+  return ((unsigned long long)o << 32) | (unsigned long long)(~row);
+}
+__device__ __forceinline__ float seg_key_value(unsigned long long key) {
+  const unsigned o = (unsigned)(key >> 32);
+  return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
+}
+
+__global__ void __launch_bounds__(256)
+bn_act_segmax_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict__ scale, const float* __restrict__ shift,
+                     long long N, int C, int relu, unsigned long long* __restrict__ keys) {
+  extern __shared__ unsigned long long s_key[];  // [C]
+  const int pieces = C >> 3;
+  const int lanes = 256 / pieces;
+  const int piece = threadIdx.x % pieces, rl = threadIdx.x / pieces;
+  const long long b = blockIdx.y;
+  for (int c = threadIdx.x; c < C; c += 256) s_key[c] = 0ull;  // (below every encoded activation)
+  __syncthreads();
+  if (rl < lanes) {
+    const long long r0 = (long long)blockIdx.x * kSegRows;
+    const long long r1 = min(N, r0 + kSegRows);
+    const F8 a = load_f8(scale + piece * 8), sh = load_f8(shift + piece * 8);
+    const __nv_bfloat16* src = y + b * N * C;
+    float best[8];
+    int bi[8];
+#pragma unroll
+    for (int e = 0; e < 8; ++e) { best[e] = 0.f; bi[e] = -1; }
+    for (long long r = r0 + rl; r < r1; r += 4LL * lanes) {  // four rows in flight, each thread's rows in order
+      uint4 raw[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const long long rr = r + (long long)u * lanes;
+        if (rr < r1) raw[u] = __ldg(reinterpret_cast<const uint4*>(src + rr * C) + piece);
+      }
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const long long rr = r + (long long)u * lanes;
+        if (rr >= r1) break;
+        const F8 v = unpack8(raw[u]);
+#pragma unroll
+        for (int e = 0; e < 8; ++e) {
+          float t = fmaf(v.v[e], a.v[e], sh.v[e]);
+          if (relu) t = fmaxf(t, 0.f);
+          if (bi[e] < 0 || t > best[e]) { best[e] = t; bi[e] = (int)rr; }  // first maximum wins
+        }
+      }
+    }
+#pragma unroll
+    for (int e = 0; e < 8; ++e)
+      if (bi[e] >= 0) atomicMax(&s_key[piece * 8 + e], seg_key(best[e], (unsigned)bi[e]));
+  }
+  __syncthreads();
+  for (int c = threadIdx.x; c < C; c += 256)
+    if (s_key[c]) atomicMax(keys + b * C + c, s_key[c]);
+}
+
+// keys [B][C] -> out = bf16(max activation), arg = its row inside the scene (int32), ymax = y at that row (bf16, exact)
+__global__ void __launch_bounds__(256)
+bn_act_segmax_finish_kernel(const unsigned long long* __restrict__ keys, const __nv_bfloat16* __restrict__ y, long long N,
+                            int C, long long BP, __nv_bfloat16* __restrict__ out, int* __restrict__ arg,
+                            __nv_bfloat16* __restrict__ ymax) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;  // (scene, piece)
+  if (i >= BP) return;
+  const int pieces = C >> 3;
+  const long long b = i / pieces;
+  const int piece = (int)(i - b * pieces);
+  F8 best, raw;
+  int ai[8];
+#pragma unroll
+  for (int e = 0; e < 8; ++e) {
+    const unsigned long long k = __ldg(keys + i * 8 + e);
+    best.v[e] = seg_key_value(k);
+    ai[e] = (int)~(unsigned)k;
+    if (ymax) raw.v[e] = __bfloat162float(y[(b * N + ai[e]) * C + piece * 8 + e]);
+  }
+  reinterpret_cast<uint4*>(out)[i] = pack8(best);
+  reinterpret_cast<int4*>(arg)[2 * i] = make_int4(ai[0], ai[1], ai[2], ai[3]);
+  reinterpret_cast<int4*>(arg)[2 * i + 1] = make_int4(ai[4], ai[5], ai[6], ai[7]);
+  if (ymax) reinterpret_cast<uint4*>(ymax)[i] = pack8(raw);
+}
+
+// d_global[b][c] += sum_n dz[b * Nq + n][c], c < C2 (dz rows ld wide): the gradient of a broadcast propagation level's
+// [global | skip] rows with respect to the global feature (modules.py:131-134 expand).  CTA = (group of up to 32 pieces,
+// scene); each thread sums a fixed set of rows in order, the row lanes are summed in order in shared memory: a fixed
+// reduction order, no atomics, the same bits on every run.
+constexpr int kSumPieces = 32;
+
+__global__ void __launch_bounds__(256)
+rows_segment_sum_kernel(const __nv_bfloat16* __restrict__ dz, long long ld, long long Nq, int C2, float* __restrict__ out) {
+  __shared__ float s_part[256 * 8];  // [lanes][pieces of the CTA][8]
+  const int pieces = C2 >> 3;
+  const int pg = min(pieces, kSumPieces);
+  const int lanes = 256 / pg;
+  const int pl = threadIdx.x % pg, rl = threadIdx.x / pg;
+  const int piece = blockIdx.x * pg + pl;
+  const long long b = blockIdx.y;
+  F8 acc{};
+  if (rl < lanes && piece < pieces) {
+    const __nv_bfloat16* src = dz + b * Nq * ld;
+    for (long long r = rl; r < Nq; r += 4LL * lanes) {
+      uint4 raw[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const long long rr = r + (long long)u * lanes;
+        if (rr < Nq) raw[u] = __ldg(reinterpret_cast<const uint4*>(src + rr * ld) + piece);
+      }
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        if (r + (long long)u * lanes >= Nq) break;
+        const F8 v = unpack8(raw[u]);
+#pragma unroll
+        for (int e = 0; e < 8; ++e) acc.v[e] += v.v[e];
+      }
+    }
+  }
+  if (rl < lanes) {
+    float* dst = s_part + ((size_t)rl * pg + pl) * 8;
+#pragma unroll
+    for (int e = 0; e < 8; ++e) dst[e] = acc.v[e];
+  }
+  __syncthreads();
+  for (int t = threadIdx.x; t < pg * 8; t += 256) {
+    const int c = (blockIdx.x * pg) * 8 + t;
+    if (c >= C2) break;
+    float s = 0.f;
+    for (int l = 0; l < lanes; ++l) s += s_part[(size_t)l * pg * 8 + t];
+    out[b * C2 + c] += s;
+  }
+}
+
 // ---------------------------------------------------------------------------------------------- BN backward
 // g of one piece: dense upstream gradient, or the pooled gradient routed to the arg-max row (K > 0)
 struct Upstream {
@@ -186,11 +328,12 @@ struct Upstream {
   const uint8_t* arg;        // pooled only: [G][C]
   int K;                     // 0 = dense
   int kshift;                // log2 K when K is a power of two (every shipped configuration), else -1
+  const int* arg32;          // pooled with int32 arg-max rows (the groups of a global level: K = the scene's N rows)
 };
-static Upstream make_upstream(const void* dz, const uint8_t* arg, int K) {
+static Upstream make_upstream(const void* dz, const uint8_t* arg, int K, const int* arg32 = nullptr) {
   int sh = -1;
   if (K > 0 && (K & (K - 1)) == 0) { sh = 0; while ((1 << sh) < K) ++sh; }
-  return Upstream{reinterpret_cast<const __nv_bfloat16*>(dz), arg, K, sh};
+  return Upstream{reinterpret_cast<const __nv_bfloat16*>(dz), arg, K, sh, arg32};
 }
 struct UpRaw { uint4 d; uint2 a; int k; };
 // load now (raw, 16 B + 8 B), route later: keeps the loads of several rows in flight without holding converted values
@@ -228,10 +371,42 @@ __device__ __forceinline__ F8 upstream_route(const UpRaw& r) {
   }
   return unpack8(d);
 }
+// pooled with int32 arg-max rows (bn_act_segmax): routed at load time — the 32 bytes of indices are not kept in flight —
+// so the result is a routed dense piece (k = -1) for upstream_route.  Rows < 2^31 (checked by the host): 32-bit division.
+__device__ __forceinline__ UpRaw upstream_load32(const Upstream& u, long long row, int piece, int C) {
+  UpRaw r;
+  unsigned g, k;
+  if (u.kshift >= 0) {
+    g = (unsigned)row >> u.kshift;
+    k = (unsigned)row & (unsigned)(u.K - 1);
+  } else {
+    g = (unsigned)row / (unsigned)u.K;
+    k = (unsigned)row - g * (unsigned)u.K;
+  }
+  uint4 d = __ldg(reinterpret_cast<const uint4*>(u.dz + (long long)g * C) + piece);
+  const uint4* ap = reinterpret_cast<const uint4*>(u.arg32 + (long long)g * C) + 2 * piece;
+  const uint4 a0 = __ldg(ap), a1 = __ldg(ap + 1);
+  // bf16 lane pairs: the low half of each word is the even channel
+  d.x &= (a0.x == k ? 0x0000ffffu : 0u) | (a0.y == k ? 0xffff0000u : 0u);
+  d.y &= (a0.z == k ? 0x0000ffffu : 0u) | (a0.w == k ? 0xffff0000u : 0u);
+  d.z &= (a1.x == k ? 0x0000ffffu : 0u) | (a1.y == k ? 0xffff0000u : 0u);
+  d.w &= (a1.z == k ? 0x0000ffffu : 0u) | (a1.w == k ? 0xffff0000u : 0u);
+  r.d = d;
+  r.a = make_uint2(0u, 0u);
+  r.k = -1;
+  return r;
+}
+// the upstream kinds the BatchNorm-backward kernels are compiled for
+enum { kUpDenseOrArg8 = 0, kUpArg32 = 1 };
+template <int UP>
+__device__ __forceinline__ UpRaw upstream_load_k(const Upstream& u, long long row, int piece, int C) {
+  if constexpr (UP == kUpArg32) return upstream_load32(u, row, piece, C);
+  else return upstream_load(u, row, piece, C);
+}
 
 // sums = [sum_r g | sum_r g * y]; the caller turns the second into sum g * xhat = rstd * (sum g y - mean * sum g) in fp64
 // (keeps mean / rstd out of the loop: 16 registers less, a third block per SM)
-template <int U, int MINB>  // U rows in flight per thread, MINB resident blocks per SM
+template <int U, int MINB, int UP = kUpDenseOrArg8>  // U rows in flight per thread, MINB resident blocks per SM
 __global__ void __launch_bounds__(kStatThreads, MINB)
 bn_bwd_reduce_kernel(Upstream up, const __nv_bfloat16* __restrict__ y, const float* __restrict__ scale,
                      const float* __restrict__ shift, long long P, int C, int relu, unsigned seed, unsigned thresh,
@@ -253,7 +428,7 @@ bn_bwd_reduce_kernel(Upstream up, const __nv_bfloat16* __restrict__ y, const flo
         const long long rr = r + (long long)u * lanes;
         if (rr < r1) {
           raw[u] = __ldg(reinterpret_cast<const uint4*>(y + rr * C) + piece);
-          ur[u] = upstream_load(up, rr, piece, C);
+          ur[u] = upstream_load_k<UP>(up, rr, piece, C);
         }
       }
 #pragma unroll
@@ -405,6 +580,7 @@ bn_bwd_reduce_staged_kernel(const __nv_bfloat16* __restrict__ dz, const __nv_bfl
 
 // dy = coef * (g - m1 - xhat * m2) = ka * g + kb * y + kc per channel, with ka = coef, kb = -coef * rstd * m2,
 // kc = coef * (rstd * m2 * mean - m1) folded by the host wrapper (coef = gamma * rstd, m1 = mean(g), m2 = mean(g * xhat))
+template <int UP = kUpDenseOrArg8>
 __global__ void __launch_bounds__(256, 2)
 bn_bwd_apply_kernel(Upstream up, const __nv_bfloat16* __restrict__ y, const float* __restrict__ scale,
                     const float* __restrict__ shift, const float* __restrict__ ka, const float* __restrict__ kb,
@@ -425,7 +601,7 @@ bn_bwd_apply_kernel(Upstream up, const __nv_bfloat16* __restrict__ y, const floa
       const long long rr = r + (long long)u * lanes;
       if (rr < r1) {
         raw[u] = __ldg(reinterpret_cast<const uint4*>(y + rr * C) + piece);
-        ur[u] = upstream_load(up, rr, piece, C);
+        ur[u] = upstream_load_k<UP>(up, rr, piece, C);
       }
     }
 #pragma unroll
@@ -453,7 +629,7 @@ bn_bwd_apply_kernel(Upstream up, const __nv_bfloat16* __restrict__ y, const floa
 // threads get 128 registers each; with 16 + 1 warps ptxas allots 96 and the five per-channel parameter vectors spill)
 // DENSE / DROP are compile-time: the pooled pass (G x K rows, no dropout) carries neither the dropout hash nor the dense
 // branch, the dense pass not the routing
-template <int RPL, int STAGES, int CONS, bool DENSE, bool DROP>
+template <int RPL, int STAGES, int CONS, bool DENSE, bool DROP, int UP = kUpDenseOrArg8>
 __global__ void __launch_bounds__(CONS + 32, 1)
 bn_bwd_apply_staged_kernel(Upstream up, const __nv_bfloat16* __restrict__ y, const float* __restrict__ scale,
                            const float* __restrict__ shift, const float* __restrict__ ka, const float* __restrict__ kb,
@@ -509,7 +685,7 @@ bn_bwd_apply_staged_kernel(Upstream up, const __nv_bfloat16* __restrict__ y, con
     if (active && !dense) {  // (before the wait: these come from L2)
 #pragma unroll
       for (int u = 0; u < RPL; ++u)
-        if (rl + u * lanes < rows) ur[u] = upstream_load(up, row0 + rl + u * lanes, piece, C);
+        if (rl + u * lanes < rows) ur[u] = upstream_load_k<UP>(up, row0 + rl + u * lanes, piece, C);
     }
     stg_wait(&full[s], use & 1u);
     if (active) {
@@ -989,25 +1165,25 @@ extern "C" int s4g_train_bn_act_maxpool_bf16(const void* y, const float* scale, 
   return S4G_OK;
 }
 
-// upstream gradient: dz [P][C] when K == 0; pooled dz [P/K][C] + arg-max [P/K][C] when K > 0
-extern "C" int s4g_train_bn_bwd_reduce_bf16(const void* dz, const uint8_t* arg, int K, const void* y, const float* scale,
-                                            const float* shift, long long P, int C, int relu, unsigned seed, float drop_p,
-                                            double* sums2c, void* stream) {
-  S4G_CHECK_ARG(dz && y && scale && shift && sums2c && P > 0 && (K == 0 || (arg && P % K == 0)),
-                "train_bn_bwd_reduce: bad arguments");
-  TRN_CHECK_C(C);
+// upstream gradient: dz [P][C] when K == 0; pooled dz [P/K][C] + arg-max [P/K][C] when K > 0 (uint8 arg, or int32 arg32)
+static int bn_bwd_reduce(const Upstream& up, const void* y, const float* scale, const float* shift, long long P, int C,
+                         int relu, unsigned seed, float drop_p, double* sums2c, void* stream) {
   cudaStream_t s = (cudaStream_t)stream;
   S4G_CUDA(cudaMemsetAsync(sums2c, 0, sizeof(double) * 2 * C, s));
   const int pieces = C >> 3, lanes = kStatThreads / pieces;
   S4G_CHECK_ARG(lanes >= 1, "train_bn_bwd_reduce: too many channels");
   const unsigned thresh = drop_p > 0.f ? (unsigned)((double)drop_p * 4294967296.0) : 0u;
-  const Upstream up = make_upstream(dz, arg, K);
+  const void* dz = up.dz;
+  const int K = up.K;
   // S4G_BWD_REDUCE_VARIANT (A/B measurements): 0 (default) = rows staged by the copy engine for dense upstream gradients,
   // 1 = registers, 2 rows in flight x 3 blocks per SM, 2 = registers, 4 x 2
   static int variant = -1;
   if (variant < 0) { const char* e = getenv("S4G_BWD_REDUCE_VARIANT"); variant = e ? atoi(e) : 0; }
   const size_t sm = (size_t)lanes * pieces * 16 * sizeof(float);
-  if (variant == 0 && K == 0 && C <= 2048 && (((uintptr_t)dz | (uintptr_t)y) & 15) == 0) {
+  if (up.arg32) {
+    bn_bwd_reduce_kernel<4, 2, kUpArg32><<<grid_for(P, kStatRows), kStatThreads, sm, s>>>(
+        up, reinterpret_cast<const bf16*>(y), scale, shift, P, C, relu, seed, thresh, 1.f / (1.f - drop_p), sums2c);
+  } else if (variant == 0 && K == 0 && C <= 2048 && (((uintptr_t)dz | (uintptr_t)y) & 15) == 0) {
     const int lanes_s = kStgConsumers / pieces;
     const int R = kStgRowsPerLane * lanes_s;
     const size_t tile_bytes = (size_t)R * C * 2;
@@ -1032,17 +1208,32 @@ extern "C" int s4g_train_bn_bwd_reduce_bf16(const void* dz, const uint8_t* arg, 
   return S4G_OK;
 }
 
-extern "C" int s4g_train_bn_bwd_apply_bf16(const void* dz, const uint8_t* arg, int K, const void* y, const float* scale,
-                                           const float* shift, const float* ka, const float* kb, const float* kc,
-                                           long long P, int C, int relu, unsigned seed, float drop_p, void* dy, void* stream) {
-  S4G_CHECK_ARG(dz && y && scale && shift && ka && kb && kc && dy && P > 0 && (K == 0 || (arg && P % K == 0)),
-                "train_bn_bwd_apply: bad arguments");
+extern "C" int s4g_train_bn_bwd_reduce_bf16(const void* dz, const uint8_t* arg, int K, const void* y, const float* scale,
+                                            const float* shift, long long P, int C, int relu, unsigned seed, float drop_p,
+                                            double* sums2c, void* stream) {
+  S4G_CHECK_ARG(dz && y && scale && shift && sums2c && P > 0 && (K == 0 || (arg && P % K == 0)),
+                "train_bn_bwd_reduce: bad arguments");
   TRN_CHECK_C(C);
+  return bn_bwd_reduce(make_upstream(dz, arg, K), y, scale, shift, P, C, relu, seed, drop_p, sums2c, stream);
+}
+
+extern "C" int s4g_train_bn_bwd_reduce_seg_bf16(const void* dz, const int* arg, long long N, const void* y, const float* scale,
+                                                const float* shift, long long P, int C, int relu, double* sums2c,
+                                                void* stream) {
+  S4G_CHECK_ARG(dz && arg && y && scale && shift && sums2c && N > 0 && P > 0 && P % N == 0 && P < (1ll << 31),
+                "train_bn_bwd_reduce_seg: bad arguments");
+  TRN_CHECK_C(C);
+  return bn_bwd_reduce(make_upstream(dz, nullptr, (int)N, arg), y, scale, shift, P, C, relu, 0u, 0.f, sums2c, stream);
+}
+
+static int bn_bwd_apply(const Upstream& up, const void* y, const float* scale, const float* shift, const float* ka,
+                        const float* kb, const float* kc, long long P, int C, int relu, unsigned seed, float drop_p, void* dy,
+                        void* stream) {
   const unsigned thresh = drop_p > 0.f ? (unsigned)((double)drop_p * 4294967296.0) : 0u;
-  const Upstream up = make_upstream(dz, arg, K);
+  const int K = up.K;
   static int variant = -1;  // S4G_BWD_APPLY_VARIANT (A/B measurements): 0 (default) = rows staged by the copy engine, 1 = registers
   if (variant < 0) { const char* e = getenv("S4G_BWD_APPLY_VARIANT"); variant = e ? atoi(e) : 0; }
-  if (variant == 0 && (((uintptr_t)dz | (uintptr_t)y | (uintptr_t)dy) & 15) == 0) {
+  if (variant == 0 && (((uintptr_t)up.dz | (uintptr_t)y | (uintptr_t)dy) & 15) == 0) {
     constexpr int kRpl = 4, kStages = 3, kCons = 480;
     const int pieces = C >> 3, lanes_s = kCons / pieces;
     const int R = kRpl * lanes_s;
@@ -1053,24 +1244,79 @@ extern "C" int s4g_train_bn_bwd_apply_bf16(const void* dz, const uint8_t* arg, i
       S4G_CUDA(cudaFuncSetAttribute(bn_bwd_apply_staged_kernel<kRpl, kStages, kCons, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
       S4G_CUDA(cudaFuncSetAttribute(bn_bwd_apply_staged_kernel<kRpl, kStages, kCons, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
       S4G_CUDA(cudaFuncSetAttribute(bn_bwd_apply_staged_kernel<kRpl, kStages, kCons, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+      S4G_CUDA(cudaFuncSetAttribute(bn_bwd_apply_staged_kernel<kRpl, kStages, kCons, false, false, kUpArg32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     }
     const long long n_tiles = (P + R - 1) / R;
     const int sms = s4g::num_sms();
     const unsigned grid = (unsigned)(n_tiles < sms ? n_tiles : sms);
     cudaStream_t st = (cudaStream_t)stream;
     const float ks = 1.f / (1.f - drop_p);
-#define S4G_APPLY_GO(DENSE_, DROP_)                                                                                        \
-  bn_bwd_apply_staged_kernel<kRpl, kStages, kCons, DENSE_, DROP_><<<grid, kCons + 32, smem, st>>>(                          \
+#define S4G_APPLY_GO(DENSE_, DROP_, ...)                                                                                   \
+  bn_bwd_apply_staged_kernel<kRpl, kStages, kCons, DENSE_, DROP_, ##__VA_ARGS__><<<grid, kCons + 32, smem, st>>>(           \
       up, reinterpret_cast<const bf16*>(y), scale, shift, ka, kb, kc, P, C, relu, seed, thresh, ks, reinterpret_cast<bf16*>(dy))
-    if (K == 0) { if (thresh) S4G_APPLY_GO(true, true); else S4G_APPLY_GO(true, false); }
+    if (up.arg32) S4G_APPLY_GO(false, false, kUpArg32);  // (a pooled block has no dropout)
+    else if (K == 0) { if (thresh) S4G_APPLY_GO(true, true); else S4G_APPLY_GO(true, false); }
     else { if (thresh) S4G_APPLY_GO(false, true); else S4G_APPLY_GO(false, false); }
 #undef S4G_APPLY_GO
+  } else if (up.arg32) {
+    bn_bwd_apply_kernel<kUpArg32><<<grid_for(P, kEltRows), 256, 0, (cudaStream_t)stream>>>(
+        up, reinterpret_cast<const bf16*>(y), scale, shift, ka, kb, kc, P, C, relu, seed, thresh, 1.f / (1.f - drop_p),
+        reinterpret_cast<bf16*>(dy));
   } else {
-    bn_bwd_apply_kernel<<<grid_for(P, kEltRows), 256, 0, (cudaStream_t)stream>>>(
+    bn_bwd_apply_kernel<><<<grid_for(P, kEltRows), 256, 0, (cudaStream_t)stream>>>(
         up, reinterpret_cast<const bf16*>(y), scale, shift, ka, kb, kc, P, C, relu, seed, thresh, 1.f / (1.f - drop_p),
         reinterpret_cast<bf16*>(dy));
   }
   S4G_LAUNCH_CHECK("train_bn_bwd_apply");
+  return S4G_OK;
+}
+
+extern "C" int s4g_train_bn_bwd_apply_bf16(const void* dz, const uint8_t* arg, int K, const void* y, const float* scale,
+                                           const float* shift, const float* ka, const float* kb, const float* kc,
+                                           long long P, int C, int relu, unsigned seed, float drop_p, void* dy, void* stream) {
+  S4G_CHECK_ARG(dz && y && scale && shift && ka && kb && kc && dy && P > 0 && (K == 0 || (arg && P % K == 0)),
+                "train_bn_bwd_apply: bad arguments");
+  TRN_CHECK_C(C);
+  return bn_bwd_apply(make_upstream(dz, arg, K), y, scale, shift, ka, kb, kc, P, C, relu, seed, drop_p, dy, stream);
+}
+
+extern "C" int s4g_train_bn_bwd_apply_seg_bf16(const void* dz, const int* arg, long long N, const void* y, const float* scale,
+                                               const float* shift, const float* ka, const float* kb, const float* kc,
+                                               long long P, int C, int relu, void* dy, void* stream) {
+  S4G_CHECK_ARG(dz && arg && y && scale && shift && ka && kb && kc && dy && N > 0 && P > 0 && P % N == 0 && P < (1ll << 31),
+                "train_bn_bwd_apply_seg: bad arguments");
+  TRN_CHECK_C(C);
+  return bn_bwd_apply(make_upstream(dz, nullptr, (int)N, arg), y, scale, shift, ka, kb, kc, P, C, relu, 0u, 0.f, dy, stream);
+}
+
+extern "C" int s4g_train_bn_act_segmax_bf16(const void* y, const float* scale, const float* shift, void* out, int* arg,
+                                            void* ymax, unsigned long long* work, int B, long long N, int C, int relu,
+                                            void* stream) {
+  S4G_CHECK_ARG(y && scale && shift && out && arg && work && B > 0 && B <= 65535 && N > 0 && N < (1ll << 31),
+                "train_bn_act_segmax: bad arguments");
+  TRN_CHECK_C(C);
+  cudaStream_t s = (cudaStream_t)stream;
+  S4G_CUDA(cudaMemsetAsync(work, 0, sizeof(unsigned long long) * (size_t)B * C, s));
+  const dim3 grid((unsigned)((N + kSegRows - 1) / kSegRows), (unsigned)B);
+  bn_act_segmax_kernel<<<grid, 256, sizeof(unsigned long long) * (size_t)C, s>>>(reinterpret_cast<const bf16*>(y), scale,
+                                                                                 shift, N, C, relu, work);
+  S4G_LAUNCH_CHECK("train_bn_act_segmax");
+  const long long bp = (long long)B * (C >> 3);
+  bn_act_segmax_finish_kernel<<<grid_for(bp, 256), 256, 0, s>>>(work, reinterpret_cast<const bf16*>(y), N, C, bp,
+                                                                reinterpret_cast<bf16*>(out), arg, reinterpret_cast<bf16*>(ymax));
+  S4G_LAUNCH_CHECK("train_bn_act_segmax_finish");
+  return S4G_OK;
+}
+
+extern "C" int s4g_train_rows_segment_sum_bf16(const void* dz, long long ld, int B, long long Nq, int C2, float* out,
+                                               void* stream) {
+  S4G_CHECK_ARG(dz && out && B > 0 && B <= 65535 && Nq > 0 && C2 > 0 && C2 % 8 == 0 && ld >= C2 && ld % 8 == 0,
+                "train_rows_segment_sum: bad arguments");
+  const int pieces = C2 >> 3;
+  const int pg = pieces < kSumPieces ? pieces : kSumPieces;
+  const dim3 grid((unsigned)((pieces + pg - 1) / pg), (unsigned)B);
+  rows_segment_sum_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const bf16*>(dz), ld, Nq, C2, out);
+  S4G_LAUNCH_CHECK("train_rows_segment_sum");
   return S4G_OK;
 }
 

@@ -29,8 +29,10 @@ class PointNet2(_tcls.PointNet2):
 
     def forward(self, data_batch, fused=None):
         """``fused`` routes as PointNet2_tcls.PointNet2.forward (an unsupported configuration with fused=True raises)."""
-        points = data_batch["scene_points"]
-        raw = super().forward(data_batch, fused=fused)
+        return self.predictions(super().forward(data_batch, fused=fused), data_batch["scene_points"])
+
+    def predictions(self, raw, points):
+        """raw head outputs -> this model's predictions (PointNet2.py:140-148); shared with train_engine.TrainEngine"""
         return {"scene_score_logits": raw["score"], "frame_R": toRotMatrix(raw["frame_R"]),
                 "frame_t": points + raw["frame_t"], "movable_logits": raw["movable_logits"]}
 

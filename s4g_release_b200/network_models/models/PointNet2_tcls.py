@@ -217,6 +217,12 @@ class PointNet2(nn.Module):
     def init_weights(self):
         pass
 
+    def predictions(self, raw, points):
+        """The prediction dict from the raw head outputs {score, frame_R, frame_t, movable_logits (after the sigmoid)}
+        of the trunk + heads (module path, fused engine, training engine).  PN2_CLS emits them as they are; the PN2
+        sibling maps them (models/PointNet2.py)."""
+        return raw
+
 
 class PointNet2Loss(nn.Module):
     """Reference PointNet2_tcls.py:156-219: weighted CE on the score classes (class 0 down-weighted),

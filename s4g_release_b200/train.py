@@ -49,9 +49,11 @@ def broadcast_parameters(module, src=0, group=None):
             dist.broadcast(t.data, src=src, group=group)
 
 
-def synthetic_labels(batch, num_points, num_frame=4000, first_seed=2000, device="cpu"):
+def synthetic_labels(batch, num_points, num_frame=4000, first_seed=2000, device="cpu", continuous_t=False):
     """SURVEY.md §8d config 4: score labels {0,1,2}, movable {0,1}, random rotations (row-major 9),
-    approach-offset class {0..3}, scene_score U[0,1]; M' = 4000 frame points as the reference's smoke block."""
+    approach-offset class {0..3}, scene_score U[0,1]; M' = 4000 frame points as the reference's smoke block.
+    ``continuous_t``: best_frame_t is a float32 (3, M') position in U[0,1)^3 instead of the class index — the label of
+    the PN2 sibling's translation head (models/PointNet2.py: frame_t = points + offset)."""
     out = {k: [] for k in ("scene_score_labels", "scene_movable_labels", "best_frame_R", "best_frame_t", "scene_score")}
     for i in range(batch):
         rs = np.random.RandomState(first_seed + i)
@@ -59,7 +61,8 @@ def synthetic_labels(batch, num_points, num_frame=4000, first_seed=2000, device=
         out["scene_movable_labels"].append(rs.randint(0, 2, size=(5, num_points)).astype(np.float32))
         q, _ = np.linalg.qr(rs.randn(num_frame, 3, 3))
         out["best_frame_R"].append(q.reshape(num_frame, 9).T.astype(np.float32))
-        out["best_frame_t"].append(rs.randint(0, 4, size=num_frame))
+        out["best_frame_t"].append(rs.rand(3, num_frame).astype(np.float32) if continuous_t else
+                                   rs.randint(0, 4, size=num_frame))
         out["scene_score"].append(rs.rand(num_points).astype(np.float32))
     return {k: torch.from_numpy(np.stack(v)).to(device) for k, v in out.items()}
 
@@ -68,7 +71,8 @@ class Trainer:
     def __init__(self, model, loss_fn, lr=1e-3, betas=(0.9, 0.999), weight_decay=0.0, step_size=20, gamma=0.5,
                  group=None, fused=False):
         """``fused``: forward + loss + backward on the B200-native training kernels (train_engine.TrainEngine: tcgen05
-        GEMMs over bf16 rows, fused BatchNorm / ReLU / max-pool passes) instead of the module path under torch autograd."""
+        GEMMs over bf16 rows, fused BatchNorm / ReLU / max-pool passes) instead of the module path under torch autograd —
+        PN2_CLS or the PN2 sibling with its own PointNet2Loss, including a global last level (TrainEngine's guard)."""
         self.model, self.loss_fn, self.group = model, loss_fn, group
         self.engine = None
         if fused:

@@ -126,15 +126,17 @@ class Block:
         wb[:, self.cf:self.cf + 3] = w[:, :3]
         return wb
 
-    def forward(self, x, pool_k=0, seed=0):
-        """x [P, Kp] bf16 -> z [P, cout] bf16, or (pooled [P / pool_k, cout], arg) when pool_k > 0."""
+    def forward(self, x, pool_k=0, seed=0, global_pool=False):
+        """x [P, Kp] bf16 -> z [P, cout] bf16, or (pooled [P / pool_k, cout], arg) when pool_k > 0.
+        ``global_pool``: pool_k is the N rows of a scene (a global set-abstraction level, any N): the max runs on
+        s4g_train_bn_act_segmax_bf16 and arg is int32 (the row inside the scene)."""
         wb = self._weight_rows()
         if FUSED_STATS:
             y, sums = gemm(x, wb, stats=True)  # conv + the BatchNorm batch statistics of its (stored) output
         else:
             y = gemm(x, wb)
             sums = colstats_raw(y)
-        return self._normalise(x, y, sums, wb, pool_k, seed)
+        return self._normalise(x, y, sums, wb, pool_k, seed, global_pool)
 
     def forward_pre(self, y, x_rows, wb):
         """the block from its PRE-activations y [P, cout] bf16 (computed elsewhere: FP_LINEAR_SPLIT); x_rows / wb = the rows
@@ -143,7 +145,7 @@ class Block:
         self.saved = self.saved + (True,)
         return z
 
-    def _normalise(self, x, y, sums, wb, pool_k, seed):
+    def _normalise(self, x, y, sums, wb, pool_k, seed, global_pool=False):
         bn = self.bn
         P = y.shape[0]
         dev = y.device
@@ -158,7 +160,16 @@ class Block:
         if track:
             bn.num_batches_tracked += 1
         mean_rstd, scale, shift = stat[:2 * C], stat[2 * C:3 * C], stat[3 * C:]
-        if pool_k:
+        if global_pool:
+            G = P // pool_k
+            z = torch.empty((G, self.cout), dtype=BF16, device=dev)
+            arg = torch.empty((G, self.cout), dtype=torch.int32, device=dev)
+            ymax = torch.empty((G, self.cout), dtype=BF16, device=dev) if SPARSE_POOL_REDUCE else None
+            work = torch.empty((G, self.cout), dtype=torch.int64, device=dev)
+            check(lib.s4g_train_bn_act_segmax_bf16(ptr(y), ptr(scale), ptr(shift), ptr(z), ptr(arg),
+                                                   ptr(ymax) if ymax is not None else None, ptr(work), G, pool_k,
+                                                   self.cout, 1, stream_ptr(dev)), "train_bn_act_segmax")
+        elif pool_k:
             G = P // pool_k
             z = torch.empty((G, self.cout), dtype=BF16, device=dev)
             arg = torch.empty((G, self.cout), dtype=torch.uint8, device=dev)
@@ -198,6 +209,9 @@ class Block:
                 dz, relu = dzm, 0
                 check(lib.s4g_train_bn_bwd_reduce_bf16(ptr(dz), None, 0, ptr(ymax), ptr(scale), ptr(shift), P // pool_k, C, 0,
                                                        seed, 0.0, ptr(sums), stream_ptr(dev)), "train_bn_bwd_reduce")
+            elif arg is not None and arg.dtype == torch.int32:  # global pool: dz routed to row arg of its scene
+                check(lib.s4g_train_bn_bwd_reduce_seg_bf16(ptr(dz), ptr(arg), pool_k, ptr(y), ptr(scale), ptr(shift), P, C,
+                                                           1, ptr(sums), stream_ptr(dev)), "train_bn_bwd_reduce_seg")
             else:
                 check(lib.s4g_train_bn_bwd_reduce_bf16(ptr(dz), ptr(arg) if pool_k else None, pool_k, ptr(y), ptr(scale),
                                                        ptr(shift), P, C, 1, seed, drop, ptr(sums), stream_ptr(dev)),
@@ -208,9 +222,14 @@ class Block:
         check(lib.s4g_train_bn_bwd_finalize(ptr(sums), P, C, ptr(self.bn.weight), ptr(mean_rstd), ptr(gw), ptr(gb), ptr(coef),
                                             stream_ptr(dev)), "train_bn_bwd_finalize")
         dy = torch.empty((P, C), dtype=BF16, device=dev)
-        check(lib.s4g_train_bn_bwd_apply_bf16(ptr(dz), ptr(arg) if pool_k else None, pool_k, ptr(y), ptr(scale), ptr(shift),
-                                              ptr(coef), ptr(coef[C:]), ptr(coef[2 * C:]), P, C, relu, seed, drop, ptr(dy),
-                                              stream_ptr(dev)), "train_bn_bwd_apply")
+        if arg is not None and arg.dtype == torch.int32:
+            check(lib.s4g_train_bn_bwd_apply_seg_bf16(ptr(dz), ptr(arg), pool_k, ptr(y), ptr(scale), ptr(shift), ptr(coef),
+                                                      ptr(coef[C:]), ptr(coef[2 * C:]), P, C, relu, ptr(dy), stream_ptr(dev)),
+                  "train_bn_bwd_apply_seg")
+        else:
+            check(lib.s4g_train_bn_bwd_apply_bf16(ptr(dz), ptr(arg) if pool_k else None, pool_k, ptr(y), ptr(scale),
+                                                  ptr(shift), ptr(coef), ptr(coef[C:]), ptr(coef[2 * C:]), P, C, relu, seed,
+                                                  drop, ptr(dy), stream_ptr(dev)), "train_bn_bwd_apply")
         if split:
             return dy, x, wb  # the caller owns the conv (it ran on other rows)
         # dW = dY^T X: a plain library GEMM (bf16 operands, fp32 result)
@@ -298,6 +317,12 @@ def group_rows_backward(dz, nbr, B, N, M, K, cf, dfeat):
                                         ptr(dfeat), None, stream_ptr(dev)), "train_rows_bwd_gather")
 
 
+def rows_segment_sum(dz, B, Nq, c2, out):
+    """out [B, c2] fp32 += the sum over each scene's Nq rows of dz's first c2 columns (bf16 [B*Nq, >= c2]); fixed order"""
+    check(lib.s4g_train_rows_segment_sum_bf16(ptr(dz), dz.stride(0), B, Nq, c2, ptr(out), stream_ptr(dz.device)),
+          "train_rows_segment_sum")
+
+
 def _grad_buffer(param):
     """param.grad as a contiguous fp32 tensor the kernels can add into (created as zeros when absent)"""
     if param.grad is None:
@@ -314,15 +339,29 @@ def _accumulate(param, grad):
         param.grad.add_(grad.reshape(param.shape))
 
 
+def _has_training_plan(model):
+    """PointNet2.fusable(), or for a configuration whose last level is one global group fusable(allow_global=True) —
+    as long as a sampled level comes first: a global FIRST level has no input features, and the module path cannot run
+    it either (PointNetSAModule.forward unsqueezes the absent feature)."""
+    cfg = getattr(model, "config", None)
+    if cfg is None or cfg["num_centroids"][-1] != 0:
+        return model.fusable()
+    return len(cfg["num_centroids"]) > 1 and model.fusable(allow_global=True)
+
+
 class TrainEngine:
-    """forward + loss + backward of PN2_CLS on the fused training kernels.  ``model``: PointNet2_tcls.PointNet2 on CUDA
-    (a fusable configuration, see PointNet2.fusable); ``loss_fn``: PointNet2Loss."""
+    """forward + loss + backward of PN2_CLS (PointNet2_tcls.PointNet2) or of the PN2 sibling (models.PointNet2) on the
+    fused training kernels.  ``model`` on CUDA, a configuration with a training plan (PointNet2.fusable; a global last
+    level paired with broadcast propagation after at least one sampled level); ``loss_fn``: the model's PointNet2Loss."""
 
     def __init__(self, model, loss_fn, seed=0):
-        if not model.fusable():
+        if not _has_training_plan(model):
             raise RuntimeError("TrainEngine: no fused plan for this configuration (PointNet2.fusable)")
         self.model, self.loss_fn = model, loss_fn
         self.cfg = model.config
+        # a last level with one global group (num_centroids = 0) and the broadcast first propagation level it pairs with
+        self.global_level = self.cfg["num_centroids"][-1] == 0
+        self._global_tables = {}  # (B, N) -> (identity neighbour table (B, 1, N) int32, zero centroids (B, 3, 1))
         self.step_count = 0
         self.seed = int(seed)
         self.sequential_heads = True
@@ -345,6 +384,17 @@ class TrainEngine:
     PRED_KEYS = ("score", "frame_R", "frame_t", "movable_logits")
     LOSS_KEYS = ("cls_loss", "R_loss", "t_loss", "mov_loss")  # PointNet2Loss: term k depends on head k only
 
+    def _global_group(self, B, N, dev):
+        """(identity neighbour table (B, 1, N) int32, zero centroids (B, 3, 1) fp32) of a global level over N points,
+        built once per shape.  Grouped with them, the rows are [features | xyz - 0 | 0]: every point of the scene exactly
+        once, with the absolute coordinates the reference concatenates (modules.py:93-98).  (Not the inference engine's
+        partial groups padded with repeated points: max ignores repeats, train-mode BatchNorm statistics do not.)"""
+        key = (B, N)
+        if key not in self._global_tables:
+            nbr = torch.arange(N, dtype=torch.int32, device=dev).expand(B, N).reshape(B, 1, N).contiguous()
+            self._global_tables[key] = (nbr, torch.zeros((B, 3, 1), dtype=torch.float32, device=dev))
+        return self._global_tables[key]
+
     def _trunk_forward(self, points):
         """set abstraction + feature propagation: points (B,3,N) fp32 -> per-point features [B*N, C] bf16"""
         cfg = self.cfg
@@ -357,9 +407,14 @@ class TrainEngine:
         for i, blocks in enumerate(self.sa):
             M, K = cfg["num_centroids"][i], cfg["num_neighbours"][i]
             N = xyz.shape[2]
-            idx = E.fps(xyz, M)
-            ctr = E.gather_xyz(xyz, idx)
-            nbr = E.ball_query(xyz, ctr, cfg["radius"][i], K)
+            glob = M == 0
+            if glob:  # one group of all N points per scene (the last level, after a sampled one: feat is set)
+                M, K = 1, N
+                nbr, ctr = self._global_group(B, N, dev)
+            else:
+                idx = E.fps(xyz, M)
+                ctr = E.gather_xyz(xyz, idx)
+                nbr = E.ball_query(xyz, ctr, cfg["radius"][i], K)
             cf = 0 if feat is None else feat.shape[1]
             x0 = torch.empty((B * M * K, cf + 8), dtype=BF16, device=dev)
             check(lib.s4g_train_group_rows_bf16(ptr(feat) if feat is not None else None, ptr(xyz), ptr(ctr), ptr(nbr), B, N, M,
@@ -367,9 +422,9 @@ class TrainEngine:
             h = x0
             for j, blk in enumerate(blocks):
                 last = j == len(blocks) - 1
-                h = blk.forward(h, pool_k=K if last else 0)
+                h = blk.forward(h, pool_k=K if last else 0, global_pool=glob and last)
             feat, _ = h
-            self._sa_ctx.append((nbr, B, N, M, K, cf))
+            self._sa_ctx.append((nbr, B, N, M, K, cf, glob))
             xyz = ctr
             lv_xyz.append(xyz)
             lv_feat.append(feat)
@@ -377,8 +432,15 @@ class TrainEngine:
         self._fp_ctx = []
         for i, blocks in enumerate(self.fp):
             dense_xyz, dense = lv_xyz[-2 - i], lv_feat[-2 - i]
-            idx3, w = E.three_nn_weights(dense_xyz, sparse_xyz)
             Nk, Nq = sparse_xyz.shape[2], dense_xyz.shape[2]
+            if i == 0 and self.global_level:  # broadcast propagation: rows [global | skip] (modules.py:131-134)
+                self._fp_ctx.append((None, None, B, Nk, Nq, sparse.shape[1], dense.shape[1], False))
+                h = E.broadcast_concat(sparse, dense, B, Nq)
+                for blk in blocks:
+                    h = blk.forward(h)
+                sparse_xyz, sparse = dense_xyz, h
+                continue
+            idx3, w = E.three_nn_weights(dense_xyz, sparse_xyz)
             split = FP_LINEAR_SPLIT and dense is None
             self._fp_ctx.append((idx3, w, B, Nk, Nq, sparse.shape[1], 0 if dense is None else dense.shape[1], split))
             if split:
@@ -395,6 +457,7 @@ class TrainEngine:
         self._lv_shapes = [None if f is None else tuple(f.shape) for f in lv_feat]
         self._n_points = sparse_xyz.shape[2]
         self._batch = B
+        self._points = points
         return sparse
 
     def _head_forward(self, k, point_feat):
@@ -428,7 +491,8 @@ class TrainEngine:
         return chain_backward(blocks, dz)
 
     def _predictions(self, leaves):
-        return {"score": leaves[0], "frame_R": leaves[1], "frame_t": leaves[2], "movable_logits": torch.sigmoid(leaves[3])}
+        raw = {"score": leaves[0], "frame_R": leaves[1], "frame_t": leaves[2], "movable_logits": torch.sigmoid(leaves[3])}
+        return self.model.predictions(raw, self._points)
 
     def forward(self, points):
         """points (B,3,N) fp32 CUDA -> predictions (fp32 (B, c, N) autograd leaves underneath); keeps what backward needs."""
@@ -470,6 +534,9 @@ class TrainEngine:
             # dz rows = [d interpolated (c2) | d dense skip (c1)]
             if c1:
                 lv_grad[-2 - i].add_(dz[:, c2:c2 + c1])
+            if idx3 is None:  # broadcast level: the global feature's gradient is the sum over each scene's rows
+                rows_segment_sum(dz, B, Nq, c2, lv_grad[-1])
+                continue
             d_sparse = interp_rows_backward(dz, idx3, w, B, Nk, Nq, c2, want_f32=(i == 0))
             if i == 0:
                 lv_grad[-1].add_(d_sparse)  # the coarsest propagation level interpolates the last SA level's features
@@ -477,20 +544,34 @@ class TrainEngine:
                 d_out = d_sparse
         for i in reversed(range(len(self.sa))):
             blocks = self.sa[i]
-            nbr, B, N, M, K, cf = self._sa_ctx[i]
+            nbr, B, N, M, K, cf, glob = self._sa_ctx[i]
             dz = lv_grad[i + 1].to(BF16)  # pooled gradient [B*M, cout]
             lv_grad[i + 1] = None
             dz = chain_backward(blocks, dz, need_dx=cf > 0)
-            if cf > 0:
+            if cf > 0 and glob:  # identity grouping: row b*N + n of the group is point n of scene b
+                lv_grad[i].add_(dz[:, :cf])
+            elif cf > 0:
                 group_rows_backward(dz, nbr, B, N, M, K, cf, lv_grad[i])
         self._sa_ctx = self._fp_ctx = None
 
     def _separable(self):
         """PointNet2Loss's four terms depend on one head each (cls <- score, R <- frame_R, t <- frame_t, mov <-
-        movable_logits, reference :162-219): the heads can then run forward + loss term + backward ONE AFTER THE OTHER,
-        so only one head's activations are alive at a time (-13 GB at 32 scenes)."""
-        from .network_models.models.PointNet2_tcls import PointNet2Loss
-        return self.sequential_heads and type(self.loss_fn) is PointNet2Loss
+        movable_logits, reference :162-219; the PN2 sibling's loss likewise, through its prediction mapping): the heads
+        can then run forward + loss term + backward ONE AFTER THE OTHER, so only one head's activations are alive at a
+        time (-13 GB at 32 scenes)."""
+        from .network_models.models import PointNet2, PointNet2_tcls
+        return self.sequential_heads and type(self.loss_fn) in (PointNet2_tcls.PointNet2Loss, PointNet2.PointNet2Loss)
+
+    def _placeholder(self, k):
+        """the value fed for head k's raw output while another head's loss term is computed: zeros, except a 6-D
+        rotation representation (the PN2 sibling's frame_R), whose Gram-Schmidt divides 0 by 0 — the identity there"""
+        B, n = self._batch, self._n_points
+        logit = self.heads[k][1]
+        z = torch.zeros((B, logit.weight.shape[0], n), dtype=torch.float32, device=logit.weight.device)
+        if k == 1 and z.shape[1] == 6:
+            z[:, 0] = 1.0
+            z[:, 4] = 1.0
+        return z
 
     def step_loss(self, data_batch, labels):
         """forward + loss + full backward; returns the (detached) loss dict.  Gradients accumulate in param.grad."""
@@ -508,9 +589,7 @@ class TrainEngine:
             self._head_saved = {}
             with torch.no_grad():
                 point_feat = self._trunk_forward(points)
-            B, n = self._batch, self._n_points
-            zeros = [torch.zeros((B, logit.weight.shape[0], n), dtype=torch.float32, device=points.device)
-                     for _, logit in self.heads]
+            zeros = [self._placeholder(k) for k in range(4)]
             losses, dzs = {}, []
             for k in range(4):
                 with torch.no_grad():
