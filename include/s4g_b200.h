@@ -293,6 +293,16 @@ int s4g_rows_segment_max_bf16(const void* in, int B, int P, int C, void* out, vo
 int s4g_broadcast_concat_bf16(const void* sparse, const void* dense, int B, int Nq, int C2, int C1, void* out,
                               void* stream);
 
+/* Input rows of PN2_LOCAL's grasp-evaluation head (PointNet2_local.py:131-147: the in-place translation update of :135,
+ * then torch.cat([per_point, frames.repeat(1, 4, 1, 1)], 1) ahead of mlp_grasp_eval): feat [B*N][C] bf16 (C % 8 == 0)
+ * -> out [B*F*S][C + 48] bf16, row (b, f, s) = feat row b*N + f, then the candidate's 12 values [R0..R8 t0..t2] x 4,
+ * each rounded to bf16 to nearest-even.
+ *   given (frames != NULL): frames (B, 12, F, S) fp32, points (B, 3, N) fp32, 1 <= F <= N, S >= 1; channels 9..11 become
+ *     t - points[b, :, f] (one fp32 subtraction), written back to frames, and are what the row holds;
+ *   self (frames == NULL): R (B, 9, N), t (B, 3, N) fp32 head outputs, F = N, S = 1. */
+int s4g_local_eval_rows_bf16(const void* feat, int B, int N, int C, float* frames, const float* points, int F, int S,
+                             const float* R, const float* t, void* out, void* stream);
+
 /* Fused shared-MLP chain on tcgen05 tensor cores (csrc/mlp_chain.cu): replaces
  * SharedMLP / Conv1d / Conv2d (nn_utils/mlp.py:95-106, nn_utils/conv.py:30-36,70-76) with eval-mode
  * BatchNorm folded in, and around it the grouping + max-pool of PointNetSAModule.forward

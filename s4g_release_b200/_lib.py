@@ -60,6 +60,7 @@ _SIGNATURES = {
     "s4g_gather_xyz_f32_i32": ([_vp, _vp, _i, _i, _i, _vp, _vp], _i),
     "s4g_rows_segment_max_bf16": ([_vp, _i, _i, _i, _vp, _vp], _i),
     "s4g_broadcast_concat_bf16": ([_vp, _vp, _i, _i, _i, _i, _vp, _vp], _i),
+    "s4g_local_eval_rows_bf16": ([_vp, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp], _i),
     "s4g_linear_tf32": ([_vp, ctypes.c_longlong, _vp, ctypes.c_longlong, _vp, _vp, ctypes.c_longlong, ctypes.c_longlong,
                          _i, _i, _i, _i, _vp], _i),
     "s4g_gemm_bf16": ([_vp, _ll, _vp, _ll, _vp, _ll, _ll, _i, _i, _vp], _i),

@@ -207,6 +207,72 @@ broadcast_concat_kernel(const uint4* __restrict__ sparse, const uint4* __restric
   }
 }
 
+// Input rows of PN2_LOCAL's grasp-evaluation head (PointNet2_local.forward_modules; reference :131-147): row (b, f, s) of [B*F*S][C + 48] is the
+// point feature of point f followed by the 12 candidate values [R0..R8 t0..t2] repeated 4 times, the order of
+// torch.cat([per_point, frames.repeat(1, 4, 1, 1)], 1).  12 values x 2 repeats = 24 bf16 = three 16-byte pieces, so the
+// 48 candidate channels are those three pieces twice.  Phase 1: one thread per row reads its 12 fp32 values (coalesced
+// across neighbouring (f, s)), in the given mode makes the translation relative to the point and writes it back to the
+// caller's frames (the reference's in-place update, :135), and stages the three bf16 pieces in shared memory.  Phase 2:
+// the block writes its rows, which are contiguous in the output, one thread per 16-byte piece.
+constexpr int kEvalRows = 256;
+
+__global__ void __launch_bounds__(kEvalRows)
+local_eval_rows_kernel(const uint4* __restrict__ feat, int N, int C8, float* frames, const float* __restrict__ points,
+                       const float* __restrict__ R, const float* __restrict__ t, int F, int S, long long rows,
+                       uint4* __restrict__ out) {
+  __shared__ uint4 s_cand[kEvalRows][3];
+  __shared__ long long s_src[kEvalRows];  // the row's point-feature row b * N + f
+  const long long r0 = (long long)blockIdx.x * kEvalRows;
+  const int nrows = (int)min((long long)kEvalRows, rows - r0);
+  const long long FS = (long long)F * S;
+  if ((int)threadIdx.x < nrows) {
+    const long long r = r0 + threadIdx.x;
+    const long long b = r / FS, fs = r - b * FS;
+    s_src[threadIdx.x] = b * N + fs / S;
+    float v[12];
+    if (frames != nullptr) {  // given: frames (B, 12, F, S); points (B, 3, N)
+      float* fr = frames + b * 12 * FS + fs;
+#pragma unroll
+      for (int k = 0; k < 9; ++k) v[k] = fr[k * FS];
+      const int f = (int)(fs / S);
+      const float* p = points + b * 3 * N + f;
+#pragma unroll
+      for (int k = 0; k < 3; ++k) {
+        v[9 + k] = __fsub_rn(fr[(9 + k) * FS], __ldg(p + (size_t)k * N));
+        fr[(9 + k) * FS] = v[9 + k];
+      }
+    } else {  // self: R (B, 9, N), t (B, 3, N); F = N, S = 1
+#pragma unroll
+      for (int k = 0; k < 9; ++k) v[k] = __ldg(R + (b * 9 + k) * N + fs);
+#pragma unroll
+      for (int k = 0; k < 3; ++k) v[9 + k] = __ldg(t + (b * 3 + k) * N + fs);
+    }
+    uint32_t h[12];
+#pragma unroll
+    for (int k = 0; k < 12; k += 2) {
+      const __nv_bfloat162 pr = __floats2bfloat162_rn(v[k], v[k + 1]);
+      h[k / 2] = *reinterpret_cast<const uint32_t*>(&pr);
+    }
+    // bf16 pairs: piece 0 = v0..v7, piece 1 = v8..v11 v0..v3, piece 2 = v4..v11
+    s_cand[threadIdx.x][0] = make_uint4(h[0], h[1], h[2], h[3]);
+    s_cand[threadIdx.x][1] = make_uint4(h[4], h[5], h[0], h[1]);
+    s_cand[threadIdx.x][2] = make_uint4(h[2], h[3], h[4], h[5]);
+  }
+  __syncthreads();
+  const int w8 = C8 + 6;
+  const int n = nrows * w8;
+  uint4* O = out + r0 * w8;
+  for (int i = threadIdx.x; i < n; i += kEvalRows) {
+    const int q = i / w8, c = i - q * w8;
+    uint4 val;
+    if (c < C8)
+      val = __ldg(feat + s_src[q] * C8 + c);
+    else
+      val = s_cand[q][(c - C8) % 3];
+    O[i] = val;
+  }
+}
+
 }  // namespace s4g
 
 extern "C" int s4g_rows_segment_max_bf16(const void* in, int B, int P, int C, void* out, void* stream) {
@@ -238,6 +304,25 @@ extern "C" int s4g_broadcast_concat_bf16(const void* sparse, const void* dense, 
       reinterpret_cast<const uint4*>(sparse), reinterpret_cast<const uint4*>(dense), Nq, C2 / 8, C1 / 8,
       reinterpret_cast<uint4*>(out));
   S4G_LAUNCH_CHECK("broadcast_concat");
+  return S4G_OK;
+}
+
+extern "C" int s4g_local_eval_rows_bf16(const void* feat, int B, int N, int C, float* frames, const float* points,
+                                        int F, int S, const float* R, const float* t, void* out, void* stream) {
+  S4G_CHECK_ARG(feat && out, "local_eval_rows: null pointer");
+  S4G_CHECK_ARG(frames ? points != nullptr : (R && t), "local_eval_rows: frames need points; without frames R and t");
+  S4G_CHECK_ARG(B >= 0 && N > 0 && C > 0 && C % 8 == 0, "local_eval_rows: bad shape (C %% 8 == 0)");
+  S4G_CHECK_ARG(frames ? (F >= 1 && F <= N && S >= 1) : (F == N && S == 1),
+                "local_eval_rows: bad candidate shape (given: 1 <= F <= N, S >= 1; self: F = N, S = 1)");
+  S4G_CHECK_ARG(((uintptr_t)feat & 15) == 0 && ((uintptr_t)out & 15) == 0,
+                "local_eval_rows: feature and output rows must be 16-byte aligned");
+  const long long rows = (long long)B * F * S;
+  S4G_CHECK_ARG((rows + s4g::kEvalRows - 1) / s4g::kEvalRows < (1ll << 31), "local_eval_rows: too many rows");
+  if (rows == 0) return S4G_OK;
+  const unsigned grid = (unsigned)((rows + s4g::kEvalRows - 1) / s4g::kEvalRows);
+  s4g::local_eval_rows_kernel<<<grid, s4g::kEvalRows, 0, (cudaStream_t)stream>>>(
+      reinterpret_cast<const uint4*>(feat), N, C / 8, frames, points, R, t, F, S, rows, reinterpret_cast<uint4*>(out));
+  S4G_LAUNCH_CHECK("local_eval_rows");
   return S4G_OK;
 }
 

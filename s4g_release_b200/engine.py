@@ -197,8 +197,7 @@ class FusedPointNet2:
         self.sa = [_fold_mlp(m.mlp) for m in model.sa_modules]
         self.fp = [_fold_mlp(m.mlp) for m in model.fp_modules]
         heads = []
-        for mlp, logit in ((model.mlp_seg, model.seg_logit), (model.mlp_R, model.R_logit),
-                           (model.mlp_t, model.t_logit), (model.mlp_movable, model.movable_logit[0])):
+        for mlp, logit in self._head_modules(model):
             w = logit.weight.detach().float()
             heads.append((_fold_mlp(mlp), w.reshape(w.shape[0], w.shape[1]).contiguous(),
                           logit.bias.detach().float().contiguous()))
@@ -209,6 +208,14 @@ class FusedPointNet2:
             self._prepare_tf32()
         elif mlp_backend != "torch":
             raise ValueError("mlp_backend must be 'tcgen05', 'tf32' or 'torch'")
+
+    _HEAD_SIGMOID = (False, False, False, True)  # per head of _head_modules: the logits epilogue applies a sigmoid
+
+    @staticmethod
+    def _head_modules(model):
+        """(SharedMLP, logit conv) of each head, in the order of the head stage's outputs."""
+        return ((model.mlp_seg, model.seg_logit), (model.mlp_R, model.R_logit), (model.mlp_t, model.t_logit),
+                (model.mlp_movable, model.movable_logit[0]))
 
     def _make_chain(self, layers, in_mode, feat_c, out_mode, group=1, sigmoid=False):
         """Builds one chain.  The planner ranks the shared-memory splits (activation slots vs weight stages) with a
@@ -324,7 +331,7 @@ class FusedPointNet2:
         self.head_chains = []
         for k, (layers, w, b) in enumerate(self.heads):
             self.head_chains.append(self._make_chain([(lw, lb, True) for lw, lb in layers] + [(w, b, False)], IN_ROWS, 0,
-                                                     OUT_LOGITS, sigmoid=(k == 3)))
+                                                     OUT_LOGITS, sigmoid=self._HEAD_SIGMOID[k]))
 
     def _global_chain(self, g):
         """The global level's max-pool chain for groups of g rows (g follows the cloud size, see global_group_table)."""
@@ -523,13 +530,14 @@ class FusedPointNet2:
             done.record()
         early_nn[fp_level] = (found, done)
 
-    def _forward_tcgen05(self, points, return_trace, timer=None, host_out=None):
+    def _trunk_tcgen05(self, points, trace, timer=None):
+        """Set abstraction + feature propagation -> (cloud (B,3,N) fp32, per-point features bf16 [B*N, C] channel-last,
+        the set-abstraction levels' features).  ``trace``: dict that receives the sampled indices, or None."""
         cfg = self.cfg
         xyz = points.float().contiguous()
         B = xyz.shape[0]
         feat = None  # bf16 [B*N, C] channel-last
         lv_xyz, lv_feat = [xyz], [None]
-        trace = {"fps": [], "ball": []}
         # The 3-NN searches of the propagation levels only need coordinates.  Farthest point sampling of levels >= 1 is
         # a latency chain on at most B x cluster SMs, so the search between levels i and i + 1 runs on a side stream
         # beside the sampling of level i + 1 (submitted after it: the sampler's CTAs are placed first): 0.54 + 0.37 ms
@@ -590,7 +598,7 @@ class FusedPointNet2:
             xyz = new_xyz
             lv_xyz.append(xyz)
             lv_feat.append(feat)
-            if return_trace:
+            if trace is not None:
                 trace["fps"].append(idx)
                 trace["ball"].append(nbr)
         if self.global_level:
@@ -637,7 +645,15 @@ class FusedPointNet2:
                 for ch in chains:
                     x = ch.run_rows(x)
             sparse_xyz, sparse = dense_xyz, x
-        n = sparse_xyz.shape[2]
+        return lv_xyz[0], sparse, lv_feat
+
+    def _head_stage(self, xyz, sparse, timer=None, host_out=None):
+        """PN2_CLS's four per-point heads on the trunk's features -> {score, frame_R, frame_t, movable_logits (after the
+        sigmoid)}, each (B, k, N) fp32."""
+        B, n = xyz.shape[0], xyz.shape[2]
+        if self.mlp_backend != "tcgen05":
+            outs = [self._head_reference(sparse, k) for k in range(4)]
+            return {"score": outs[0], "frame_R": outs[1], "frame_t": outs[2], "movable_logits": torch.sigmoid(outs[3])}
         names = ("score", "frame_R", "frame_t", "movable_logits")
         with _sec(timer, "heads.mlp"):
             outs = [None] * 4
@@ -665,12 +681,70 @@ class FusedPointNet2:
                 outs[k] = o
         if host_out is not None:
             torch.cuda.current_stream().wait_stream(self._copy_stream)  # the caller's synchronize covers the copies
-        preds = dict(zip(names, outs))
-        if return_trace:
-            trace["point_feature"] = sparse.float().reshape(B, n, -1)
-            trace["sa_feature"] = [f.float().reshape(B, -1, f.shape[1]) for f in lv_feat[1:]]
-            return preds, trace
-        return preds
+        return dict(zip(names, outs))
+
+    def _head_reference(self, sparse, k):
+        """Head k on the torch / tf32 backends: (B, N, C) fp32 features -> (B, k_out, N) logits, no sigmoid."""
+        layers, w, b = self.heads[k]
+        return self._logits(self._mlp(sparse, layers), w, b).transpose(1, 2).contiguous()
+
+    def _trunk_reference(self, points, trace):
+        """The trunk on the torch / tf32 backends -> (cloud (B,3,N), per-point features (B, N, C) fp32, the set-abstraction
+        levels' features)."""
+        cfg = self.cfg
+        xyz = points.float().contiguous()
+        feat = None
+        lv_xyz, lv_feat = [xyz], [None]
+        for i, layers in enumerate(self.sa):
+            if cfg["num_centroids"][i] == 0:  # global level: the same partial groups as the fused path
+                g, nbr, ctr = self._global_group(xyz.shape[0], xyz.shape[2])
+                feat = self._sa_torch(xyz, feat, ctr, nbr, layers).amax(dim=1, keepdim=True)  # (B,1,C)
+                xyz = ctr[:, :, :1]
+                lv_xyz.append(xyz)
+                lv_feat.append(feat)
+                continue
+            idx = self.fps(xyz, cfg["num_centroids"][i])
+            new_xyz = torch.gather(xyz, 2, idx.long().unsqueeze(1).expand(-1, 3, -1)).contiguous()
+            nbr = self.ball_query(xyz, new_xyz, cfg["radius"][i], cfg["num_neighbours"][i])
+            feat = self._sa_torch(xyz, feat, new_xyz, nbr, layers)
+            xyz = new_xyz
+            lv_xyz.append(xyz)
+            lv_feat.append(feat)
+            if trace is not None:
+                trace["fps"].append(idx)
+                trace["ball"].append(nbr)
+        sparse_xyz, sparse = xyz, feat
+        for i, layers in enumerate(self.fp):
+            dense_xyz, dense = lv_xyz[-2 - i], lv_feat[-2 - i]
+            if i == 0 and self.global_level:  # broadcast propagation, [global | skip] (modules.py:131-134)
+                x = sparse.expand(-1, dense_xyz.shape[2], -1)
+                sparse = self._mlp(x if dense is None else torch.cat([x, dense], dim=-1), layers)
+            else:
+                sparse = self._fp_torch(dense_xyz, sparse_xyz, dense, sparse, layers)
+            sparse_xyz = dense_xyz
+        return lv_xyz[0], sparse, lv_feat
+
+    def _run(self, points, return_trace, timer, head_stage):
+        """The trunk on this engine's backend, then ``head_stage(cloud, per-point features)``."""
+        if not points.is_cuda:
+            raise RuntimeError("scene_points must be a CUDA tensor (there is no CPU path)")
+        trace = {"fps": [], "ball": []} if return_trace else None
+        with torch.cuda.device(points.device):
+            if self.mlp_backend == "tcgen05":
+                xyz, sparse, lv_feat = self._trunk_tcgen05(points, trace, timer)
+            else:
+                xyz, sparse, lv_feat = self._trunk_reference(points, trace)
+            preds = head_stage(xyz, sparse)
+            if trace is None:
+                return preds
+            if self.mlp_backend == "tcgen05":
+                B, n = xyz.shape[0], xyz.shape[2]
+                trace["point_feature"] = sparse.float().reshape(B, n, -1)
+                trace["sa_feature"] = [f.float().reshape(B, -1, f.shape[1]) for f in lv_feat[1:]]
+            else:
+                trace["point_feature"] = sparse
+                trace["sa_feature"] = lv_feat[1:]
+        return preds, trace
 
     # ---------------------------------------------------------------- forward
     @torch.no_grad()
@@ -679,52 +753,85 @@ class FusedPointNet2:
         (same keys / shapes as the result); each head's output is then copied to it on a side stream as soon as that
         head finishes, overlapping the device -> host transfer with the remaining heads (the copies are ordered before
         the current stream's next operation, so one synchronize() after the call makes them visible)."""
-        if not points.is_cuda:
-            raise RuntimeError("scene_points must be a CUDA tensor (there is no CPU path)")
-        if self.mlp_backend == "tcgen05":
-            with torch.cuda.device(points.device):
-                return self._forward_tcgen05(points, return_trace, timer, host_out)
-        cfg = self.cfg
-        with torch.cuda.device(points.device):
-            xyz = points.float().contiguous()
-            feat = None
-            lv_xyz, lv_feat = [xyz], [None]
-            trace = {"fps": [], "ball": []}
-            for i, layers in enumerate(self.sa):
-                if cfg["num_centroids"][i] == 0:  # global level: the same partial groups as the fused path
-                    g, nbr, ctr = self._global_group(xyz.shape[0], xyz.shape[2])
-                    feat = self._sa_torch(xyz, feat, ctr, nbr, layers).amax(dim=1, keepdim=True)  # (B,1,C)
-                    xyz = ctr[:, :, :1]
-                    lv_xyz.append(xyz)
-                    lv_feat.append(feat)
-                    continue
-                idx = self.fps(xyz, cfg["num_centroids"][i])
-                new_xyz = torch.gather(xyz, 2, idx.long().unsqueeze(1).expand(-1, 3, -1)).contiguous()
-                nbr = self.ball_query(xyz, new_xyz, cfg["radius"][i], cfg["num_neighbours"][i])
-                feat = self._sa_torch(xyz, feat, new_xyz, nbr, layers)
-                xyz = new_xyz
-                lv_xyz.append(xyz)
-                lv_feat.append(feat)
-                if return_trace:
-                    trace["fps"].append(idx)
-                    trace["ball"].append(nbr)
-            sparse_xyz, sparse = xyz, feat
-            for i, layers in enumerate(self.fp):
-                dense_xyz, dense = lv_xyz[-2 - i], lv_feat[-2 - i]
-                if i == 0 and self.global_level:  # broadcast propagation, [global | skip] (modules.py:131-134)
-                    x = sparse.expand(-1, dense_xyz.shape[2], -1)
-                    sparse = self._mlp(x if dense is None else torch.cat([x, dense], dim=-1), layers)
-                else:
-                    sparse = self._fp_torch(dense_xyz, sparse_xyz, dense, sparse, layers)
-                sparse_xyz = dense_xyz
-            outs = []
-            for layers, w, b in self.heads:
-                h = self._mlp(sparse, layers)
-                outs.append(self._logits(h, w, b).transpose(1, 2).contiguous())
-            preds = {"score": outs[0], "frame_R": outs[1], "frame_t": outs[2],
-                     "movable_logits": torch.sigmoid(outs[3])}
-        if return_trace:
-            trace["point_feature"] = sparse
-            trace["sa_feature"] = lv_feat[1:]
-            return preds, trace
-        return preds
+        return self._run(points, return_trace, timer, lambda xyz, sparse: self._head_stage(xyz, sparse, timer, host_out))
+
+
+def check_local_frames(points, frames):
+    """The given candidates of PN2_LOCAL's evaluation head: (B, 12, F, S) fp32 contiguous on the points' device with
+    1 <= F <= N and S >= 1, else ValueError.  The fused path writes their translations back in place, as the reference
+    does, so it takes no copy."""
+    B, _, N = points.shape
+    if not (isinstance(frames, torch.Tensor) and frames.dim() == 4 and frames.shape[0] == B and frames.shape[1] == 12):
+        raise ValueError("local_search_frame must be a (B, 12, n_frames, n_search) tensor with B = %d" % B)
+    if frames.device != points.device or frames.dtype != torch.float32 or not frames.is_contiguous():
+        raise ValueError("local_search_frame must be a contiguous float32 tensor on %s (got %s %s%s)"
+                         % (points.device, frames.dtype, frames.device, "" if frames.is_contiguous() else ", strided"))
+    F, S = frames.shape[2], frames.shape[3]
+    if not (1 <= F <= N and S >= 1):
+        raise ValueError("local_search_frame needs 1 <= n_frames <= %d points and n_search >= 1 (got %d, %d)" % (N, F, S))
+
+
+class FusedPointNet2Local(FusedPointNet2):
+    """PN2_LOCAL (models/PointNet2_local.py): the trunk of FusedPointNet2 unchanged, its own head stage.  Three per-point
+    heads (frame_R 9, frame_t 3, movable 2 logits, no sigmoid) and the grasp-evaluation head: one logits chain over the
+    rows [point feature | candidate (R 9, t 3) x 4] that ``local_eval_rows`` writes, one row per candidate."""
+
+    _HEAD_SIGMOID = (False, False, False, False)
+
+    @staticmethod
+    def _head_modules(model):
+        return ((model.mlp_R, model.R_logit), (model.mlp_t, model.t_logit), (model.mlp_movable, model.movable_logit),
+                (model.mlp_grasp_eval, model.grasp_eval_logit))
+
+    @staticmethod
+    def local_eval_rows(feat, xyz, frames=None, R=None, t=None):
+        """feat bf16 [B*N, C]; given: frames (B, 12, F, S) fp32, whose translations become relative to xyz (B,3,N) IN
+        PLACE; self: R (B, 9, N), t (B, 3, N) fp32 -> bf16 [B*F*S, C + 48] rows [feature | (R, t) x 4]."""
+        B, _, N = xyz.shape
+        C = feat.shape[1]
+        F, S = (frames.shape[2], frames.shape[3]) if frames is not None else (N, 1)
+        out = torch.empty((B * F * S, C + 48), dtype=torch.bfloat16, device=feat.device)
+        check(lib.s4g_local_eval_rows_bf16(ptr(feat), B, N, C, ptr(frames) if frames is not None else None, ptr(xyz),
+                                           F, S, ptr(R) if R is not None else None, ptr(t) if t is not None else None,
+                                           ptr(out), stream_ptr(feat.device)), "local_eval_rows")
+        return out
+
+    def _local_head_stage(self, xyz, sparse, frames, timer):
+        """-> raw {local_search_logits (B, k, F, S), frame_R (B, 9, N), frame_t (B, 3, N) offset, movable_logits}."""
+        B, n = xyz.shape[0], xyz.shape[2]
+        F, S = (frames.shape[2], frames.shape[3]) if frames is not None else (n, 1)
+        if self.mlp_backend != "tcgen05":
+            R, t, mov = [self._head_reference(sparse, k) for k in range(3)]
+            if frames is None:  # the prediction itself, one candidate per point
+                cand = torch.cat([R, t], dim=1).transpose(1, 2).unsqueeze(2)  # (B, N, 1, 12)
+                per_point = sparse.unsqueeze(2)
+            else:  # the reference's in-place update of the caller's frames (PointNet2_local.py:135)
+                frames[:, 9:] = frames[:, 9:] - xyz[:, :, :F].unsqueeze(-1).expand(-1, -1, -1, S)
+                cand = frames.permute(0, 2, 3, 1)  # (B, F, S, 12)
+                per_point = sparse[:, :F].unsqueeze(2).expand(-1, -1, S, -1)
+            x = torch.cat([per_point, cand.repeat(1, 1, 1, 4)], dim=-1)
+            layers, w, b = self.heads[3]
+            logits = self._logits(self._mlp(x, layers), w, b).permute(0, 3, 1, 2).contiguous()
+        else:
+            R_ch, t_ch, mov_ch, eval_ch = self.head_chains
+            with _sec(timer, "heads.R"):
+                R = R_ch.run_rows(sparse, n_points=n)
+            with _sec(timer, "heads.t"):
+                t = t_ch.run_rows(sparse, n_points=n)
+            with _sec(timer, "heads.movable"):
+                mov = mov_ch.run_rows(sparse, n_points=n)
+            with _sec(timer, "heads.eval_rows"):
+                rows = self.local_eval_rows(sparse, xyz, frames, R, t)
+            with _sec(timer, "heads.eval_mlp"):
+                logits = eval_ch.run_rows(rows, n_points=F * S).view(B, -1, F, S)
+        return {"local_search_logits": logits, "frame_R": R, "frame_t": t, "movable_logits": mov}
+
+    @torch.no_grad()
+    def forward(self, points, frames=None, return_trace=False, timer=None):
+        """points (B,3,N) fp32 CUDA; ``frames``: None (each point's own (R, t) prediction is its one candidate) or the
+        given candidates (B, 12, F, S) fp32 (check_local_frames), whose translation rows are made relative to their
+        point IN PLACE, as the reference does.  -> the raw head outputs; the model adds the points to frame_t."""
+        if frames is not None:
+            check_local_frames(points, frames)
+        return self._run(points, return_trace, timer,
+                         lambda xyz, sparse: self._local_head_stage(xyz, sparse, frames, timer))

@@ -6,7 +6,13 @@ Encoder / decoder as PN2 and PN2_CLS (the same sm_100a operators through pointne
 [point feature | candidate frame (R 9 + t 3) repeated 4 times = 48 channels] (:86-87, :131-147).  With
 ``data_batch["local_search_frame"]`` (B, 12, n_frames, n_search) the candidates are given — their translations are made
 relative to the point they belong to, IN PLACE like the reference (:135) — else the network's own (R, t) prediction
-is the single candidate per point.  This head structure has no fused-engine plan: the model runs on the module path.
+is the single candidate per point.
+
+Two execution paths share the parameters: the module path (the default, ``fused=None`` or ``fused=False``) and, only
+when asked with ``forward(..., fused=True)``, the fused sm_100a engine (``engine.FusedPointNet2Local``): the trunk of
+PN2_CLS, the three per-point heads as logits chains, and the evaluation head as one logits chain over bf16 rows
+[point feature | candidate x 4] written by one kernel.  The given candidates' translations are updated in place there
+too, with the same fp32 subtraction.
 """
 import torch
 import torch.nn as nn
@@ -14,12 +20,14 @@ import torch.nn.functional as F
 
 from ..nn_utils.functional import smooth_cross_entropy
 from ..nn_utils.mlp import SharedMLP
+from .PointNet2_tcls import FusedEngineCache, _widths_ok, trunk_fusable
 from .pointnet2_utils.modules import PointNetSAModule, PointnetFPModule
 
 
-class PointNet2(nn.Module):
+class PointNet2(FusedEngineCache, nn.Module):
     _SA_MODULE = PointNetSAModule
     _FP_MODULE = PointnetFPModule
+    _ENGINE = "FusedPointNet2Local"
 
     def __init__(self,
                  score_classes,
@@ -35,6 +43,10 @@ class PointNet2(nn.Module):
         n_sa, n_fp = len(num_centroids), len(fp_channels)
         assert len(radius) == n_sa and len(num_neighbours) == n_sa and len(sa_channels) == n_sa
         assert n_sa == n_fp and len(num_fp_neighbours) == n_fp
+        self.config = dict(score_classes=score_classes, num_centroids=tuple(num_centroids), radius=tuple(radius),
+                           num_neighbours=tuple(num_neighbours), sa_channels=tuple(map(tuple, sa_channels)),
+                           fp_channels=tuple(map(tuple, fp_channels)), num_fp_neighbours=tuple(num_fp_neighbours),
+                           seg_channels=tuple(seg_channels), dropout_prob=dropout_prob)
         self.sa_modules = nn.ModuleList()
         c = 0
         for i in range(n_sa):
@@ -59,12 +71,46 @@ class PointNet2(nn.Module):
         self.mlp_movable = SharedMLP(c, seg_channels, ndim=1, dropout_prob=dropout_prob)
         self.movable_logit = nn.Conv1d(seg_channels[-1], 2, 1, bias=True)
         self.init_weights()
+        self._engine = None
+        self._engine_key = None
 
     def init_weights(self):
         nn.init.zeros_(self.t_logit.weight)
         nn.init.zeros_(self.t_logit.bias)
 
-    def forward(self, data_batch):
+    def fusable(self, allow_global=False):
+        """Whether the fused engine has a plan for this configuration: the trunk rules of PN2_CLS
+        (PointNet2_tcls.trunk_fusable, ``allow_global`` as there), head widths that are multiples of 16 and <= 512, at
+        most 16 evaluation classes.  ``forward(fused=True)`` asks with ``allow_global=True``."""
+        c = self.config
+        if not trunk_fusable(c, allow_global):
+            return False
+        if not _widths_ok(c["seg_channels"]) or any(w > 512 for w in c["seg_channels"]):
+            return False
+        return c["score_classes"] <= 16
+
+    def forward(self, data_batch, fused=None):
+        """``fused``: None / False = the module path; True = the fused engine, for every configuration
+        ``fusable(allow_global=True)`` accepts (others raise RuntimeError before any GPU work; given frames that are not
+        (B, 12, F, S) contiguous float32 on the points' device with 1 <= F <= N, S >= 1 raise ValueError)."""
+        if not fused:
+            return self.forward_modules(data_batch)
+        points = data_batch["scene_points"]
+        if not self.fusable(allow_global=True):
+            raise RuntimeError("the fused engine has no plan for this configuration (see PointNet2_local.PointNet2.fusable);"
+                               " call with fused=False for the module path")
+        frames = data_batch["local_search_frame"] if "local_search_frame" in data_batch else None
+        if frames is not None:
+            from ...engine import check_local_frames
+            check_local_frames(points, frames)
+        return self.predictions(self.fused_engine().forward(points, frames), points)
+
+    def predictions(self, raw, points):
+        """The engine's raw head outputs -> this model's predictions: ``frame_t`` is the offset added to the points."""
+        return {"local_search_logits": raw["local_search_logits"], "frame_R": raw["frame_R"],
+                "frame_t": points + raw["frame_t"], "movable_logits": raw["movable_logits"]}
+
+    def forward_modules(self, data_batch):
         points = data_batch["scene_points"]
         xyz, feature = points, None
         level_xyz, level_feature = [xyz], [feature]

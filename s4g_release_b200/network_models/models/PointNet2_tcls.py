@@ -37,7 +37,96 @@ PN2_CLS_CONFIG = dict(
 NUM_INPUT = 25600
 
 
-class PointNet2(nn.Module):
+def _widths_ok(chans):
+    return all(w % 16 == 0 and w >= 16 for w in chans)
+
+
+def trunk_fusable(c, allow_global=False):
+    """Whether the fused engine has a plan for the trunk (encoder + decoder) of the configuration dict ``c``: every level
+    samples centroids, neighbourhoods of 8 / 16 / 32 / 64 points, 3-NN propagation, hidden widths that are multiples of
+    16 and <= 512 inside a chain (a FP chain is cut after a wider layer, so only its LAST layer may be).
+
+    ``allow_global=True`` also admits a LAST set-abstraction level with one global group (num_centroids = 0,
+    num_neighbours = -1) paired with a first propagation level that broadcasts its feature (num_fp_neighbours[0] = 0).
+    Shared by the models whose heads the engine runs (PN2_CLS, the PN2 sibling, PN2_LOCAL)."""
+    cent, nbrs, fp_nbrs = c["num_centroids"], c["num_neighbours"], c["num_fp_neighbours"]
+    if allow_global and cent[-1] == 0 and nbrs[-1] < 0 and fp_nbrs[0] == 0:
+        cent, nbrs, fp_nbrs = cent[:-1], nbrs[:-1], fp_nbrs[1:]  # the rules below cover the remaining levels
+    if not all(n > 0 for n in cent) or not all(k in (8, 16, 32, 64) for k in nbrs):
+        return False
+    if not all(k == 3 for k in fp_nbrs):
+        return False
+    for chans in c["sa_channels"]:
+        if not _widths_ok(chans) or any(w > 512 for w in chans[:-1]) or chans[-1] > 1024:
+            return False
+    for chans in c["fp_channels"]:
+        if not _widths_ok(chans) or any(w > 1024 for w in chans):
+            return False
+    return True
+
+
+class FusedEngineCache:
+    """The fused inference engine of a model, cached and bound to its CURRENT parameters.  ``_ENGINE`` names the engine
+    class in engine.py; the model sets ``_engine = _engine_key = None`` in its constructor."""
+    _ENGINE = "FusedPointNet2"
+
+    def _param_fingerprint(self):
+        """Device + summed version counters of every parameter and buffer: changes on in-place updates under no_grad
+        (optimizer steps, EMA), on top of the explicit invalidation in train() / _apply() / load_state_dict().  Writes
+        through ``p.data`` bypass the version counter — call ``invalidate_engine()`` after those."""
+        tensors = self.__dict__.get("_engine_tensors")
+        if tensors is None:
+            tensors = list(self.parameters()) + list(self.buffers())
+            self.__dict__["_engine_tensors"] = tensors
+        return (tensors[0].device, tensors[0].dtype, sum(t._version for t in tensors))
+
+    def invalidate_engine(self):
+        self._engine = None
+        self._engine_key = None
+        self.__dict__.pop("_engine_tensors", None)
+
+    def attach_engine(self, engine):
+        """Use an engine built by the caller (e.g. with another MLP backend) for this module's current parameters."""
+        self._engine = engine
+        self._engine_key = self._param_fingerprint()
+
+    def fused_engine(self, refresh=False):
+        """The fused sm_100a inference engine bound to this module's CURRENT parameters (rebuilt when they changed)."""
+        key = self._param_fingerprint()
+        if self._engine is None or refresh or key != self._engine_key:
+            from ... import engine
+            self._engine = getattr(engine, self._ENGINE)(self)
+            self._engine_key = key
+        return self._engine
+
+    def train(self, mode=True):
+        self.invalidate_engine()  # parameters may change: re-fold BN on the next eval forward
+        return super().train(mode)
+
+    def _apply(self, fn, *args, **kwargs):
+        self.invalidate_engine()  # .to() / .cuda() / .half(): the engine's buffers live on the old device
+        return super()._apply(fn, *args, **kwargs)
+
+    def load_state_dict(self, *args, **kwargs):
+        self.invalidate_engine()
+        return super().load_state_dict(*args, **kwargs)
+
+    def __getstate__(self):  # copy.deepcopy / torch.save(model): the engine holds ctypes handles
+        state = self.__dict__.copy()
+        state["_engine"], state["_engine_key"] = None, None
+        state.pop("_engine_tensors", None)
+        return state
+
+    def __deepcopy__(self, memo):
+        import copy
+        clone = self.__class__.__new__(self.__class__)
+        memo[id(self)] = clone
+        for k, v in self.__getstate__().items():
+            clone.__dict__[k] = copy.deepcopy(v, memo)
+        return clone
+
+
+class PointNet2(FusedEngineCache, nn.Module):
     _SA_MODULE = PointNetSAModule
     _FP_MODULE = PointnetFPModule
     _R_OUT, _T_OUT = 9, 4  # frame_R: flattened 3x3; frame_t: 4 approach-offset classes (the PN2 sibling: 6 and 3)
@@ -116,88 +205,19 @@ class PointNet2(nn.Module):
 
     # ------------------------------------------------------------------ fused (inference) path
     def fusable(self, allow_global=False):
-        """Whether the fused engine has a plan for this configuration (engine.py / csrc/chain_plan.cu): every level
-        samples centroids, neighbourhoods of 8 / 16 / 32 / 64 points, 3-NN propagation, hidden widths that are multiples
-        of 16 and <= 512 inside a chain (a FP chain is cut after a wider layer, so only its LAST layer may be), at most
-        16 logits per head.
+        """Whether the fused engine has a plan for this configuration (engine.py / csrc/chain_plan.cu): the trunk rules of
+        ``trunk_fusable``, head widths that are multiples of 16 and <= 512, at most 16 logits per head.  Anything else
+        runs on the module path, like the reference.
 
-        ``allow_global=True`` also admits a LAST set-abstraction level with one global group (num_centroids = 0,
-        num_neighbours = -1) paired with a first propagation level that broadcasts its feature (num_fp_neighbours[0]
-        = 0) — e.g. this class's own default constructor arguments.  ``forward(fused=True)`` accepts those; the
-        automatic route (``fused=None``) uses the default answer and runs them on the module path, like the reference."""
+        ``allow_global=True`` also admits a global last level (see ``trunk_fusable``) — e.g. this class's own default
+        constructor arguments.  ``forward(fused=True)`` accepts those; the automatic route (``fused=None``) uses the
+        default answer and runs them on the module path, like the reference."""
         c = self.config
-        cent, nbrs, fp_nbrs = c["num_centroids"], c["num_neighbours"], c["num_fp_neighbours"]
-        if allow_global and cent[-1] == 0 and nbrs[-1] < 0 and fp_nbrs[0] == 0:
-            cent, nbrs, fp_nbrs = cent[:-1], nbrs[:-1], fp_nbrs[1:]  # the rules below cover the remaining levels
-        if not all(n > 0 for n in cent) or not all(k in (8, 16, 32, 64) for k in nbrs):
+        if not trunk_fusable(c, allow_global):
             return False
-        if not all(k == 3 for k in fp_nbrs):
-            return False
-        widths_ok = lambda chans: all(w % 16 == 0 and w >= 16 for w in chans)
-        for chans in c["sa_channels"]:
-            if not widths_ok(chans) or any(w > 512 for w in chans[:-1]) or chans[-1] > 1024:
-                return False
-        for chans in c["fp_channels"]:
-            if not widths_ok(chans) or any(w > 1024 for w in chans):
-                return False
-        if not widths_ok(c["seg_channels"]) or any(w > 512 for w in c["seg_channels"]):
+        if not _widths_ok(c["seg_channels"]) or any(w > 512 for w in c["seg_channels"]):
             return False
         return max(c["score_classes"], self._R_OUT, self._T_OUT, c["num_removal_directions"]) <= 16
-
-    def _param_fingerprint(self):
-        """Device + summed version counters of every parameter and buffer: changes on in-place updates under no_grad
-        (optimizer steps, EMA), on top of the explicit invalidation in train() / _apply() / load_state_dict().  Writes
-        through ``p.data`` bypass the version counter — call ``invalidate_engine()`` after those."""
-        tensors = self.__dict__.get("_engine_tensors")
-        if tensors is None:
-            tensors = list(self.parameters()) + list(self.buffers())
-            self.__dict__["_engine_tensors"] = tensors
-        return (tensors[0].device, tensors[0].dtype, sum(t._version for t in tensors))
-
-    def invalidate_engine(self):
-        self._engine = None
-        self._engine_key = None
-        self.__dict__.pop("_engine_tensors", None)
-
-    def attach_engine(self, engine):
-        """Use an engine built by the caller (e.g. with another MLP backend) for this module's current parameters."""
-        self._engine = engine
-        self._engine_key = self._param_fingerprint()
-
-    def fused_engine(self, refresh=False):
-        """The fused sm_100a inference engine bound to this module's CURRENT parameters (rebuilt when they changed)."""
-        key = self._param_fingerprint()
-        if self._engine is None or refresh or key != self._engine_key:
-            from ...engine import FusedPointNet2
-            self._engine = FusedPointNet2(self)
-            self._engine_key = key
-        return self._engine
-
-    def train(self, mode=True):
-        self.invalidate_engine()  # parameters may change: re-fold BN on the next eval forward
-        return super().train(mode)
-
-    def _apply(self, fn, *args, **kwargs):
-        self.invalidate_engine()  # .to() / .cuda() / .half(): the engine's buffers live on the old device
-        return super()._apply(fn, *args, **kwargs)
-
-    def load_state_dict(self, *args, **kwargs):
-        self.invalidate_engine()
-        return super().load_state_dict(*args, **kwargs)
-
-    def __getstate__(self):  # copy.deepcopy / torch.save(model): the engine holds ctypes handles
-        state = self.__dict__.copy()
-        state["_engine"], state["_engine_key"] = None, None
-        state.pop("_engine_tensors", None)
-        return state
-
-    def __deepcopy__(self, memo):
-        import copy
-        clone = self.__class__.__new__(self.__class__)
-        memo[id(self)] = clone
-        for k, v in self.__getstate__().items():
-            clone.__dict__[k] = copy.deepcopy(v, memo)
-        return clone
 
     def forward(self, data_batch, fused=None, host_out=None):
         """``fused``: None = the fused engine in eval + no_grad on CUDA when ``fusable()``, else the module path;
