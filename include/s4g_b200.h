@@ -84,7 +84,10 @@ int s4g_group_points_backward_f32(const float* grad_out, const int64_t* index, i
 
 /* point_search (3-NN) — csrc/interpolate.h:8-11, interpolate_kernel.cu:92-132.
  * query (B,3,Nq), key (B,3,Nk) -> index (B,Nq,3) int64, distance (B,Nq,3) = SQUARED distances,
- * ascending, earlier key wins ties.  num_neighbours must be 3 and Nk >= 3. */
+ * ascending, earlier key wins ties.  num_neighbours must be 3 and Nk >= 3.  A key counts only when its squared
+ * distance is below 1e40 (+inf in fp32), so NaN and overflowing distances never do.  When c < 3 keys count (a NaN
+ * query, NaN keys, |x| >~ 2e19 in fp32), the slots keep the reference's start values (interpolate_kernel.cu:53-54):
+ * slot c is (distance 1e40, index -1) and the slots after it (0, index 0). */
 int s4g_point_search_f32(const float* query, const float* key, int B, int Nq, int Nk, int num_neighbours,
                          int64_t* index, float* distance, void* stream);
 
@@ -263,7 +266,10 @@ int s4g_train_sum_bf16(const void* a, const void* b, const void* c, const void* 
 
 /* PointSearch (interpolate_kernel.cu:33-81) fused with the inverse-squared-distance weights of
  * FeatureInterpolator.forward (pointnet2_utils/modules.py:115-120).  index (B,Nq,3) int32,
- * weight (B,Nq,3) fp32 (normalised). */
+ * weight (B,Nq,3) fp32 (normalised): v_k = 1/max(d_k, 1e-10), w_k = v_k / ((v_0 + v_1) + v_2), IEEE fp32, on the
+ * distances s4g_point_search_f32 returns, so with fewer than three finite distances too (an all-NaN query gets
+ * [0, 0.5, 0.5]).  Where point_search returns index -1 this writes 0; the weight there is 0, so every index is a valid
+ * key row in [0, Nk). */
 int s4g_three_nn_weights_f32_i32(const float* query, const float* key, int B, int Nq, int Nk, int* index,
                                  float* weight, void* stream);
 

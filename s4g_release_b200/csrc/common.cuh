@@ -41,6 +41,19 @@ __device__ __forceinline__ float sqdist(float dx, float dy, float dz) {
   return __fmaf_rn(dz, dz, __fmaf_rn(dx, dx, __fmul_rn(dy, dy)));
 }
 
+// The reference's 3-NN starts from distances {1e40, 0, 0} and indices {-1, 0, 0} (interpolate_kernel.cu:53-54; 1e40 is
+// +inf in fp32) and inserts a key only when its distance is below a slot's.  The searches here start all three slots at
+// `big` (1e40 in the dtype), which reaches the same state once two keys are below `big`.  With fewer (NaN points,
+// distances that overflow), this rewrites the slots to the reference's leftovers: with c keys below `big`, slot c is
+// (big, -1) and the slots after it (0, index 0).  Slots are ascending, so the filled ones come first; a slot at `big` or
+// above counts as unfilled, which also drops keys a search kept on a tie at +inf.  No-op when c = 3.
+template <typename T>
+__device__ __forceinline__ void three_nn_reference_tail(T& d0, T& d1, T& d2, int& i0, int& i1, int& i2, T big) {
+  if (!(d2 < big)) { d2 = big; i2 = -1; }
+  if (!(d1 < big)) { d1 = big; i1 = -1; d2 = T(0); i2 = 0; }
+  if (!(d0 < big)) { d0 = big; i0 = -1; d1 = T(0); i1 = 0; }
+}
+
 // SM count of the CURRENT device (cached per device: a process may drive several GPUs)
 inline int num_sms() {
   static int cache[64] = {};

@@ -30,7 +30,7 @@ three_nn_weights_kernel(const float* __restrict__ query, const float* __restrict
   const float x1 = Q[iq], y1 = Q[Nq + iq], z1 = Q[2 * Nq + iq];
   const float inf = __int_as_float(0x7f800000);
   float d0 = inf, d1 = inf, d2 = inf;
-  int i0 = 0, i1 = 0, i2 = 0;
+  int i0 = -1, i1 = -1, i2 = -1;
   for (int base = 0; base < Nk; base += kNnwTile) {
     const int n = min(kNnwTile, Nk - base);
     __syncthreads();
@@ -52,13 +52,15 @@ three_nn_weights_kernel(const float* __restrict__ query, const float* __restrict
     }
   }
   if (valid) {
+    // the reference's distances when fewer than three are finite; its index -1 (weight 1/inf = 0) is written as 0
+    three_nn_reference_tail(d0, d1, d2, i0, i1, i2, inf);
     const float v0 = __fdiv_rn(1.0f, fmaxf(d0, 1e-10f));
     const float v1 = __fdiv_rn(1.0f, fmaxf(d1, 1e-10f));
     const float v2 = __fdiv_rn(1.0f, fmaxf(d2, 1e-10f));
     const float norm = __fadd_rn(__fadd_rn(v0, v1), v2);
     int* oi = index + ((size_t)b * Nq + i) * 3;
     float* ow = weight + ((size_t)b * Nq + i) * 3;
-    oi[0] = i0; oi[1] = i1; oi[2] = i2;
+    oi[0] = max(i0, 0); oi[1] = max(i1, 0); oi[2] = max(i2, 0);
     ow[0] = __fdiv_rn(v0, norm); ow[1] = __fdiv_rn(v1, norm); ow[2] = __fdiv_rn(v2, norm);
   }
 }

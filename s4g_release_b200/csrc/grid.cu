@@ -378,16 +378,20 @@ __device__ __forceinline__ void top3_insert(Top3& t, float d, int j) {
   }
 }
 
-// output: MODE 0 -> int64 index + squared distance (pn2_ext.point_search); MODE 1 -> int32 index + weights
+// output: MODE 0 -> int64 index + squared distance (pn2_ext.point_search); MODE 1 -> int32 index + weights.
+// Slots without a key below +inf (they hold +inf / 0x7fffffff, or a key kept on a tie at +inf) become the reference's
+// leftovers first; MODE 1 then computes the weights from those distances and writes index 0 for the reference's -1,
+// whose weight is 1/inf = 0, so every index it writes is a valid key row.
 template <int MODE>
-__device__ __forceinline__ void top3_store(const Top3& t, size_t q, void* index, float* out) {
+__device__ __forceinline__ void top3_store(Top3 t, size_t q, void* index, float* out) {
+  three_nn_reference_tail(t.d0, t.d1, t.d2, t.i0, t.i1, t.i2, __int_as_float(0x7f800000));
   if (MODE == 0) {
     int64_t* oi = reinterpret_cast<int64_t*>(index) + q * 3;
     oi[0] = t.i0; oi[1] = t.i1; oi[2] = t.i2;
     out[q * 3 + 0] = t.d0; out[q * 3 + 1] = t.d1; out[q * 3 + 2] = t.d2;
   } else {
     int* oi = reinterpret_cast<int*>(index) + q * 3;
-    oi[0] = t.i0; oi[1] = t.i1; oi[2] = t.i2;
+    oi[0] = max(t.i0, 0); oi[1] = max(t.i1, 0); oi[2] = max(t.i2, 0);
     const float v0 = __fdiv_rn(1.0f, fmaxf(t.d0, 1e-10f));
     const float v1 = __fdiv_rn(1.0f, fmaxf(t.d1, 1e-10f));
     const float v2 = __fdiv_rn(1.0f, fmaxf(t.d2, 1e-10f));

@@ -139,8 +139,8 @@ group_backward64_kernel(const double* __restrict__ grad_out, const int64_t* __re
 }
 
 // 3-NN (interpolate_kernel.cu:33-81): one thread per query, keys staged through shared memory; strict '<'
-// insertion in key order.  The reference starts from {1e40, 0, 0} / {-1, 0, 0}; with Nk >= 3 (checked by the
-// caller) the zeros are shifted out by the first keys, the same state an all-1e40 start reaches.
+// insertion in key order.  The reference starts from {1e40, 0, 0} / {-1, 0, 0}: the same state as this all-1e40 start
+// once two keys are closer than 1e40; three_nn_reference_tail restores the reference's slots when fewer are.
 constexpr int kNn64Tile = 1024;
 __global__ void __launch_bounds__(256)
 point_search64_kernel(const double* __restrict__ query, const double* __restrict__ key, int Nq, int Nk,
@@ -175,6 +175,7 @@ point_search64_kernel(const double* __restrict__ query, const double* __restrict
     }
   }
   if (valid) {
+    three_nn_reference_tail(d0, d1, d2, i0, i1, i2, 1e40);
     int64_t* oi = index + ((size_t)b * Nq + i) * 3;
     double* od = distance + ((size_t)b * Nq + i) * 3;
     oi[0] = i0; oi[1] = i1; oi[2] = i2;

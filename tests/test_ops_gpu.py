@@ -93,7 +93,8 @@ BQ_CASES = [
     ("uniform", 3, 777, 333, 0.2, 7), ("uniform", 2, 100, 100, 0.5, 128), ("uniform", 2, 50, 3, 1e-4, 8),
     ("lattice", 2, 2000, 500, 0.125, 32), ("lattice", 2, 2000, 500, 0.25, 64), ("dup", 2, 3000, 400, 0.05, 32),
     ("identical", 2, 300, 20, 0.1, 16), ("uniform", 2, 33, 33, 10.0, 40), ("uniform", 1, 4099, 517, 0.07, 33),
-    # grid path (N >= 4096): ties, duplicates, buffer overflow -> exact linear-scan fallback, huge / tiny radii
+    # linear-scan kernel (N < 8192) on ties, duplicates, identical points, huge / tiny radii; the 20000-point case runs
+    # the grid kernel (N >= 8192), whose edge cases are in test_geometry_edges_gpu.py
     ("lattice", 2, 6000, 700, 0.125, 32), ("lattice", 2, 6000, 300, 0.3, 64), ("dup", 2, 8000, 900, 0.05, 32),
     ("identical", 2, 5000, 40, 0.1, 16), ("uniform", 2, 5000, 300, 10.0, 128), ("uniform", 2, 5000, 300, 1e-4, 8),
     ("uniform", 1, 20000, 1000, 0.05, 200), ("uniform", 3, 4096, 512, 0.11, 64),
