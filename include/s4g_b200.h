@@ -215,6 +215,21 @@ int s4g_train_bn_bwd_reduce_seg_bf16(const void* dz, const int* arg, long long N
 int s4g_train_bn_bwd_apply_seg_bf16(const void* dz, const int* arg, long long N, const void* y, const float* scale,
                                     const float* shift, const float* ka, const float* kb, const float* kc, long long P, int C,
                                     int relu, void* dy, void* stream);
+/* Channel dropout (F.dropout2d, the evaluation head's SharedMLP(ndim=2), nn_utils/mlp.py:27) in place of element dropout:
+ * rows [P][C] of P / scene_rows scenes (P < 2^31, whole scenes); each (scene, channel) is kept with probability
+ * 1 - drop_p, deterministically from (seed, scene, channel): the element hash of s4g_train_bn_act_bf16 evaluated at
+ * row = scene.  Kept channels are scaled by 1 / (1 - drop_p) on every row of their scene, dropped ones are zero.
+ * The forward (z = chdrop(relu(y * scale + shift))) and the two BatchNorm-backward passes, which recompute the mask;
+ * otherwise as s4g_train_bn_act_bf16 / s4g_train_bn_bwd_reduce_bf16 / s4g_train_bn_bwd_apply_bf16 with a dense dz.
+ * Rows 16-byte aligned. */
+int s4g_train_bn_act_chdrop_bf16(const void* y, const float* scale, const float* shift, void* z, long long P, int C, int relu,
+                                 long long scene_rows, unsigned seed, float drop_p, void* stream);
+int s4g_train_bn_bwd_reduce_chdrop_bf16(const void* dz, const void* y, const float* scale, const float* shift, long long P,
+                                        int C, int relu, long long scene_rows, unsigned seed, float drop_p, double* sums2c,
+                                        void* stream);
+int s4g_train_bn_bwd_apply_chdrop_bf16(const void* dz, const void* y, const float* scale, const float* shift, const float* ka,
+                                       const float* kb, const float* kc, long long P, int C, int relu, long long scene_rows,
+                                       unsigned seed, float drop_p, void* dy, void* stream);
 /* The backward of a broadcast propagation level (num_fp_neighbours = 0, modules.py:131-134 expand) for its global input:
  * out[b][c] += sum_n dz[b*Nq + n][c] for c < C2 (dz rows ld wide, bf16; out fp32 [B][C2]).  Fixed summation order, no
  * atomics: the same bits on every run. */
@@ -308,6 +323,14 @@ int s4g_broadcast_concat_bf16(const void* sparse, const void* dense, int B, int 
  *   self (frames == NULL): R (B, 9, N), t (B, 3, N) fp32 head outputs, F = N, S = 1. */
 int s4g_local_eval_rows_bf16(const void* feat, int B, int N, int C, float* frames, const float* points, int F, int S,
                              const float* R, const float* t, void* out, void* stream);
+/* Its transpose (csrc/train_ops.cu), for the training step: d rows [B*F*S][C + 48] bf16 ->
+ *   dfeat [B*N][C] bf16: row b*N + f = the sum of the first C columns of rows (b, f, 0..S-1), accumulated in fp32 in
+ *     that order and rounded once; rows f >= F are zero;
+ *   self mode only (dR, dt != NULL; F = N, S = 1): dR (B, 9, N) and dt (B, 3, N) fp32 += the sum over the 4 repeats of
+ *     columns C..C+47 (the leaf gradients of the R and t logits the rows were written from).
+ * No float atomics, 64-bit offsets (row buffers over 2 GiB); rows 16-byte aligned. */
+int s4g_local_eval_rows_bwd_bf16(const void* d, int B, int N, int C, int F, int S, void* dfeat, float* dR, float* dt,
+                                 void* stream);
 
 /* Fused shared-MLP chain on tcgen05 tensor cores (csrc/mlp_chain.cu): replaces
  * SharedMLP / Conv1d / Conv2d (nn_utils/mlp.py:95-106, nn_utils/conv.py:30-36,70-76) with eval-mode

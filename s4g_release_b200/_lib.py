@@ -81,6 +81,11 @@ _SIGNATURES = {
     "s4g_train_bn_bwd_reduce_seg_bf16": ([_vp, _vp, _ll, _vp, _vp, _vp, _ll, _i, _i, _vp, _vp], _i),
     "s4g_train_bn_bwd_apply_seg_bf16": ([_vp, _vp, _ll, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _i, _i, _vp, _vp], _i),
     "s4g_train_rows_segment_sum_bf16": ([_vp, _ll, _i, _ll, _i, _vp, _vp], _i),
+    "s4g_train_bn_act_chdrop_bf16": ([_vp, _vp, _vp, _vp, _ll, _i, _i, _ll, ctypes.c_uint, _f, _vp], _i),
+    "s4g_train_bn_bwd_reduce_chdrop_bf16": ([_vp, _vp, _vp, _vp, _ll, _i, _i, _ll, ctypes.c_uint, _f, _vp, _vp], _i),
+    "s4g_train_bn_bwd_apply_chdrop_bf16": ([_vp, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _i, _i, _ll, ctypes.c_uint, _f, _vp, _vp],
+                                           _i),
+    "s4g_local_eval_rows_bwd_bf16": ([_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp], _i),
     "s4g_train_group_rows_bf16":([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp], _i),
     "s4g_train_group_rows_bwd": ([_vp, _ll, _vp, _i, _i, _i, _i, _i, _vp, _vp], _i),
     "s4g_train_interp_rows_bwd": ([_vp, _ll, _vp, _vp, _i, _i, _i, _i, _vp, _vp], _i),

@@ -138,6 +138,44 @@ bn_act_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict__ sca
   }
 }
 
+// the same with channel dropout (F.dropout2d): one keep decision per (scene, channel), scene = row / scene_rows — the
+// element hash evaluated at row = scene, so every row of a scene shares it (rows < 2^31: one 32-bit division per row)
+__global__ void __launch_bounds__(256)
+bn_act_chdrop_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict__ scale, const float* __restrict__ shift,
+                     __nv_bfloat16* __restrict__ z, long long P, int C, int relu, unsigned seed, unsigned thresh,
+                     float keep_scale, unsigned scene_rows) {
+  const int pieces = C >> 3;
+  const int lanes = 256 / pieces;
+  const int piece = threadIdx.x % pieces, rl = threadIdx.x / pieces;
+  if (rl >= lanes) return;
+  const long long r1 = min(P, ((long long)blockIdx.x + 1) * kEltRows);
+  const F8 a = load_f8(scale + piece * 8), b = load_f8(shift + piece * 8);
+  for (long long r = (long long)blockIdx.x * kEltRows + rl; r < r1; r += 4LL * lanes) {
+    uint4 raw[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const long long rr = r + (long long)u * lanes;
+      if (rr < r1) raw[u] = __ldg(reinterpret_cast<const uint4*>(y + rr * C) + piece);
+    }
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const long long rr = r + (long long)u * lanes;
+      if (rr >= r1) break;
+      const F8 v = unpack8(raw[u]);
+      const long long scene = (unsigned)rr / scene_rows;
+      F8 o;
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        float t = fmaf(v.v[e], a.v[e], b.v[e]);
+        if (relu) t = fmaxf(t, 0.f);
+        if (thresh) t = keep_elem(seed, scene, piece * 8 + e, C, thresh) ? t * keep_scale : 0.f;
+        o.v[e] = t;
+      }
+      reinterpret_cast<uint4*>(z + rr * C)[piece] = pack8(o);
+    }
+  }
+}
+
 __global__ void __launch_bounds__(256)
 bn_act_maxpool_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict__ scale, const float* __restrict__ shift,
                       __nv_bfloat16* __restrict__ out, uint8_t* __restrict__ arg, __nv_bfloat16* __restrict__ ymax, long long G,
@@ -326,7 +364,7 @@ rows_segment_sum_kernel(const __nv_bfloat16* __restrict__ dz, long long ld, long
 struct Upstream {
   const __nv_bfloat16* dz;   // dense: [P][C];   pooled: [G][C]
   const uint8_t* arg;        // pooled only: [G][C]
-  int K;                     // 0 = dense
+  int K;                     // 0 = dense;  kUpChanDrop (dense): the rows of one scene
   int kshift;                // log2 K when K is a power of two (every shipped configuration), else -1
   const int* arg32;          // pooled with int32 arg-max rows (the groups of a global level: K = the scene's N rows)
 };
@@ -396,12 +434,29 @@ __device__ __forceinline__ UpRaw upstream_load32(const Upstream& u, long long ro
   r.k = -1;
   return r;
 }
-// the upstream kinds the BatchNorm-backward kernels are compiled for
-enum { kUpDenseOrArg8 = 0, kUpArg32 = 1 };
+// the upstream kinds the BatchNorm-backward kernels are compiled for; kUpChanDrop: dense, with channel dropout (one keep
+// decision per (scene, channel), scene = row / u.K) in place of element dropout
+enum { kUpDenseOrArg8 = 0, kUpArg32 = 1, kUpChanDrop = 2 };
 template <int UP>
 __device__ __forceinline__ UpRaw upstream_load_k(const Upstream& u, long long row, int piece, int C) {
-  if constexpr (UP == kUpArg32) return upstream_load32(u, row, piece, C);
-  else return upstream_load(u, row, piece, C);
+  if constexpr (UP == kUpArg32) {
+    return upstream_load32(u, row, piece, C);
+  } else if constexpr (UP == kUpChanDrop) {
+    UpRaw r;
+    r.d = __ldg(reinterpret_cast<const uint4*>(u.dz + row * C) + piece);
+    r.a = make_uint2(0u, 0u);
+    r.k = -1;
+    return r;
+  } else {
+    return upstream_load(u, row, piece, C);
+  }
+}
+// the row the dropout hash is evaluated at: the row itself, or for channel dropout its scene (rows < 2^31, checked by
+// the host: one 32-bit division per row)
+template <int UP>
+__device__ __forceinline__ long long drop_row(const Upstream& u, long long row) {
+  if constexpr (UP == kUpChanDrop) return (long long)((unsigned)row / (unsigned)u.K);
+  else return row;
 }
 
 // sums = [sum_r g | sum_r g * y]; the caller turns the second into sum g * xhat = rstd * (sum g y - mean * sum g) in fp64
@@ -437,11 +492,12 @@ bn_bwd_reduce_kernel(Upstream up, const __nv_bfloat16* __restrict__ y, const flo
         if (rr >= r1) break;
         const F8 v = unpack8(raw[u]);
         const F8 d = upstream_route(ur[u]);
+        const long long dr = drop_row<UP>(up, rr);
 #pragma unroll
         for (int e = 0; e < 8; ++e) {
           float g = d.v[e];
           if (relu && !(fmaf(v.v[e], a.v[e], b.v[e]) > 0.f)) g = 0.f;
-          if (thresh) g = keep_elem(seed, rr, piece * 8 + e, C, thresh) ? g * keep_scale : 0.f;
+          if (thresh) g = keep_elem(seed, dr, piece * 8 + e, C, thresh) ? g * keep_scale : 0.f;
           s.v[e] += g;
           q.v[e] = fmaf(g, v.v[e], q.v[e]);
         }
@@ -610,12 +666,13 @@ bn_bwd_apply_kernel(Upstream up, const __nv_bfloat16* __restrict__ y, const floa
       if (rr >= r1) break;
       const F8 v = unpack8(raw[u]);
       const F8 d = upstream_route(ur[u]);
+      const long long dr = drop_row<UP>(up, rr);
       F8 o;
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
         float g = d.v[e];
         if (relu && !(fmaf(v.v[e], a.v[e], b.v[e]) > 0.f)) g = 0.f;
-        if (thresh) g = keep_elem(seed, rr, piece * 8 + e, C, thresh) ? g * keep_scale : 0.f;
+        if (thresh) g = keep_elem(seed, dr, piece * 8 + e, C, thresh) ? g * keep_scale : 0.f;
         o.v[e] = fmaf(A.v[e], g, fmaf(Bc.v[e], v.v[e], Cc.v[e]));
       }
       reinterpret_cast<uint4*>(dy + rr * C)[piece] = pack8(o);
@@ -705,12 +762,13 @@ bn_bwd_apply_staged_kernel(Upstream up, const __nv_bfloat16* __restrict__ y, con
         if (rr >= rows) break;
         const F8 v = unpack8(yr[u]);
         const F8 d = upstream_route(ur[u]);
+        const long long dr = drop_row<UP>(up, row0 + rr);
         F8 o;
 #pragma unroll
         for (int e = 0; e < 8; ++e) {
           float g = d.v[e];
           if (relu && !(fmaf(v.v[e], a.v[e], b.v[e]) > 0.f)) g = 0.f;
-          if (DROP) g = keep_elem(seed, row0 + rr, piece * 8 + e, C, thresh) ? g * keep_scale : 0.f;
+          if (DROP) g = keep_elem(seed, dr, piece * 8 + e, C, thresh) ? g * keep_scale : 0.f;
           o.v[e] = fmaf(A.v[e], g, fmaf(Bc.v[e], v.v[e], Cc.v[e]));
         }
         reinterpret_cast<uint4*>(dy + (row0 + rr) * C)[piece] = pack8(o);
@@ -1120,6 +1178,63 @@ head_logits_dw_kernel(const float* __restrict__ dl, const __nv_bfloat16* __restr
   }
 }
 
+// ---------------------------------------------------------------------------------------------- evaluation rows backward
+// The transpose of local_eval_rows_kernel (csrc/fused_ops.cu): d rows [B*F*S][C + 48] ->
+//   point features  dfeat[b*N + f] = sum_s d[(b, f, s)][0..C), s = 0, 1, ... in fp32, one rounding to bf16; 0 for f >= F.
+//                   Thread = (scene, point, 16-byte piece); a warp reads whole 16-byte pieces of two or more rows.
+//   candidates      (self mode: F = N, S = 1) dR[b][k][n] += sum_r d[(b, n)][C + 12 r + k] (k < 9), dt likewise with
+//                   k = 9..11: r = 0..3 in order, fp32, one plain add per output (each thread owns its point).
+// grid.x = the point-feature blocks, then (self mode) the candidate blocks; grid.y = scene.  No atomics, 64-bit offsets.
+constexpr int kEvalBwdU = 4;  // rows in flight per thread
+
+__global__ void __launch_bounds__(256)
+local_eval_rows_bwd_kernel(const __nv_bfloat16* __restrict__ d, int N, int C, int F, int S, unsigned feat_blocks,
+                           __nv_bfloat16* __restrict__ dfeat, float* __restrict__ dR, float* __restrict__ dt) {
+  const long long b = blockIdx.y;
+  const long long W = C + 48;
+  if (blockIdx.x < feat_blocks) {
+    const int pieces = C >> 3;
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= N * pieces) return;
+    const int n = i / pieces, piece = i - n * pieces;
+    F8 acc{};
+    if (n < F) {
+      const __nv_bfloat16* src = d + (b * F + n) * (long long)S * W + piece * 8;
+      for (int s0 = 0; s0 < S; s0 += kEvalBwdU) {
+        uint4 raw[kEvalBwdU];
+#pragma unroll
+        for (int u = 0; u < kEvalBwdU; ++u)
+          if (s0 + u < S) raw[u] = __ldg(reinterpret_cast<const uint4*>(src + (long long)(s0 + u) * W));
+#pragma unroll
+        for (int u = 0; u < kEvalBwdU; ++u) {
+          if (s0 + u >= S) break;
+          const F8 v = unpack8(raw[u]);
+#pragma unroll
+          for (int e = 0; e < 8; ++e) acc.v[e] += v.v[e];
+        }
+      }
+    }
+    reinterpret_cast<uint4*>(dfeat + (b * N + n) * C)[piece] = pack8(acc);
+    return;
+  }
+  const int n = (blockIdx.x - feat_blocks) * 256 + threadIdx.x;
+  if (n >= N) return;
+  const uint4* src = reinterpret_cast<const uint4*>(d + (b * N + n) * W + C);
+  float v[48];
+#pragma unroll
+  for (int q = 0; q < 6; ++q) {
+    const F8 f = unpack8(__ldg(src + q));
+#pragma unroll
+    for (int e = 0; e < 8; ++e) v[q * 8 + e] = f.v[e];
+  }
+#pragma unroll
+  for (int k = 0; k < 12; ++k) {
+    const float s = ((v[k] + v[12 + k]) + v[24 + k]) + v[36 + k];
+    float* o = k < 9 ? dR + (b * 9 + k) * N + n : dt + (b * 3 + k - 9) * N + n;
+    *o += s;
+  }
+}
+
 static unsigned grid_for(long long work, int threads) { return (unsigned)((work + threads - 1) / threads); }
 
 }  // namespace trn
@@ -1287,6 +1402,89 @@ extern "C" int s4g_train_bn_bwd_apply_seg_bf16(const void* dz, const int* arg, l
                 "train_bn_bwd_apply_seg: bad arguments");
   TRN_CHECK_C(C);
   return bn_bwd_apply(make_upstream(dz, nullptr, (int)N, arg), y, scale, shift, ka, kb, kc, P, C, relu, 0u, 0.f, dy, stream);
+}
+
+// channel dropout: rows [P][C] of P / scene_rows scenes; one keep decision per (scene, channel).  The rows are read and
+// written as 16-byte pieces (and the apply pass stages them with bulk copies): 16-byte aligned
+#define TRN_CHECK_CHDROP(what, rows_or)                                                                                   \
+  S4G_CHECK_ARG(P > 0 && P < (1ll << 31) && scene_rows > 0 && P % scene_rows == 0 && drop_p >= 0.f && drop_p < 1.f,   \
+                what ": bad arguments (rows < 2^31 in whole scenes, 0 <= drop_p < 1)");                                 \
+  S4G_CHECK_ARG(((uintptr_t)(rows_or) & 15) == 0, what ": rows must be 16-byte aligned")
+
+extern "C" int s4g_train_bn_act_chdrop_bf16(const void* y, const float* scale, const float* shift, void* z, long long P, int C,
+                                            int relu, long long scene_rows, unsigned seed, float drop_p, void* stream) {
+  S4G_CHECK_ARG(y && scale && shift && z, "train_bn_act_chdrop: null pointer");
+  TRN_CHECK_CHDROP("train_bn_act_chdrop", (uintptr_t)y | (uintptr_t)z);
+  TRN_CHECK_C(C);
+  const unsigned thresh = drop_p > 0.f ? (unsigned)((double)drop_p * 4294967296.0) : 0u;
+  bn_act_chdrop_kernel<<<grid_for(P, kEltRows), 256, 0, (cudaStream_t)stream>>>(
+      reinterpret_cast<const bf16*>(y), scale, shift, reinterpret_cast<bf16*>(z), P, C, relu, seed, thresh,
+      1.f / (1.f - drop_p), (unsigned)scene_rows);
+  S4G_LAUNCH_CHECK("train_bn_act_chdrop");
+  return S4G_OK;
+}
+
+extern "C" int s4g_train_bn_bwd_reduce_chdrop_bf16(const void* dz, const void* y, const float* scale, const float* shift,
+                                                   long long P, int C, int relu, long long scene_rows, unsigned seed,
+                                                   float drop_p, double* sums2c, void* stream) {
+  S4G_CHECK_ARG(dz && y && scale && shift && sums2c, "train_bn_bwd_reduce_chdrop: null pointer");
+  TRN_CHECK_CHDROP("train_bn_bwd_reduce_chdrop", (uintptr_t)dz | (uintptr_t)y);
+  TRN_CHECK_C(C);
+  cudaStream_t s = (cudaStream_t)stream;
+  S4G_CUDA(cudaMemsetAsync(sums2c, 0, sizeof(double) * 2 * C, s));
+  const int pieces = C >> 3, lanes = kStatThreads / pieces;
+  S4G_CHECK_ARG(lanes >= 1, "train_bn_bwd_reduce_chdrop: too many channels");
+  const unsigned thresh = drop_p > 0.f ? (unsigned)((double)drop_p * 4294967296.0) : 0u;
+  const Upstream up{reinterpret_cast<const bf16*>(dz), nullptr, (int)scene_rows, -1, nullptr};
+  const size_t sm = (size_t)lanes * pieces * 16 * sizeof(float);
+  bn_bwd_reduce_kernel<4, 2, kUpChanDrop><<<grid_for(P, kStatRows), kStatThreads, sm, s>>>(
+      up, reinterpret_cast<const bf16*>(y), scale, shift, P, C, relu, seed, thresh, 1.f / (1.f - drop_p), sums2c);
+  S4G_LAUNCH_CHECK("train_bn_bwd_reduce_chdrop");
+  return S4G_OK;
+}
+
+extern "C" int s4g_train_bn_bwd_apply_chdrop_bf16(const void* dz, const void* y, const float* scale, const float* shift,
+                                                  const float* ka, const float* kb, const float* kc, long long P, int C,
+                                                  int relu, long long scene_rows, unsigned seed, float drop_p, void* dy,
+                                                  void* stream) {
+  S4G_CHECK_ARG(dz && y && scale && shift && ka && kb && kc && dy, "train_bn_bwd_apply_chdrop: null pointer");
+  TRN_CHECK_CHDROP("train_bn_bwd_apply_chdrop", (uintptr_t)dz | (uintptr_t)y | (uintptr_t)dy);
+  TRN_CHECK_C(C);
+  const unsigned thresh = drop_p > 0.f ? (unsigned)((double)drop_p * 4294967296.0) : 0u;
+  const float ks = 1.f / (1.f - drop_p);
+  const Upstream up{reinterpret_cast<const bf16*>(dz), nullptr, (int)scene_rows, -1, nullptr};
+  // rows staged by the copy engine, as bn_bwd_apply's dense passes
+  constexpr int kRpl = 4, kStages = 3, kCons = 480;
+  auto kernel = bn_bwd_apply_staged_kernel<kRpl, kStages, kCons, true, true, kUpChanDrop>;
+  const int pieces = C >> 3, lanes_s = kCons / pieces;
+  const int R = kRpl * lanes_s;
+  const size_t smem = (size_t)kStages * 2 * R * C * 2;
+  static bool attr[64] = {};
+  if (s4g::first_use_on_device(attr))
+    S4G_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  const long long n_tiles = (P + R - 1) / R;
+  const int sms = s4g::num_sms();
+  kernel<<<(unsigned)(n_tiles < sms ? n_tiles : sms), kCons + 32, smem, (cudaStream_t)stream>>>(
+      up, reinterpret_cast<const bf16*>(y), scale, shift, ka, kb, kc, P, C, relu, seed, thresh, ks, reinterpret_cast<bf16*>(dy));
+  S4G_LAUNCH_CHECK("train_bn_bwd_apply_chdrop");
+  return S4G_OK;
+}
+#undef TRN_CHECK_CHDROP
+
+extern "C" int s4g_local_eval_rows_bwd_bf16(const void* d, int B, int N, int C, int F, int S, void* dfeat, float* dR, float* dt,
+                                            void* stream) {
+  S4G_CHECK_ARG(d && dfeat && (dR == nullptr) == (dt == nullptr), "local_eval_rows_bwd: null pointer (dR and dt go together)");
+  S4G_CHECK_ARG(B > 0 && B <= 65535 && N > 0 && C > 0 && C % 8 == 0 && 1 <= F && F <= N && S >= 1 &&
+                    (long long)N * (C >> 3) < (1ll << 31),
+                "local_eval_rows_bwd: bad shape (C %% 8 == 0, 1 <= F <= N, S >= 1)");
+  S4G_CHECK_ARG(!dR || (F == N && S == 1), "local_eval_rows_bwd: the candidate gradient needs self mode (F = N, S = 1)");
+  S4G_CHECK_ARG((((uintptr_t)d | (uintptr_t)dfeat) & 15) == 0, "local_eval_rows_bwd: rows must be 16-byte aligned");
+  const unsigned feat_blocks = grid_for((long long)N * (C >> 3), 256);
+  const dim3 grid(feat_blocks + (dR ? grid_for(N, 256) : 0u), (unsigned)B);
+  local_eval_rows_bwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const bf16*>(d), N, C, F, S, feat_blocks,
+                                                                      reinterpret_cast<bf16*>(dfeat), dR, dt);
+  S4G_LAUNCH_CHECK("local_eval_rows_bwd");
+  return S4G_OK;
 }
 
 extern "C" int s4g_train_bn_act_segmax_bf16(const void* y, const float* scale, const float* shift, void* out, int* arg,

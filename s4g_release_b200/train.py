@@ -67,17 +67,51 @@ def synthetic_labels(batch, num_points, num_frame=4000, first_seed=2000, device=
     return {k: torch.from_numpy(np.stack(v)).to(device) for k, v in out.items()}
 
 
+def synthetic_local_batch(points, num_frames, num_search, score_classes=3, first_seed=3000):
+    """PN2_LOCAL's given candidates and labels for the scenes ``points`` (B, 3, N), seeded per scene -> (frames, labels)
+    on the points' device:
+      frames  ``local_search_frame`` (B, 12, F, S) float32: random rotations (row-major 9) and translations within a few
+              cm of their point (point f of the scene, f < F);
+      labels  of PointNet2_local.PointNet2Loss: scored_grasp_labels (B, F, S) int64 in [0, score_classes),
+              scene_movable_labels (B, N) int64 in {0, 1}, best_frame_R (B, 9, F) rotations, best_frame_t (B, 3, F) float32
+              near the points (the layout of tests/golden/pn2_local.npz).
+    Self mode (no given candidates) evaluates F = N points with S = 1 candidate each: pass those and drop the frames."""
+    B, _, N = points.shape
+    if not (1 <= num_frames <= N and num_search >= 1):
+        raise ValueError("synthetic_local_batch needs 1 <= num_frames <= %d and num_search >= 1" % N)
+    F, S = num_frames, num_search
+    pts = points.detach().float().cpu().numpy()
+    frames = []
+    out = {k: [] for k in ("scored_grasp_labels", "scene_movable_labels", "best_frame_R", "best_frame_t")}
+    for i in range(B):
+        rs = np.random.RandomState(first_seed + i)
+        anchor = pts[i, :, :F]
+        q, _ = np.linalg.qr(rs.randn(F * S, 3, 3))
+        t = anchor[:, :, None] + 0.02 * rs.randn(3, F, S)
+        frames.append(np.concatenate([q.reshape(F, S, 9).transpose(2, 0, 1), t]).astype(np.float32))
+        out["scored_grasp_labels"].append(rs.randint(0, score_classes, size=(F, S)).astype(np.int64))
+        out["scene_movable_labels"].append(rs.randint(0, 2, size=N).astype(np.int64))
+        q, _ = np.linalg.qr(rs.randn(F, 3, 3))
+        out["best_frame_R"].append(q.reshape(F, 9).T.astype(np.float32))
+        out["best_frame_t"].append((anchor + 0.02 * rs.randn(3, F)).astype(np.float32))
+    dev = points.device
+    return (torch.from_numpy(np.stack(frames)).to(dev),
+            {k: torch.from_numpy(np.stack(v)).to(dev) for k, v in out.items()})
+
+
 class Trainer:
     def __init__(self, model, loss_fn, lr=1e-3, betas=(0.9, 0.999), weight_decay=0.0, step_size=20, gamma=0.5,
                  group=None, fused=False):
         """``fused``: forward + loss + backward on the B200-native training kernels (train_engine.TrainEngine: tcgen05
         GEMMs over bf16 rows, fused BatchNorm / ReLU / max-pool passes) instead of the module path under torch autograd —
-        PN2_CLS or the PN2 sibling with its own PointNet2Loss, including a global last level (TrainEngine's guard)."""
+        PN2_CLS, the PN2 sibling or PN2_LOCAL (train_engine.LocalTrainEngine, picked from the model's class) with its
+        own PointNet2Loss, including a global last level (TrainEngine's guard).  PN2_LOCAL's given candidates
+        (``data_batch["local_search_frame"]``) are updated in place by each step, as by the module path's forward."""
         self.model, self.loss_fn, self.group = model, loss_fn, group
         self.engine = None
         if fused:
-            from .train_engine import TrainEngine
-            self.engine = TrainEngine(model, loss_fn)
+            from .train_engine import engine_for
+            self.engine = engine_for(model, loss_fn)
         broadcast_parameters(model, 0, group)
         self.bucket = GradBucket(model.parameters())
         self.optimizer = torch.optim.Adam(self.bucket.params, lr=lr, betas=betas, weight_decay=weight_decay)

@@ -26,7 +26,7 @@ Activations are bf16, so this is the numerical regime of bf16 autocast training,
 import torch
 
 from ._lib import check, lib, ptr, stream_ptr
-from .engine import FusedPointNet2
+from .engine import FusedPointNet2, FusedPointNet2Local, check_local_frames
 
 BF16 = torch.bfloat16
 
@@ -102,12 +102,16 @@ def colstats(y):
 class Block:
     """One conv (bias-free 1x1) + BatchNorm + ReLU block of a SharedMLP in training mode, on rows.
     ``in_perm``: for the first block of a set-abstraction level, the number of gathered feature channels Cf — the input
-    rows are [features(Cf) | xyz(3) | 0 x 5] while the reference's weight columns are [xyz(3) | features(Cf)]."""
+    rows are [features(Cf) | xyz(3) | 0 x 5] while the reference's weight columns are [xyz(3) | features(Cf)].
+    ``channel_drop``: dropout with one keep decision per (scene, channel), F.dropout2d of a SharedMLP(ndim=2), instead of
+    per element; the caller sets ``scene_rows`` (the rows of one scene) before each forward."""
 
-    def __init__(self, module, grouped_cf=None, drop_p=0.0):
+    def __init__(self, module, grouped_cf=None, drop_p=0.0, channel_drop=False):
         self.conv, self.bn = module.conv, module.bn
         self.cf = grouped_cf
         self.drop_p = float(drop_p)
+        self.channel_drop = bool(channel_drop)
+        self.scene_rows = 0
         self.cout = self.conv.weight.shape[0]
         self.cin = self.conv.weight.shape[1]
         self.saved = None
@@ -177,6 +181,11 @@ class Block:
             check(lib.s4g_train_bn_act_maxpool_bf16(ptr(y), ptr(scale), ptr(shift), ptr(z), ptr(arg),
                                                     ptr(ymax) if ymax is not None else None, G, pool_k, self.cout, 1,
                                                     stream_ptr(dev)), "train_bn_act_maxpool")
+        elif self.channel_drop:
+            arg = ymax = None
+            z = torch.empty((P, self.cout), dtype=BF16, device=dev)
+            check(lib.s4g_train_bn_act_chdrop_bf16(ptr(y), ptr(scale), ptr(shift), ptr(z), P, self.cout, 1, self.scene_rows,
+                                                   seed, self.drop_p, stream_ptr(dev)), "train_bn_act_chdrop")
         else:
             arg = ymax = None
             z = torch.empty((P, self.cout), dtype=BF16, device=dev)
@@ -212,6 +221,10 @@ class Block:
             elif arg is not None and arg.dtype == torch.int32:  # global pool: dz routed to row arg of its scene
                 check(lib.s4g_train_bn_bwd_reduce_seg_bf16(ptr(dz), ptr(arg), pool_k, ptr(y), ptr(scale), ptr(shift), P, C,
                                                            1, ptr(sums), stream_ptr(dev)), "train_bn_bwd_reduce_seg")
+            elif self.channel_drop:
+                check(lib.s4g_train_bn_bwd_reduce_chdrop_bf16(ptr(dz), ptr(y), ptr(scale), ptr(shift), P, C, 1,
+                                                              self.scene_rows, seed, drop, ptr(sums), stream_ptr(dev)),
+                      "train_bn_bwd_reduce_chdrop")
             else:
                 check(lib.s4g_train_bn_bwd_reduce_bf16(ptr(dz), ptr(arg) if pool_k else None, pool_k, ptr(y), ptr(scale),
                                                        ptr(shift), P, C, 1, seed, drop, ptr(sums), stream_ptr(dev)),
@@ -226,6 +239,10 @@ class Block:
             check(lib.s4g_train_bn_bwd_apply_seg_bf16(ptr(dz), ptr(arg), pool_k, ptr(y), ptr(scale), ptr(shift), ptr(coef),
                                                       ptr(coef[C:]), ptr(coef[2 * C:]), P, C, relu, ptr(dy), stream_ptr(dev)),
                   "train_bn_bwd_apply_seg")
+        elif self.channel_drop:
+            check(lib.s4g_train_bn_bwd_apply_chdrop_bf16(ptr(dz), ptr(y), ptr(scale), ptr(shift), ptr(coef), ptr(coef[C:]),
+                                                         ptr(coef[2 * C:]), P, C, relu, self.scene_rows, seed, drop, ptr(dy),
+                                                         stream_ptr(dev)), "train_bn_bwd_apply_chdrop")
         else:
             check(lib.s4g_train_bn_bwd_apply_bf16(ptr(dz), ptr(arg) if pool_k else None, pool_k, ptr(y), ptr(scale),
                                                   ptr(shift), ptr(coef), ptr(coef[C:]), ptr(coef[2 * C:]), P, C, relu, seed,
@@ -255,7 +272,8 @@ def chain_backward(blocks, dz, need_dx=True):
     """backward through the blocks of one shared MLP, last to first; returns the gradient of the chain's input rows"""
     pre = None
     for j in reversed(range(len(blocks))):
-        prev = blocks[j - 1] if (j > 0 and FUSED_BWD_REDUCE) else None
+        # (a channel-dropout block keeps its separate reduce: the fused epilogue knows element dropout only)
+        prev = blocks[j - 1] if (j > 0 and FUSED_BWD_REDUCE and not getattr(blocks[j - 1], "channel_drop", False)) else None
         out = blocks[j].backward(dz, need_dx=(j > 0 or need_dx), prev=prev, pre=pre)
         dz, pre = out if prev is not None else (out, None)
     return dz  # ((d y, x rows, weights) when the first block was built from pre-activations: Block.forward_pre)
@@ -357,6 +375,8 @@ class TrainEngine:
     def __init__(self, model, loss_fn, seed=0):
         if not _has_training_plan(model):
             raise RuntimeError("TrainEngine: no fused plan for this configuration (PointNet2.fusable)")
+        if type(self) is TrainEngine and _is_local(model):
+            raise TypeError("TrainEngine: PN2_LOCAL trains on LocalTrainEngine (train_engine.engine_for picks it)")
         self.model, self.loss_fn = model, loss_fn
         self.cfg = model.config
         # a last level with one global group (num_centroids = 0) and the broadcast first propagation level it pairs with
@@ -372,8 +392,12 @@ class TrainEngine:
             self.sa.append(blocks)
             cf = blocks[-1].cout
         self.fp = [[Block(b) for b in m.mlp] for m in model.fp_modules]
-        p = self.cfg["dropout_prob"]
-        self.heads = [([Block(b, drop_p=dp) for b in mlp], logit) for mlp, logit, dp in (
+        self.heads = self._make_heads(model, self.cfg["dropout_prob"])
+
+    @staticmethod
+    def _make_heads(model, p):
+        """[(blocks, final conv)] of the heads, in the order of PRED_KEYS"""
+        return [([Block(b, drop_p=dp) for b in mlp], logit) for mlp, logit, dp in (
             (model.mlp_seg, model.seg_logit, p), (model.mlp_R, model.R_logit, 0.0), (model.mlp_t, model.t_logit, 0.0),
             (model.mlp_movable, model.movable_logit[0], p))]
 
@@ -460,16 +484,19 @@ class TrainEngine:
         self._points = points
         return sparse
 
-    def _head_forward(self, k, point_feat):
-        """head k: 4 blocks + the biased 1x1 conv -> fp32 logits (B, c, N), an autograd LEAF (the loss runs in torch)"""
+    def _head_forward(self, k, point_feat, positions=None):
+        """head k: 4 blocks + the biased 1x1 conv -> fp32 logits (B, c, N), an autograd LEAF (the loss runs in torch).
+        ``positions``: the trailing shape of the logits when the input rows are not the N points of each scene."""
         blocks, logit = self.heads[k]
         h = point_feat
         for j, blk in enumerate(blocks):
             h = blk.forward(h, seed=self._seed(10 * k + j))
-        B, n = self._batch, self._n_points
+        B = self._batch
+        positions = tuple(positions) if positions is not None else (self._n_points,)
+        n = h.shape[0] // B
         c = logit.weight.shape[0]
         w = logit.weight.detach().reshape(c, -1).contiguous()
-        out = torch.empty((B, c, n), dtype=torch.float32, device=h.device)
+        out = torch.empty((B, c) + positions, dtype=torch.float32, device=h.device)
         check(lib.s4g_train_head_logits_fwd(ptr(h), ptr(w), ptr(logit.bias), ptr(out), h.shape[0], h.shape[1], c, n,
                                             stream_ptr(h.device)), "train_head_logits_fwd")
         self._head_saved[k] = (h, w)
@@ -480,7 +507,8 @@ class TrainEngine:
         blocks, logit = self.heads[k]
         h, w = self._head_saved.pop(k)
         dl = leaf.grad
-        B, c, n = dl.shape
+        B, c = dl.shape[:2]
+        n = h.shape[0] // B
         dz = torch.empty_like(h)
         check(lib.s4g_train_head_logits_bwd(ptr(dl), ptr(w), ptr(dz), h.shape[0], h.shape[1], c, n, stream_ptr(h.device)),
               "train_head_logits_bwd")
@@ -607,3 +635,123 @@ class TrainEngine:
                 del dzs
                 self._trunk_backward(d_out)
         return losses
+
+
+def _is_local(model):
+    from .network_models.models import PointNet2_local
+    return isinstance(model, PointNet2_local.PointNet2)
+
+
+def engine_for(model, loss_fn, seed=0):
+    """The training engine of the model's class: LocalTrainEngine for PN2_LOCAL, TrainEngine for PN2_CLS and the PN2
+    sibling."""
+    return (LocalTrainEngine if _is_local(model) else TrainEngine)(model, loss_fn, seed)
+
+
+class LocalTrainEngine(TrainEngine):
+    """PN2_LOCAL (models/PointNet2_local.py): the trunk of TrainEngine unchanged, its own head stage (as
+    engine.FusedPointNet2Local over FusedPointNet2).  Heads, in PRED_KEYS order: frame_R (9) and frame_t (3) without
+    dropout, movable (2) with element dropout, and the grasp-evaluation head over the rows [point feature | candidate
+    (R, t) x 4] of FusedPointNet2Local.local_eval_rows, logits (B, k, F, S).  Its SharedMLP(ndim=2) drops with
+    F.dropout2d (nn_utils/mlp.py:27): one keep decision per (scene, channel), shared by the scene's F * S rows, so its
+    blocks use channel dropout.  No sigmoid anywhere.
+
+    Given candidates (data_batch["local_search_frame"], checked by engine.check_local_frames before any GPU work): their
+    translations are made relative to their point IN PLACE, once per step, as one module-path forward does.  The loss
+    is then separable (cls <- evaluation, R <- frame_R, t <- frame_t, mov <- movable) and the heads run one after the
+    other.  Self mode (no candidates): each point's candidate is its own R and t logits, which the reference does not
+    detach (PointNet2_local.py forward_modules), so cls_loss reaches the R and t heads through the rows.  The step takes
+    the joint path; its backward runs the evaluation head first and adds the rows' candidate gradient into the R and t
+    logits' gradients before those heads run."""
+
+    PRED_KEYS = ("frame_R", "frame_t", "movable_logits", "local_search_logits")
+    LOSS_KEYS = ("R_loss", "t_loss", "mov_loss", "cls_loss")  # PointNet2_local.PointNet2Loss: term k <- head k
+    EVAL = 3
+
+    def __init__(self, model, loss_fn, seed=0):
+        super().__init__(model, loss_fn, seed)
+        self._frames = None
+
+    @staticmethod
+    def _make_heads(model, p):
+        return [([Block(b) for b in model.mlp_R], model.R_logit), ([Block(b) for b in model.mlp_t], model.t_logit),
+                ([Block(b, drop_p=p) for b in model.mlp_movable], model.movable_logit),
+                ([Block(b, drop_p=p, channel_drop=True) for b in model.mlp_grasp_eval], model.grasp_eval_logit)]
+
+    def _candidates(self):
+        """(F, S): candidate points per scene, candidates per point"""
+        fr = self._frames
+        return (fr.shape[2], fr.shape[3]) if fr is not None else (self._n_points, 1)
+
+    def _eval_forward(self, point_feat, R=None, t=None):
+        """the evaluation head -> logits (B, k, F, S), an autograd leaf; R, t: the self-mode candidates (B, 9 | 3, N)"""
+        F, S = self._candidates()
+        rows = FusedPointNet2Local.local_eval_rows(point_feat, self._points.float().contiguous(), self._frames, R, t)
+        for blk in self.heads[self.EVAL][0]:
+            blk.scene_rows = F * S
+        return super()._head_forward(self.EVAL, rows, positions=(F, S))
+
+    def _eval_backward(self, leaf, R=None, t=None):
+        """-> d(point features) [B*N, C] bf16; in self mode also adds the candidate gradient into R.grad and t.grad"""
+        d = super()._head_backward(self.EVAL, leaf)  # d rows [B*F*S, C + 48]
+        F, S = self._candidates()
+        B, N = self._batch, self._n_points
+        C = d.shape[1] - 48
+        dfeat = torch.empty((B * N, C), dtype=BF16, device=d.device)
+        dR, dt = (ptr(_grad_buffer(R)), ptr(_grad_buffer(t))) if R is not None else (None, None)
+        check(lib.s4g_local_eval_rows_bwd_bf16(ptr(d), B, N, C, F, S, ptr(dfeat), dR, dt, stream_ptr(d.device)),
+              "local_eval_rows_bwd")
+        return dfeat
+
+    def _head_forward(self, k, point_feat, positions=None):
+        if k == self.EVAL:  # (the separable step: given candidates)
+            return self._eval_forward(point_feat)
+        return super()._head_forward(k, point_feat, positions)
+
+    def _head_backward(self, k, leaf):
+        if k == self.EVAL:
+            return self._eval_backward(leaf)
+        return super()._head_backward(k, leaf)
+
+    def _predictions(self, leaves):
+        return self.model.predictions(dict(zip(self.PRED_KEYS, leaves)), self._points)
+
+    def _placeholder(self, k):
+        logit = self.heads[k][1]
+        positions = self._candidates() if k == self.EVAL else (self._n_points,)
+        return torch.zeros((self._batch, logit.weight.shape[0]) + tuple(positions), dtype=torch.float32,
+                           device=logit.weight.device)
+
+    def _separable(self):
+        from .network_models.models import PointNet2_local
+        return self.sequential_heads and self._frames is not None and type(self.loss_fn) is PointNet2_local.PointNet2Loss
+
+    def forward(self, points):
+        self._head_saved = {}
+        self._point_feat = self._trunk_forward(points)
+        leaves = [self._head_forward(k, self._point_feat) for k in range(3)]
+        cand = leaves[:2] if self._frames is None else (None, None)
+        leaves.append(self._eval_forward(self._point_feat, *cand))
+        self._head_leaves = leaves
+        return self._predictions(leaves)
+
+    def backward(self):
+        R, t, mov, ev = self._head_leaves
+        cand = (R, t) if self._frames is None else (None, None)
+        d_eval = self._eval_backward(ev, *cand)  # first: it adds to R.grad and t.grad in self mode
+        dzs = [self._head_backward(k, leaf) for k, leaf in enumerate((R, t, mov))] + [d_eval]
+        self._head_leaves = self._point_feat = None
+        self._trunk_backward(_sum_rows(dzs))
+
+    def step_loss(self, data_batch, labels):
+        """as TrainEngine.step_loss; ``data_batch["local_search_frame"]`` (optional): the given candidates, updated in
+        place"""
+        points = data_batch["scene_points"]
+        frames = data_batch["local_search_frame"] if "local_search_frame" in data_batch else None
+        if frames is not None:
+            check_local_frames(points, frames)
+        self._frames = frames
+        try:
+            return super().step_loss(data_batch, labels)
+        finally:
+            self._frames = None
