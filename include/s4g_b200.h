@@ -302,6 +302,11 @@ int s4g_interp_concat_act_bf16(const void* sparse, const int* index, const float
 /* gather_points for xyz with int32 indices (functions.py:10-25): (B,3,N),(B,M) -> (B,3,M). */
 int s4g_gather_xyz_f32_i32(const float* xyz, const int* index, int B, int N, int M, float* out, void* stream);
 
+/* gather_points for channel-last bf16 features (EdgeSAModule.forward's centroid features, modules.py:280-282):
+ * src [B*N][C] bf16, index (B,M) int32 in [0, N) -> out [B*M][C] bf16, out[b*M + m] = src[b*N + index[b][m]], bit-equal.
+ * C % 8 == 0, rows 16-byte aligned; 64-bit offsets (tables over 2 GiB). */
+int s4g_gather_rows_bf16(const void* src, const int* index, int B, int N, int M, int C, void* out, void* stream);
+
 /* The max over the neighbours of a GLOBAL set-abstraction level (num_centroids = 0: one group of all N points centred
  * at the origin, PointNetSAModule.forward, modules.py:93-98 + :106 torch.max(new_feature, 3)).  The fused path runs the
  * group through the gathered max-pool chain as P partial groups; this reduces the P partial rows of each scene:
@@ -338,7 +343,8 @@ int s4g_local_eval_rows_bwd_bf16(const void* d, int B, int N, int C, int F, int 
  * (pointnet2_utils/modules.py:208-244) or the final biased 1x1 conv (+sigmoid) of the heads
  * (models/PointNet2_tcls.py:126-148).
  *   in_mode : 0 = bf16 rows [P][stride];  1 = gathered set-abstraction input (feat_c feature channels
- *             + relative xyz; reference channel order [xyz | feat] is handled by the weight packer)
+ *             + relative xyz; reference channel order [xyz | feat] is handled by the weight packer);
+ *             6 = the same for an edge level, with a per-centroid term in layer 0 (s4g_chain_run_gather_term)
  *   out_mode: 2 = bf16 rows [P][out_c];  3 = max-pool over groups of `group` rows -> bf16 [P/group][out_c];
  *             4 = fp32 logits, channel-first (P/n_points, out_c, n_points), bias, optional sigmoid
  * Layer l computes relu?(W_l x + bias_l) with W_l (cout x cin, fp32, BN-folded) packed to bf16 by
@@ -392,8 +398,19 @@ int s4g_chain_set_params(s4g_chain* chain, const void* weights_dev, const float*
 int s4g_chain_set_xyz_layer(s4g_chain* chain, const float* w4_host, int relu);
 int s4g_chain_run_rows(const s4g_chain* chain, const void* in_rows, int in_stride, long long P, void* out,
                        int n_points, void* stream);
+/* Refuses chains created with in_mode 6 (edge chains, below). */
 int s4g_chain_run_gather(const s4g_chain* chain, const void* feat, const float* xyz, const float* ctr, const int* nbr,
                          int B, int N, int M, int K, void* out, void* stream);
+/* Edge set abstraction (EdgeSAModule, pointnet2_utils/modules.py:250-284, fed by EdgeQueryGrouper, :202-221): the MLP's
+ * first layer sees [x_j - x_c | f_j | f_j - f_c] (3 + 2C channels).  With its BN-folded weight split by those column
+ * groups, W' = [W_x | W_a | W_b], that layer is
+ *   [W_x | W_a + W_b] [x_j - x_c ; f_j] + b' + u_c,   u_c = -W_b f_c,
+ * i.e. a plain gathered layer over 3 + C channels plus a term of the centroid alone.  A chain created with in_mode 6
+ * (gathered max-pool, >= 2 layers, feat_c > 0, layer 0 = the 3 + C -> cout[0] weights [W_x | W_a + W_b]) adds
+ * term[b * M + m][c] (bf16 [B*M][cout[0]], 16-byte aligned) to layer 0's shift, in fp32, for every row of centroid m's
+ * group, before the ReLU and the bf16 rounding.  Refuses every other chain. */
+int s4g_chain_run_gather_term(const s4g_chain* chain, const void* feat, const float* xyz, const float* ctr, const int* nbr,
+                              const void* term, int B, int N, int M, int K, void* out, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Device-side cloud pre-processing (csrc/preprocess.cu) — GraspDetector._pre_processing / sample_single_cloud

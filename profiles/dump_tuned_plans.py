@@ -12,7 +12,12 @@ from bench import seeded_model  # noqa: E402
 from s4g_release_b200 import engine  # noqa: E402
 
 t0 = time.time()
-eng = engine.FusedPointNet2(seeded_model().cuda(), autotune="force")
+if "--edge" in sys.argv:  # the chains of EDGEPN2D at its default arguments (the table keeps its two edge chains, in_mode 6)
+    from bench_global import seeded  # noqa: E402
+    from s4g_release_b200.network_models.models.EdgePointNet2Down import EdgePointNet2Down  # noqa: E402
+    eng = engine.FusedEdgePointNet2Down(seeded(EdgePointNet2Down).cuda(), autotune="force")
+else:
+    eng = engine.FusedPointNet2(seeded_model().cuda(), autotune="force")
 torch.cuda.synchronize()
 out = engine.export_tuned_plans()
 out["_seconds"] = round(time.time() - t0, 2)

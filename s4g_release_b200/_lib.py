@@ -58,6 +58,7 @@ _SIGNATURES = {
     "s4g_interp_concat_bf16": ([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp], _i),
     "s4g_interp_concat_act_bf16": ([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp], _i),
     "s4g_gather_xyz_f32_i32": ([_vp, _vp, _i, _i, _i, _vp, _vp], _i),
+    "s4g_gather_rows_bf16": ([_vp, _vp, _i, _i, _i, _i, _vp, _vp], _i),
     "s4g_rows_segment_max_bf16": ([_vp, _i, _i, _i, _vp, _vp], _i),
     "s4g_broadcast_concat_bf16": ([_vp, _vp, _i, _i, _i, _i, _vp, _vp], _i),
     "s4g_local_eval_rows_bf16": ([_vp, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp], _i),
@@ -113,6 +114,7 @@ _SIGNATURES = {
     "s4g_chain_set_xyz_layer": ([_vp, _vp, _i], _i),
     "s4g_chain_run_rows": ([_vp, _vp, _i, ctypes.c_longlong, _vp, _i, _vp], _i),
     "s4g_chain_run_gather": ([_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp], _i),
+    "s4g_chain_run_gather_term": ([_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp], _i),
     "s4g_cloud_transform_select_f32": ([_vp, _i, _i, _vp, _i, _vp, _vp, _vp], _i),
     "s4g_voxel_keys_f32": ([_vp, _i, _vp, _f, _vp, _vp, _vp], _i),
     "s4g_voxel_means_f32": ([_vp, _i, _vp, _vp, _vp, _vp, _i, _vp], _i),

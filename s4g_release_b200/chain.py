@@ -7,7 +7,7 @@ import torch
 
 from ._lib import check, lib, ptr, stream_ptr
 
-IN_ROWS, IN_GATHER, IN_XYZ_MLP = 0, 1, 5
+IN_ROWS, IN_GATHER, IN_XYZ_MLP, IN_GATHER_EDGE = 0, 1, 5, 6
 OUT_ROWS, OUT_MAXPOOL, OUT_LOGITS = 2, 3, 4
 
 
@@ -22,7 +22,9 @@ class MlpChain:
     the CUDA cores while it stages the tile.  Off by default — measured on the first set-abstraction level
     (64 x 5120 x 64 rows, 3 -> 128 -> 128 -> 256): 5.57 ms against 4.27 ms with the K = 16 tensor-core layer; the two
     loader warps cannot issue the 49 k FMAs of a tile as fast as the rest of the tile runs.
-    ``tma_in=1`` (row chains, cin[0] % 64 == 0): input blocks arrive by TMA tensor copies (s4g_chain_create_tuned_in)."""
+    ``tma_in=1`` (row chains, cin[0] % 64 == 0): input blocks arrive by TMA tensor copies (s4g_chain_create_tuned_in).
+    ``in_mode=IN_GATHER_EDGE``: an edge level's gathered max-pool chain; ``run_gather`` then takes the per-centroid term
+    of layer 0 (s4g_chain_run_gather_term)."""
 
     def __init__(self, layers, device, in_mode=IN_ROWS, feat_c=0, out_mode=OUT_ROWS, group=1, sigmoid=False,
                  xyz_layer_on_cuda_cores=False, slots=0, pairs=-1, coop=-1, subs=1, tma_in=0):
@@ -106,14 +108,23 @@ class MlpChain:
               "chain_run_rows")
         return out
 
-    def run_gather(self, feat, xyz, ctr, nbr):
-        """feat: bf16 [B*N, C] or None; xyz (B,3,N) fp32; ctr (B,3,M) fp32; nbr (B,M,K) int32."""
+    def run_gather(self, feat, xyz, ctr, nbr, term=None):
+        """feat: bf16 [B*N, C] or None; xyz (B,3,N) fp32; ctr (B,3,M) fp32; nbr (B,M,K) int32; term: an edge chain's
+        bf16 [B*M, cout[0]] per-centroid term of layer 0 (required for IN_GATHER_EDGE, refused otherwise)."""
         B, _, N = xyz.shape
         M, K = nbr.shape[1], nbr.shape[2]
         rows = B * M if self.out_mode == OUT_MAXPOOL else B * M * K
         out = torch.empty((rows, self.out_c), dtype=torch.bfloat16, device=xyz.device)
-        check(lib.s4g_chain_run_gather(self._h, ptr(feat) if feat is not None else None, ptr(xyz), ptr(ctr), ptr(nbr),
-                                       B, N, M, K, ptr(out), stream_ptr(xyz.device)), "chain_run_gather")
+        f = ptr(feat) if feat is not None else None
+        if self.in_mode == IN_GATHER_EDGE:
+            assert term is not None and term.dtype == torch.bfloat16 and term.is_contiguous()
+            assert tuple(term.shape) == (B * M, self.cout[0]) and term.device == xyz.device
+            check(lib.s4g_chain_run_gather_term(self._h, f, ptr(xyz), ptr(ctr), ptr(nbr), ptr(term), B, N, M, K, ptr(out),
+                                                stream_ptr(xyz.device)), "chain_run_gather_term")
+        else:
+            assert term is None, "only an IN_GATHER_EDGE chain takes a group term"
+            check(lib.s4g_chain_run_gather(self._h, f, ptr(xyz), ptr(ctr), ptr(nbr), B, N, M, K, ptr(out),
+                                           stream_ptr(xyz.device)), "chain_run_gather")
         return out
 
     def __del__(self):

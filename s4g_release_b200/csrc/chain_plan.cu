@@ -421,8 +421,9 @@ void evaluate(Candidate& c) {
 
 int plan_chain(s4g_chain* ch, int n_layers, const int* cin, const int* cout, const int* relu, int in_mode, int feat_c,
                int out_mode, int out_c, int group, int sigmoid, int force_slots, int force_pairs, int force_coop, int subs, int tma_in) {
+  const bool gathered = in_mode == IN_GATHER || in_mode == IN_GATHER_EDGE;
   S4G_CHECK_ARG(!tma_in || (in_mode == IN_ROWS && out_mode != OUT_MAXPOOL && cin[0] % 64 == 0) ||
-                    (in_mode == IN_GATHER && out_mode == OUT_MAXPOOL && n_layers > 1 && feat_c > 0 && feat_c % 64 == 0 &&
+                    (gathered && out_mode == OUT_MAXPOOL && n_layers > 1 && feat_c > 0 && feat_c % 64 == 0 &&
                      group % 4 == 0),
                 "mlp_chain: TMA input needs row input with a multiple of 64 channels and no max-pool, or a gathered "
                 "max-pool chain of >= 2 layers over a feature table of a multiple of 64 channels, group % 4 == 0");
@@ -433,8 +434,11 @@ int plan_chain(s4g_chain* ch, int n_layers, const int* cin, const int* cout, con
   } coop_scope(force_coop);
   memset(ch, 0, sizeof(*ch));
   S4G_CHECK_ARG(n_layers >= 1 && n_layers <= kMaxLayers, "mlp_chain: 1..%d layers supported", kMaxLayers);
-  S4G_CHECK_ARG(in_mode == IN_ROWS || in_mode == IN_GATHER || in_mode == IN_XYZ_MLP, "mlp_chain: bad in_mode");
+  S4G_CHECK_ARG(in_mode == IN_ROWS || gathered || in_mode == IN_XYZ_MLP, "mlp_chain: bad in_mode");
   S4G_CHECK_ARG(out_mode >= OUT_ROWS && out_mode <= OUT_LOGITS, "mlp_chain: bad out_mode");
+  // the per-group term is added by the hidden epilogue: layer 0 must not be the transposed max-pool layer
+  S4G_CHECK_ARG(in_mode != IN_GATHER_EDGE || (out_mode == OUT_MAXPOOL && n_layers > 1 && feat_c > 0),
+                "mlp_chain: an edge chain is a gathered max-pool chain of >= 2 layers over a feature table");
   ch->n_layers = n_layers;
   ch->in_mode = in_mode;
   ch->out_mode = out_mode;
@@ -445,7 +449,7 @@ int plan_chain(s4g_chain* ch, int n_layers, const int* cin, const int* cout, con
     ch->cin_pad[l] = round_up(cin[l], 16);
     ch->cout_pad[l] = round_up(cout[l], 16);
   }
-  if (in_mode == IN_GATHER) {
+  if (gathered) {
     S4G_CHECK_ARG(feat_c % 16 == 0 && cin[0] == feat_c + 3, "mlp_chain: gather input must be feat_c(%%16==0) + 3 xyz");
     ch->cin_pad[0] = feat_c + 16;
   } else if (in_mode == IN_XYZ_MLP) {
@@ -532,6 +536,7 @@ int plan_chain(s4g_chain* ch, int n_layers, const int* cin, const int* cout, con
   p.out_c = out_c;
   p.group = group > 0 ? group : 1;
   p.sigmoid = sigmoid;
+  p.term_c = in_mode == IN_GATHER_EDGE ? cout[0] : 0;
   ch->w_bytes = wb;
   ch->smem_bytes = (size_t)S * kSlotBytes + (size_t)d.stages * kStageBytes + 1024;
   ch->sim_cycles_per_tile = best.cycles;

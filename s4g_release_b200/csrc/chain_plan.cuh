@@ -61,7 +61,11 @@ constexpr int kMaxBlocks = 32;  // activation blocks per tile
 // IN_XYZ_MLP: gathered input without features whose 3 -> cin[0] first layer (K = 3: 81 % of a K = 16 MMA step
 // would be padding, and its epilogue a whole MMA -> epilogue -> MMA round trip) is computed by the loader warps
 // on the CUDA cores in fp32, straight into the activation block the chain's layer 0 reads
-enum InMode { IN_ROWS = 0, IN_GATHER = 1, IN_XYZ_MLP = 5 };
+// IN_GATHER_EDGE: IN_GATHER whose layer-0 epilogue also adds a per-group bf16 term term[row / K][col] to the shift, in
+// fp32, before the ReLU and the rounding — the centroid part -W_b f_c of an edge level (EdgeQueryGrouper's rows
+// [x_j - x_c | f_j | f_j - f_c] multiply as [W_x | W_a + W_b] [x_j - x_c ; f_j] - W_b f_c).  Planned exactly like
+// IN_GATHER; a mode of its own so that its kernels and tuned plans never mix with the plain chains'.
+enum InMode { IN_ROWS = 0, IN_GATHER = 1, IN_XYZ_MLP = 5, IN_GATHER_EDGE = 6 };
 enum OutMode { OUT_ROWS = 2, OUT_MAXPOOL = 3, OUT_LOGITS = 4 };
 
 // MF_PAIR: the job's MMAs are N = 256 wide and fill accumulators acc and acc + 1 (adjacent TMEM blocks)
@@ -143,6 +147,9 @@ struct ChainParams {
   int n_points;              // LOGITS: points per batch element
   int sigmoid;
   long long* prof;           // optional: 16 cycle counters per CTA (see s4g_chain_set_profile); null = off
+  // IN_GATHER_EDGE: bf16 [P / K][term_c] per-group term of layer 0 (term_c = layer 0's output width)
+  const void* term;
+  int term_c;
 };
 
 }  // namespace s4g

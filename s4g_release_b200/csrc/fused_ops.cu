@@ -275,7 +275,39 @@ local_eval_rows_kernel(const uint4* __restrict__ feat, int N, int C8, float* fra
   }
 }
 
+// Rows of a bf16 row table at int32 indices: out[b * M + m] = src[b * N + index[b][m]] — the centroid features of an edge
+// set-abstraction level (EdgeSAModule.forward gathers them at the level's sampled indices, modules.py:280-282).  One
+// thread per 16-byte piece of an output row; offsets in 64 bit, so tables over 2 GiB work.
+__global__ void __launch_bounds__(256)
+gather_rows_kernel(const uint4* __restrict__ src, const int* __restrict__ index, int N, int M, int C8,
+                   uint4* __restrict__ out) {
+  const int b = blockIdx.y;
+  const int n = M * C8;
+  const uint4* S = src + (size_t)b * N * C8;
+  const int* I = index + (size_t)b * M;
+  uint4* O = out + (size_t)b * n;
+  for (int i = blockIdx.x * 256 + threadIdx.x; i < n; i += gridDim.x * 256) {
+    const int m = i / C8, c = i - m * C8;
+    O[i] = __ldg(S + (size_t)__ldg(I + m) * C8 + c);
+  }
+}
+
 }  // namespace s4g
+
+extern "C" int s4g_gather_rows_bf16(const void* src, const int* index, int B, int N, int M, int C, void* out,
+                                    void* stream) {
+  S4G_CHECK_ARG(src && index && out, "gather_rows: null pointer");
+  S4G_CHECK_ARG(B >= 0 && B <= 65535 && N > 0 && M > 0 && C > 0 && C % 8 == 0 && (long long)M * (C / 8) < (1ll << 31),
+                "gather_rows: bad shape (C %% 8 == 0)");
+  S4G_CHECK_ARG(((uintptr_t)src & 15) == 0 && ((uintptr_t)out & 15) == 0, "gather_rows: rows must be 16-byte aligned");
+  if (B == 0) return S4G_OK;
+  const long long pieces = (long long)M * (C / 8);
+  const dim3 grid((unsigned)std::min<long long>((pieces + 255) / 256, 1024), (unsigned)B);
+  s4g::gather_rows_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const uint4*>(src), index, N, M, C / 8,
+                                                                   reinterpret_cast<uint4*>(out));
+  S4G_LAUNCH_CHECK("gather_rows");
+  return S4G_OK;
+}
 
 extern "C" int s4g_rows_segment_max_bf16(const void* in, int B, int P, int C, void* out, void* stream) {
   S4G_CHECK_ARG(in && out, "rows_segment_max: null pointer");

@@ -193,6 +193,25 @@ __device__ __forceinline__ uint4 epi_piece_r(const float* v, const float4 b0, co
                     bias_act_pack(v[4], v[5], b1.x, b1.y, relu), bias_act_pack(v[6], v[7], b1.z, b1.w, relu));
 }
 
+// shifts += a per-group term, NV / 4 16-byte pieces of bf16 (IN_GATHER_EDGE, layer 0); t == nullptr: no term
+template <int NV>
+__device__ __forceinline__ void add_term(float4* bv, const __nv_bfloat16* t) {
+  if (t == nullptr) return;
+#pragma unroll
+  for (int g = 0; g < NV / 2; ++g) {
+    const uint4 q = __ldg(reinterpret_cast<const uint4*>(t) + g);
+    const uint32_t w[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {  // bf16 -> fp32 is a 16-bit shift
+      float4& b = bv[2 * g + h];
+      b.x += __uint_as_float(w[2 * h] << 16);
+      b.y += __uint_as_float(w[2 * h] & 0xffff0000u);
+      b.z += __uint_as_float(w[2 * h + 1] << 16);
+      b.w += __uint_as_float(w[2 * h + 1] & 0xffff0000u);
+    }
+  }
+}
+
 template <bool PROF>
 __device__ __forceinline__ long long tick() {
   if constexpr (PROF) return clock64();
@@ -226,7 +245,9 @@ __device__ __forceinline__ void ring_at(const Ring& base, const ChainParams& p, 
 // carries the loader and the final epilogue it uses.
 // TMA_IN (row input only): the input blocks are fetched by one thread with 2-D tensor copies (64 channels x 128 rows
 // per box) into the 128-byte-swizzled K-major layout, instead of 64 threads x 16-byte cp.async into the interleaved one.
-template <bool PROF, bool XYZ_MLP, int OUT, bool GATHER, bool TMA_IN = false>
+// EDGE (IN_GATHER_EDGE): layer 0's epilogue adds the per-group term p.term[row / K] to the shifts.  Compile-time, so the
+// other chains carry none of its code.
+template <bool PROF, bool XYZ_MLP, int OUT, bool GATHER, bool TMA_IN = false, bool EDGE = false>
 __global__ void __launch_bounds__(kChainThreads, 1) mlp_chain_kernel(const __grid_constant__ ChainParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* slots = smem;
@@ -752,12 +773,19 @@ __global__ void __launch_bounds__(kChainThreads, 1) mlp_chain_kernel(const __gri
           const unsigned fpar = (unsigned)(job.same ? it : it - 1) & 1u;
           uint8_t* dst = slots + (size_t)slot * kSlotBytes + ((size_t)(c0 >> 3) * kTileRows + erow) * 16;
           __nv_bfloat16* orow = reinterpret_cast<__nv_bfloat16*>(p.out) + row * (long long)p.out_c + job.c_begin + c0;
+          // edge chain, layer 0: this row's group term (rows past P stay without one; their groups are never emitted)
+          const __nv_bfloat16* trow = nullptr;
+          if constexpr (EDGE) {
+            if (job.layer == 0 && row < p.P)
+              trow = reinterpret_cast<const __nv_bfloat16*>(p.term) + (long long)((int)row / p.K) * p.term_c + job.c_begin + c0;
+          }
           // full-width warps (64 columns, or 32 in a cooperative job): 32-column slabs, the second slab's shifts
           // travelling under its TMEM load.  Narrow layers (a multiple of 16 columns left): a compact 16-column
           // loop — the kernel's instruction footprint is what the common path pays for.
           if (ncol == 64 || ncol == 32) {
             float va[32];
             tmem_ld32_issue(t_addr, va);
+            if constexpr (EDGE) add_term<8>(bv, trow);
             if (need_free) {
               mbar_wait(&blk_free[job.pred], fpar);
               c_free += tick<PROF>() - t1;
@@ -773,6 +801,7 @@ __global__ void __launch_bounds__(kChainThreads, 1) mlp_chain_kernel(const __gri
               tmem_ld32_issue(t_addr + 32u, va);
 #pragma unroll
               for (int g = 0; g < 8; ++g) bv[g] = __ldg(reinterpret_cast<const float4*>(bias + 32) + g);
+              if constexpr (EDGE) add_term<8>(bv, trow ? trow + 32 : nullptr);
               tmem_wait();
 #pragma unroll
               for (int g = 0; g < 4; ++g) {
@@ -790,6 +819,7 @@ __global__ void __launch_bounds__(kChainThreads, 1) mlp_chain_kernel(const __gri
               float4 bw[4];
 #pragma unroll
               for (int g = 0; g < 4; ++g) bw[g] = __ldg(reinterpret_cast<const float4*>(bias + c) + g);
+              if constexpr (EDGE) add_term<4>(bw, trow ? trow + c : nullptr);
               tmem_wait();
 #pragma unroll
               for (int g = 0; g < 2; ++g) {
@@ -987,7 +1017,7 @@ extern "C" int s4g_chain_pack_weights(const s4g_chain* ch, int layer, const floa
   const s4g::ChainParams& p = ch->prm;
   __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(packed_host);
   size_t off = 0;  // in elements
-  const bool gather0 = (layer == 0 && ch->in_mode == s4g::IN_GATHER);
+  const bool gather0 = (layer == 0 && (ch->in_mode == s4g::IN_GATHER || ch->in_mode == s4g::IN_GATHER_EDGE));
   const int fc = p.feat_c;
   for (int j = 0; j < p.n_mma; ++j) {
     const s4g_chain::ChunkSrc& cs = ch->chunk[j];
@@ -1043,9 +1073,9 @@ extern "C" int s4g_chain_set_profile(s4g_chain* ch, void* counters_dev) {
 }
 
 namespace s4g {
-template <bool PROF, bool XYZ_MLP, int OUT, bool GATHER, bool TMA_IN = false>
+template <bool PROF, bool XYZ_MLP, int OUT, bool GATHER, bool TMA_IN = false, bool EDGE = false>
 static int launch_chain(const ChainParams& p, int grid, size_t smem, cudaStream_t stream) {
-  auto kern = mlp_chain_kernel<PROF, XYZ_MLP, OUT, GATHER, TMA_IN>;
+  auto kern = mlp_chain_kernel<PROF, XYZ_MLP, OUT, GATHER, TMA_IN, EDGE>;
   static bool attr_set[64] = {};
   if (s4g::first_use_on_device(attr_set)) {
     S4G_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
@@ -1062,10 +1092,16 @@ static int s4g_chain_launch(const s4g_chain* ch, s4g::ChainParams& p, cudaStream
   const int tiles = (p.P + tile_rows - 1) / tile_rows;
   const int grid = tiles < s4g::num_sms() ? tiles : s4g::num_sms();
   const bool gather = p.in_mode != s4g::IN_ROWS, xyz = p.in_mode == s4g::IN_XYZ_MLP, prof = p.prof != nullptr;
+  const bool edge = p.in_mode == s4g::IN_GATHER_EDGE;
   S4G_CHECK_ARG(!(xyz && prof), "mlp_chain: the cycle counters are not built for IN_XYZ_MLP chains");
   S4G_CHECK_ARG(!(p.tma_in && prof), "mlp_chain: the cycle counters are not built for TMA-input chains");
+  S4G_CHECK_ARG(!(edge && prof), "mlp_chain: the cycle counters are not built for edge chains");
   int rc = S4G_E_UNSUPPORTED;
-  if (p.tma_in) {
+  if (edge) {  // (the planner admits edge chains only as gathered max-pool chains)
+    if (ch->out_mode == s4g::OUT_MAXPOOL)
+      rc = p.tma_in ? s4g::launch_chain<false, false, s4g::OUT_MAXPOOL, true, true, true>(p, grid, ch->smem_bytes, stream)
+                    : s4g::launch_chain<false, false, s4g::OUT_MAXPOOL, true, false, true>(p, grid, ch->smem_bytes, stream);
+  } else if (p.tma_in) {
     if (ch->out_mode == s4g::OUT_ROWS && !gather) rc = s4g::launch_chain<false, false, s4g::OUT_ROWS, false, true>(p, grid, ch->smem_bytes, stream);
     if (ch->out_mode == s4g::OUT_LOGITS) rc = s4g::launch_chain<false, false, s4g::OUT_LOGITS, false, true>(p, grid, ch->smem_bytes, stream);
     if (ch->out_mode == s4g::OUT_MAXPOOL && gather) rc = s4g::launch_chain<false, false, s4g::OUT_MAXPOOL, true, true>(p, grid, ch->smem_bytes, stream);
@@ -1144,9 +1180,10 @@ extern "C" int s4g_chain_run_rows(const s4g_chain* ch, const void* in_rows, int 
 }
 
 // gathered in (set abstraction): feat [B*N][feat_c] bf16 (or NULL when feat_c == 0), xyz (B,3,N) fp32,
-// ctr (B,3,M) fp32, nbr (B,M,K) int32.  out: MAXPOOL -> bf16 [B*M][out_c]; ROWS -> bf16 [B*M*K][out_c].
-extern "C" int s4g_chain_run_gather(const s4g_chain* ch, const void* feat, const float* xyz, const float* ctr,
-                                    const int* nbr, int B, int N, int M, int K, void* out, void* stream) {
+// ctr (B,3,M) fp32, nbr (B,M,K) int32; term bf16 [B*M][cout[0]] of an edge chain, else NULL.
+// out: MAXPOOL -> bf16 [B*M][out_c]; ROWS -> bf16 [B*M*K][out_c].
+static int run_gather(const s4g_chain* ch, const void* feat, const float* xyz, const float* ctr, const int* nbr,
+                      const void* term, int B, int N, int M, int K, void* out, void* stream) {
   S4G_CHECK_ARG(ch && xyz && ctr && nbr && out, "mlp_chain: null pointer");
   S4G_CHECK_ARG(ch->in_mode != s4g::IN_ROWS, "mlp_chain: chain was planned for row input");
   S4G_CHECK_ARG(ch->in_mode != s4g::IN_XYZ_MLP || ch->prm.xyz_set, "mlp_chain: s4g_chain_set_xyz_layer was not called");
@@ -1161,10 +1198,27 @@ extern "C" int s4g_chain_run_gather(const s4g_chain* ch, const void* feat, const
   p.nbr = nbr;
   p.N = N; p.M = M; p.K = K;
   p.out = out;
+  p.term = term;
   if (p.tma_in && p.P > 0) {  // tile::gather4 copies: box = 64 channels x 1 row of the feature table
     S4G_CHECK_ARG(K % 4 == 0 && ((uintptr_t)nbr & 15) == 0, "mlp_chain: TMA gather needs K % 4 == 0 and 16-byte aligned indices");
     const int rc = encode_rows_map(&p.in_map, feat, ch->prm.feat_c, (long long)B * N, 1);
     if (rc != S4G_OK) return rc;
   }
   return s4g_chain_launch(ch, p, (cudaStream_t)stream);
+}
+
+extern "C" int s4g_chain_run_gather(const s4g_chain* ch, const void* feat, const float* xyz, const float* ctr,
+                                    const int* nbr, int B, int N, int M, int K, void* out, void* stream) {
+  S4G_CHECK_ARG(!ch || ch->in_mode != s4g::IN_GATHER_EDGE, "mlp_chain: an edge chain runs with s4g_chain_run_gather_term");
+  return run_gather(ch, feat, xyz, ctr, nbr, nullptr, B, N, M, K, out, stream);
+}
+
+// An edge level (EdgeSAModule): the gathered max-pool chain whose layer 0 adds term[b * M + m] (bf16, cout[0] wide,
+// 16-byte aligned rows) to the shifts of every row of centroid m's group, before the ReLU.
+extern "C" int s4g_chain_run_gather_term(const s4g_chain* ch, const void* feat, const float* xyz, const float* ctr,
+                                         const int* nbr, const void* term, int B, int N, int M, int K, void* out,
+                                         void* stream) {
+  S4G_CHECK_ARG(ch && ch->in_mode == s4g::IN_GATHER_EDGE, "mlp_chain: s4g_chain_run_gather_term needs an edge chain");
+  S4G_CHECK_ARG(term != nullptr && ((uintptr_t)term & 15) == 0, "mlp_chain: the group term must be 16-byte aligned");
+  return run_gather(ch, feat, xyz, ctr, nbr, term, B, N, M, K, out, stream);
 }

@@ -22,7 +22,7 @@ import numpy as np
 import torch
 
 from ._lib import check, lib, ptr, stream_ptr
-from .chain import IN_GATHER, IN_ROWS, OUT_LOGITS, OUT_MAXPOOL, OUT_ROWS, MlpChain
+from .chain import IN_GATHER, IN_GATHER_EDGE, IN_ROWS, OUT_LOGITS, OUT_MAXPOOL, OUT_ROWS, MlpChain
 
 BN_EPS = 1e-5
 GLOBAL_GROUPS = (8, 16, 32, 64)  # the max-pool group sizes the chain planner accepts
@@ -170,7 +170,7 @@ def candidate_plans(in_mode, feat_c, out_mode):
     cands += [(sl, -1, co, 2, 0) for sl in (0, 3, 4, 5) for co in (-1, 0, 1)]
     # the same plans with the input blocks fetched by TMA: tensor copies for row chains (refused unless
     # cin % 64 == 0), tile::gather4 copies of the neighbours' feature rows for gathered max-pool chains
-    if (in_mode == IN_ROWS and out_mode != OUT_MAXPOOL) or (in_mode == IN_GATHER and feat_c > 0):
+    if (in_mode == IN_ROWS and out_mode != OUT_MAXPOOL) or (in_mode in (IN_GATHER, IN_GATHER_EDGE) and feat_c > 0):
         cands += [c[:4] + (1,) for c in cands]
     return cands
 
@@ -242,7 +242,7 @@ class FusedPointNet2:
         while rows * row_bytes > free_bytes // 8 and tiles > sms * 4:
             tiles //= 2
             rows = tiles * 128
-        if in_mode == IN_GATHER:
+        if in_mode in (IN_GATHER, IN_GATHER_EDGE):
             K = group
             M = rows // K
             N = 4 * M
@@ -252,7 +252,10 @@ class FusedPointNet2:
             near = torch.randint(0, 512, (1, M, K), device=dev, dtype=torch.int64, generator=g)
             nbr = ((torch.arange(M, device=dev).view(1, M, 1) * (N // M) + near) % N).to(torch.int32)
             feat = torch.randn(N, feat_c, device=dev, generator=g).to(torch.bfloat16) if feat_c else None
-            run = lambda ch: ch.run_gather(feat, xyz, ctr, nbr)
+            term = None
+            if in_mode == IN_GATHER_EDGE:
+                term = torch.randn(M, layers[0][0].shape[0], device=dev, generator=g).to(torch.bfloat16)
+            run = lambda ch: ch.run_gather(feat, xyz, ctr, nbr, term)
         else:
             x = torch.randn(rows, layers[0][0].shape[1], device=dev, generator=g).to(torch.bfloat16)
             n_points = rows if out_mode == OUT_LOGITS else 0
@@ -306,8 +309,7 @@ class FusedPointNet2:
         self.sa_chains = []  # the sampled levels
         feat_c = 0
         for i, layers in enumerate(self.sa[:len(self.sa) - self.global_level]):
-            self.sa_chains.append(self._make_chain([(w, b, True) for w, b in layers], IN_GATHER, feat_c, OUT_MAXPOOL,
-                                                   group=cfg["num_neighbours"][i]))
+            self.sa_chains.append(self._sa_chain(i, layers, feat_c))
             feat_c = layers[-1][0].shape[0]
         self._global_feat_c = feat_c
         if self.global_level and self.sa_chains:  # the global level's cloud size is the previous level's centroid count
@@ -332,6 +334,21 @@ class FusedPointNet2:
         for k, (layers, w, b) in enumerate(self.heads):
             self.head_chains.append(self._make_chain([(lw, lb, True) for lw, lb in layers] + [(w, b, False)], IN_ROWS, 0,
                                                      OUT_LOGITS, sigmoid=self._HEAD_SIGMOID[k]))
+
+    def _sa_chain(self, i, layers, feat_c):
+        """The gathered max-pool chain of sampled level i over a feature table of feat_c channels."""
+        return self._make_chain([(w, b, True) for w, b in layers], IN_GATHER, feat_c, OUT_MAXPOOL,
+                                group=self.cfg["num_neighbours"][i])
+
+    def _sa_level(self, i, feat, xyz, new_xyz, nbr, idx, timer):
+        """Sampled level i's MLP + max-pool on the tcgen05 trunk: bf16 [B*N, C] (or None) -> bf16 [B*M, C'].  ``idx``:
+        the level's sampled indices (B, M)."""
+        with _sec(timer, "sa%d.mlp" % i):
+            return self.sa_chains[i].run_gather(feat, xyz, new_xyz, nbr)
+
+    def _sa_reference(self, i, xyz, feat, new_xyz, nbr, idx, layers):
+        """Sampled level i on the torch / tf32 backends: (B, N, C) fp32 (or None) -> (B, M, C')."""
+        return self._sa_torch(xyz, feat, new_xyz, nbr, layers)
 
     def _global_chain(self, g):
         """The global level's max-pool chain for groups of g rows (g follows the cloud size, see global_group_table)."""
@@ -438,8 +455,9 @@ class FusedPointNet2:
             x = torch.relu(torch.addmm(b, x.reshape(-1, x.shape[-1]), w.t()).reshape(*x.shape[:-1], w.shape[0]))
         return x
 
-    def _sa_torch(self, xyz, feat_cl, new_xyz, nbr, layers, chunk=4):
-        """xyz (B,3,N); feat_cl (B,N,C) or None; nbr (B,M,K) -> (B,M,Cout) channel-last."""
+    def _sa_torch(self, xyz, feat_cl, new_xyz, nbr, layers, chunk=4, ctr_feat=None):
+        """xyz (B,3,N); feat_cl (B,N,C) or None; nbr (B,M,K) -> (B,M,Cout) channel-last.  ``ctr_feat`` (B,M,C): an edge
+        level's centroid features; the rows are then EdgeQueryGrouper's [x_j - x_c | f_j | f_j - f_c]."""
         B, M, K = nbr.shape
         out = []
         xyz_cl = xyz.transpose(1, 2)  # (B,N,3)
@@ -452,7 +470,8 @@ class FusedPointNet2:
             if feat_cl is not None:
                 C = feat_cl.shape[-1]
                 g_f = torch.gather(feat_cl[sl], 1, idx.unsqueeze(-1).expand(-1, -1, C)).reshape(-1, M, K, C)
-                g = torch.cat([g, g_f], dim=-1)
+                parts = [g, g_f] if ctr_feat is None else [g, g_f, g_f - ctr_feat[sl].unsqueeze(2)]
+                g = torch.cat(parts, dim=-1)
             out.append(self._mlp(g, layers).max(dim=2)[0])
         return torch.cat(out, 0)
 
@@ -547,7 +566,7 @@ class FusedPointNet2:
         overlap = self.overlap_geometry
         main = torch.cuda.current_stream()
         pending, early_nn = None, {}
-        for i, chain in enumerate(self.sa_chains):
+        for i in range(len(self.sa_chains)):
             ball_grid = None
             # (levels below the one-call form's grid threshold stay on the linear scan: with the build hidden the grid
             # query of the second level, 5 120 points, still measured 0.30 ms against 0.26 ms)
@@ -589,8 +608,7 @@ class FusedPointNet2:
             finally:
                 if ball_grid:  # host struct + stream-ordered arena: released whatever happened in between
                     lib.s4g_ball_grid_free(ball_grid, stream_ptr(xyz.device))
-            with _sec(timer, "sa%d.mlp" % i):
-                feat = chain.run_gather(feat, xyz, new_xyz, nbr)
+            feat = self._sa_level(i, feat, xyz, new_xyz, nbr, idx, timer)
             if overlap and i + 1 < n_sa and len(self.fp_chains) == n_sa:
                 ready = torch.cuda.Event()
                 ready.record()  # after this level's chain: the search starts together with the next level's sampling
@@ -706,7 +724,7 @@ class FusedPointNet2:
             idx = self.fps(xyz, cfg["num_centroids"][i])
             new_xyz = torch.gather(xyz, 2, idx.long().unsqueeze(1).expand(-1, 3, -1)).contiguous()
             nbr = self.ball_query(xyz, new_xyz, cfg["radius"][i], cfg["num_neighbours"][i])
-            feat = self._sa_torch(xyz, feat, new_xyz, nbr, layers)
+            feat = self._sa_reference(i, xyz, feat, new_xyz, nbr, idx, layers)
             xyz = new_xyz
             lv_xyz.append(xyz)
             lv_feat.append(feat)
@@ -835,3 +853,66 @@ class FusedPointNet2Local(FusedPointNet2):
             check_local_frames(points, frames)
         return self._run(points, return_trace, timer,
                          lambda xyz, sparse: self._local_head_stage(xyz, sparse, frames, timer))
+
+
+class FusedEdgePointNet2Down(FusedPointNet2):
+    """EDGEPN2D (models/EdgePointNet2Down.py): the PN2 sibling whose sampled levels with input features are edge levels
+    (EdgeSAModule).  Their first layer sees EdgeQueryGrouper's rows [x_j - x_c | f_j | f_j - f_c] (3 + 2C channels); with
+    the folded weight split by those column groups, W' = [W_x | W_a | W_b], it is
+        [W_x | W_a + W_b] [x_j - x_c ; f_j] + b' + u_c,   u_c = -W_b f_c,
+    so on the tcgen05 trunk an edge level is the plain gathered chain over 3 + C channels with the weights
+    [W_x | W_a + W_b], plus the centroid term u: the centroid rows (``gather_rows`` at the level's sampled indices) through
+    a one-layer row chain (-W_b, zero shift, no ReLU), added by the edge chain's layer-0 epilogue before the ReLU.  The
+    (B, 3 + 2C, M, K) edge tensor never exists.  The torch / tf32 backends build the edge rows literally and use the
+    unsplit weights: an independent check of the split.  Level 0 (no input features) and the global level are PN2's."""
+
+    def __init__(self, model, *args, **kwargs):
+        from .network_models.models.pointnet2_utils.modules import EdgeSAModule
+        c = 0
+        self.edge_levels = []  # per set-abstraction level: an edge level (sampled, with input features)
+        for m in model.sa_modules:
+            self.edge_levels.append(isinstance(m, EdgeSAModule) and m.num_centroids > 0 and c > 0)
+            c = m.out_channels
+        self._term_chains = {}  # edge level -> the row chain of its centroid term u
+        super().__init__(model, *args, **kwargs)
+
+    @staticmethod
+    def split_edge_layer(w, c):
+        """Folded first-layer weight of an edge level, fp32 [cout, 3 + 2c] with columns [xyz | neighbour | difference]
+        -> ([W_x | W_a + W_b] [cout, 3 + c], -W_b [cout, c]), in the input's precision (split before any bf16 cast)."""
+        assert w.dim() == 2 and w.shape[1] == 3 + 2 * c, "edge layer expects 3 + 2 x %d input channels" % c
+        wx, wa, wb = w[:, :3], w[:, 3:3 + c], w[:, 3 + c:]
+        return torch.cat([wx, wa + wb], dim=1).contiguous(), (-wb).contiguous()
+
+    def _sa_chain(self, i, layers, feat_c):
+        if not self.edge_levels[i]:
+            return super()._sa_chain(i, layers, feat_c)
+        (w0, b0), rest = layers[0], layers[1:]
+        w_plain, w_u = self.split_edge_layer(w0, feat_c)
+        self._term_chains[i] = self._make_chain([(w_u, torch.zeros_like(b0), False)], IN_ROWS, 0, OUT_ROWS)
+        return self._make_chain([(w_plain, b0, True)] + [(w, b, True) for w, b in rest], IN_GATHER_EDGE, feat_c,
+                                OUT_MAXPOOL, group=self.cfg["num_neighbours"][i])
+
+    @staticmethod
+    def gather_rows(rows, idx):
+        """bf16 [B*N, C] rows, int32 indices (B, M) -> bf16 [B*M, C], row b*M + m = rows[b*N + idx[b, m]]."""
+        B, M = idx.shape
+        C = rows.shape[1]
+        out = torch.empty((B * M, C), dtype=torch.bfloat16, device=rows.device)
+        check(lib.s4g_gather_rows_bf16(ptr(rows), ptr(idx), B, rows.shape[0] // B, M, C, ptr(out),
+                                       stream_ptr(rows.device)), "gather_rows")
+        return out
+
+    def _sa_level(self, i, feat, xyz, new_xyz, nbr, idx, timer):
+        if not self.edge_levels[i]:
+            return super()._sa_level(i, feat, xyz, new_xyz, nbr, idx, timer)
+        with _sec(timer, "sa%d.term" % i):
+            term = self._term_chains[i].run_rows(self.gather_rows(feat, idx))  # u = -W_b f_c, bf16 [B*M, cout0]
+        with _sec(timer, "sa%d.mlp" % i):
+            return self.sa_chains[i].run_gather(feat, xyz, new_xyz, nbr, term)
+
+    def _sa_reference(self, i, xyz, feat, new_xyz, nbr, idx, layers):
+        if not self.edge_levels[i]:
+            return super()._sa_reference(i, xyz, feat, new_xyz, nbr, idx, layers)
+        ctr_feat = torch.gather(feat, 1, idx.long().unsqueeze(-1).expand(-1, -1, feat.shape[-1]))
+        return self._sa_torch(xyz, feat, new_xyz, nbr, layers, ctr_feat=ctr_feat)

@@ -1,8 +1,10 @@
 """EDGEPN2D — PN2 with EdgeConv set-abstraction levels (reference: network_models/models/EdgePointNet2Down.py:9-33).
 
 The reference's class is the PN2 sibling with ``_SA_MODULE = EdgeSAModule`` and the plain PointnetFPModule decoder; the
-builder reads the ``MODEL.EDGEPN2D`` node.  Edge set abstraction concatenates centroid features to every neighbour, which
-the fused engine has no plan for: this model always runs on the module path (sm_100a operators + torch autograd)."""
+builder reads the ``MODEL.EDGEPN2D`` node.  An edge level concatenates centroid features to every neighbour; the fused
+engine (engine.FusedEdgePointNet2Down) runs it without building those rows, by splitting the level's first layer into a
+neighbour part and a centroid part.  The fused engine is opt-in, ``forward(..., fused=True)``; otherwise the model runs
+on the module path (sm_100a operators + torch autograd), as does its training."""
 from . import PointNet2 as _pn2
 from .pointnet2_utils.modules import EdgeSAModule, PointnetFPModule
 
@@ -12,9 +14,27 @@ PointNet2Loss, PointNet2Metric = _pn2.PointNet2Loss, _pn2.PointNet2Metric
 class EdgePointNet2Down(_pn2.PointNet2):
     _SA_MODULE = EdgeSAModule
     _FP_MODULE = PointnetFPModule
+    _ENGINE = "FusedEdgePointNet2Down"
 
-    def fusable(self):
-        return False
+    def fusable(self, allow_global=False):
+        """Whether the fused engine has a plan for this configuration: the PN2 sibling's rules (PointNet2_tcls.PointNet2.
+        fusable, ``allow_global`` as there) and every edge level (sampled, with input features) at least two layers deep
+        — the centroid term joins the first layer's epilogue, and a one-layer level's first layer is its max-pool."""
+        if not super().fusable(allow_global):
+            return False
+        c = self.config
+        return all(len(ch) > 1 for i, ch in enumerate(c["sa_channels"]) if i > 0 and c["num_centroids"][i] != 0)
+
+    def forward(self, data_batch, fused=None):
+        """``fused``: None / False = the module path; True = the fused engine, for every configuration
+        ``fusable(allow_global=True)`` accepts (others raise RuntimeError before any GPU work)."""
+        points = data_batch["scene_points"]
+        if not fused:
+            return self.predictions(self.forward_modules(points), points)
+        if not self.fusable(allow_global=True):
+            raise RuntimeError("the fused engine has no plan for this configuration (see EdgePointNet2Down.fusable); "
+                               "call with fused=False for the module path")
+        return self.predictions(self.fused_engine().forward(points), points)
 
 
 def build_edgepointnet2down(cfg):

@@ -373,6 +373,12 @@ class TrainEngine:
     level paired with broadcast propagation after at least one sampled level); ``loss_fn``: the model's PointNet2Loss."""
 
     def __init__(self, model, loss_fn, seed=0):
+        from .network_models.models.pointnet2_utils.modules import EdgeSAModule
+        if any(isinstance(m, EdgeSAModule) for m in getattr(model, "sa_modules", ())):
+            # an edge level's first layer reads [x_j - x_c | f_j | f_j - f_c] rows, not the [f | xyz] rows these kernels
+            # group; its backward would also owe the centroid features a gradient
+            raise RuntimeError("TrainEngine: no fused training step for edge set-abstraction levels (EdgeSAModule, "
+                               "EDGEPN2D); train this model on the module path (Trainer(fused=False))")
         if not _has_training_plan(model):
             raise RuntimeError("TrainEngine: no fused plan for this configuration (PointNet2.fusable)")
         if type(self) is TrainEngine and _is_local(model):
