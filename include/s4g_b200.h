@@ -307,6 +307,27 @@ int s4g_gather_xyz_f32_i32(const float* xyz, const int* index, int B, int N, int
  * C % 8 == 0, rows 16-byte aligned; 64-bit offsets (tables over 2 GiB). */
 int s4g_gather_rows_bf16(const void* src, const int* index, int B, int N, int M, int C, void* out, void* stream);
 
+/* Edge feature propagation (EdgeFPModule, pointnet2_utils/modules.py:287-308, fed by EdgeFeatureInterpolator, :227-247):
+ * per dense point q and each of its 3 nearest sparse points k the MLP's first layer sees [interp_q | n_k - interp_q | d_q]
+ * (2 C2 + C1 channels).  With its BN-folded weight split by those column groups, W' = [W_i | W_n | W_d], and shift b',
+ *   y0[q,k] = sum_j w_qj U[idx_qj] + V[idx_qk] + T_q + b',   U = (W_i - W_n) S,  V = W_n S,  T = W_d d,
+ * whatever the weights sum to.  This writes out[(b*Nq + q)*3 + k][c] = relu(((sum_j w_qj U + V[idx_qk]) + T_q) + b') in
+ * fp32, in that order, rounded to bf16 once; the sum over j is fma(U2,w2, fma(U1,w1, U0*w0)); the ReLU is fmaxf(y, 0), so a
+ * NaN pre-activation gives 0.
+ *   uv     [B*Nk][2C] bf16, rows [U | V] (C = cout of the first layer, C % 8 == 0);
+ *   index, weight (B,Nq,3) from s4g_three_nn_weights_f32_i32: int32 in [0, Nk), which it writes for non-finite clouds too;
+ *   exactly one skip: t_rows [B*Nq][C] bf16 (T computed), or the cloud itself xyz (B,3,Nq) fp32 with w_xyz [C][3] fp32
+ *   (T = fma(W_d2, z, fma(W_d1, y, W_d0 x)) in fp32: coordinates are not rounded to bf16);
+ *   shift [C] fp32 = b'.  Rows and shift 16-byte aligned; 64-bit offsets (outputs over 2 GiB), Nq * C / 8 < 2^31. */
+int s4g_edge_interp_rows_bf16(const void* uv, const int* index, const float* weight, const void* t_rows, const float* xyz,
+                              const float* w_xyz, const float* shift, int B, int Nk, int Nq, int C, void* out,
+                              void* stream);
+
+/* EdgeFPModule's torch.mean over the 3 neighbour rows (modules.py:308): in [3R][C] bf16 -> out [R][C] bf16,
+ * out[r] = ((in[3r] + in[3r+1]) + in[3r+2]) / 3 in fp32 with IEEE division, rounded once.  C % 8 == 0, rows 16-byte
+ * aligned, R * C / 8 < 2^31; 64-bit offsets. */
+int s4g_rows_group_mean_bf16(const void* in, long long R, int C, void* out, void* stream);
+
 /* The max over the neighbours of a GLOBAL set-abstraction level (num_centroids = 0: one group of all N points centred
  * at the origin, PointNetSAModule.forward, modules.py:93-98 + :106 torch.max(new_feature, 3)).  The fused path runs the
  * group through the gathered max-pool chain as P partial groups; this reduces the P partial rows of each scene:

@@ -16,6 +16,10 @@ if "--edge" in sys.argv:  # the chains of EDGEPN2D at its default arguments (the
     from bench_global import seeded  # noqa: E402
     from s4g_release_b200.network_models.models.EdgePointNet2Down import EdgePointNet2Down  # noqa: E402
     eng = engine.FusedEdgePointNet2Down(seeded(EdgePointNet2Down).cuda(), autotune="force")
+elif "--edge-downup" in sys.argv:  # EDGEPN2DU at its default arguments (the table keeps its edge propagation chains)
+    from bench_global import seeded  # noqa: E402
+    from s4g_release_b200.network_models.models.EdgePointNet2DownUp import EdgePointNet2DownUp  # noqa: E402
+    eng = engine.FusedEdgePointNet2DownUp(seeded(EdgePointNet2DownUp).cuda(), autotune="force")
 else:
     eng = engine.FusedPointNet2(seeded_model().cuda(), autotune="force")
 torch.cuda.synchronize()

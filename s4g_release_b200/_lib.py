@@ -59,6 +59,8 @@ _SIGNATURES = {
     "s4g_interp_concat_act_bf16": ([_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp], _i),
     "s4g_gather_xyz_f32_i32": ([_vp, _vp, _i, _i, _i, _vp, _vp], _i),
     "s4g_gather_rows_bf16": ([_vp, _vp, _i, _i, _i, _i, _vp, _vp], _i),
+    "s4g_edge_interp_rows_bf16": ([_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp], _i),
+    "s4g_rows_group_mean_bf16": ([_vp, _ll, _i, _vp, _vp], _i),
     "s4g_rows_segment_max_bf16": ([_vp, _i, _i, _i, _vp, _vp], _i),
     "s4g_broadcast_concat_bf16": ([_vp, _vp, _i, _i, _i, _i, _vp, _vp], _i),
     "s4g_local_eval_rows_bf16": ([_vp, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp], _i),

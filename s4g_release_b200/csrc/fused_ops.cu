@@ -292,7 +292,141 @@ gather_rows_kernel(const uint4* __restrict__ src, const int* __restrict__ index,
   }
 }
 
+// First layer of an edge feature-propagation level (EdgeFPModule, modules.py:287-308, rows from EdgeFeatureInterpolator,
+// :227-247) from its split pre-activations: row q * 3 + k of the output is
+//   relu(((sum_j w_qj U[idx_qj] + V[idx_qk]) + T_q) + b')
+// in fp32, in that order, rounded to bf16 once; the interpolation sum is interp_pair's fma(U2,w2, fma(U1,w1, U0*w0)).
+// uv: bf16 [B*Nk][2C] rows [U | V]; T_q is either a bf16 row of t_rows [B*Nq][C] or, for the cloud as skip feature,
+// fma(W_d[c][2], z, fma(W_d[c][1], y, W_d[c][0] * x)) from the planar fp32 cloud (B,3,Nq) — coordinates stay fp32.
+// One thread per (query, 16-byte piece of 8 channels), so narrow levels (C = 64: 8 pieces) still use every lane; the
+// threads of one query write adjacent pieces of its three rows.  Offsets in 64 bit.
+__device__ __forceinline__ void bf16x8_to_f32(uint4 v, float* f) {
+  const uint32_t p[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    f[2 * i] = __uint_as_float(p[i] << 16);
+    f[2 * i + 1] = __uint_as_float(p[i] & 0xffff0000u);
+  }
+}
+
+__device__ __forceinline__ uint4 f32_to_bf16x8(const float* f) {
+  uint32_t p[4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const __nv_bfloat162 h = __floats2bfloat162_rn(f[2 * i], f[2 * i + 1]);
+    p[i] = *reinterpret_cast<const uint32_t*>(&h);
+  }
+  return make_uint4(p[0], p[1], p[2], p[3]);
+}
+
+template <bool kXyz>
+__global__ void __launch_bounds__(256)
+edge_interp_rows_kernel(const uint4* __restrict__ uv, const int* __restrict__ index, const float* __restrict__ weight,
+                        const uint4* __restrict__ t_rows, const float* __restrict__ xyz, const float* __restrict__ w_xyz,
+                        const float* __restrict__ shift, int Nk, int Nq, int C8, uint4* __restrict__ out) {
+  const int b = blockIdx.y;
+  const int i = blockIdx.x * 256 + threadIdx.x;
+  if (i >= Nq * C8) return;
+  const int q = i / C8, c = i - q * C8;
+  const size_t row = (size_t)b * Nq + q;  // batch-global query row
+  const uint4* src[3];
+  float w[3];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    src[k] = uv + ((size_t)b * Nk + __ldg(index + row * 3 + k)) * (2 * C8) + c;
+    w[k] = __ldg(weight + row * 3 + k);
+  }
+  uint4 u[3], v[3];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    u[k] = __ldg(src[k]);
+    v[k] = __ldg(src[k] + C8);
+  }
+  float tq[8];
+  if (kXyz) {
+    const float* X = xyz + (size_t)b * 3 * Nq + q;
+    const float x = __ldg(X), y = __ldg(X + Nq), z = __ldg(X + 2 * (size_t)Nq);
+#pragma unroll
+    for (int e = 0; e < 8; ++e) {
+      const float* wd = w_xyz + (size_t)(8 * c + e) * 3;
+      tq[e] = __fmaf_rn(__ldg(wd + 2), z, __fmaf_rn(__ldg(wd + 1), y, __fmul_rn(__ldg(wd), x)));
+    }
+  } else {
+    bf16x8_to_f32(__ldg(t_rows + row * C8 + c), tq);
+  }
+  float sh[8], f0[8], f1[8], f2[8], base[8];
+  const float4 s0 = __ldg(reinterpret_cast<const float4*>(shift) + 2 * c);
+  const float4 s1 = __ldg(reinterpret_cast<const float4*>(shift) + 2 * c + 1);
+  sh[0] = s0.x; sh[1] = s0.y; sh[2] = s0.z; sh[3] = s0.w; sh[4] = s1.x; sh[5] = s1.y; sh[6] = s1.z; sh[7] = s1.w;
+  bf16x8_to_f32(u[0], f0);
+  bf16x8_to_f32(u[1], f1);
+  bf16x8_to_f32(u[2], f2);
+#pragma unroll
+  for (int e = 0; e < 8; ++e) base[e] = __fmaf_rn(f2[e], w[2], __fmaf_rn(f1[e], w[1], __fmul_rn(f0[e], w[0])));
+  uint4* o = out + row * 3 * C8 + c;
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    float y[8];
+    bf16x8_to_f32(v[k], y);
+#pragma unroll
+    for (int e = 0; e < 8; ++e) y[e] = fmaxf(__fadd_rn(__fadd_rn(__fadd_rn(base[e], y[e]), tq[e]), sh[e]), 0.f);
+    o[(size_t)k * C8] = f32_to_bf16x8(y);
+  }
+}
+
+// torch.mean over EdgeFPModule's K = 3 neighbour rows (modules.py:308): out[r] = ((in[3r] + in[3r+1]) + in[3r+2]) / 3 in
+// fp32 (IEEE division), rounded to bf16 once.  One thread per 16-byte piece of an output row; offsets in 64 bit.
+__global__ void __launch_bounds__(256)
+rows_group_mean_kernel(const uint4* __restrict__ in, int R, int C8, uint4* __restrict__ out) {
+  const int n = R * C8;
+  for (int i = blockIdx.x * 256 + threadIdx.x; i < n; i += gridDim.x * 256) {
+    const int r = i / C8, c = i - r * C8;
+    const uint4* p = in + (size_t)r * 3 * C8 + c;
+    float a[8], b[8], d[8];
+    bf16x8_to_f32(__ldg(p), a);
+    bf16x8_to_f32(__ldg(p + C8), b);
+    bf16x8_to_f32(__ldg(p + 2 * C8), d);
+#pragma unroll
+    for (int e = 0; e < 8; ++e) a[e] = __fdiv_rn(__fadd_rn(__fadd_rn(a[e], b[e]), d[e]), 3.0f);
+    out[(size_t)r * C8 + c] = f32_to_bf16x8(a);
+  }
+}
+
 }  // namespace s4g
+
+extern "C" int s4g_edge_interp_rows_bf16(const void* uv, const int* index, const float* weight, const void* t_rows,
+                                         const float* xyz, const float* w_xyz, const float* shift, int B, int Nk, int Nq,
+                                         int C, void* out, void* stream) {
+  S4G_CHECK_ARG(uv && index && weight && shift && out, "edge_interp_rows: null pointer");
+  S4G_CHECK_ARG((t_rows != nullptr) != (xyz != nullptr), "edge_interp_rows: exactly one of t_rows and xyz");
+  S4G_CHECK_ARG(xyz == nullptr || w_xyz != nullptr, "edge_interp_rows: the cloud as skip feature needs w_xyz");
+  S4G_CHECK_ARG(B >= 0 && B <= 65535 && Nq > 0 && Nk > 0 && C > 0 && C % 8 == 0 && (long long)Nq * (C / 8) < (1ll << 31),
+                "edge_interp_rows: bad shape (C %% 8 == 0)");
+  S4G_CHECK_ARG(((uintptr_t)uv & 15) == 0 && ((uintptr_t)out & 15) == 0 && ((uintptr_t)t_rows & 15) == 0 &&
+                    ((uintptr_t)shift & 15) == 0,
+                "edge_interp_rows: rows and shift must be 16-byte aligned");
+  if (B == 0) return S4G_OK;
+  const dim3 grid((unsigned)(((long long)Nq * (C / 8) + 255) / 256), (unsigned)B);
+  auto kernel = xyz != nullptr ? s4g::edge_interp_rows_kernel<true> : s4g::edge_interp_rows_kernel<false>;
+  kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const uint4*>(uv), index, weight,
+                                                 reinterpret_cast<const uint4*>(t_rows), xyz, w_xyz, shift, Nk, Nq, C / 8,
+                                                 reinterpret_cast<uint4*>(out));
+  S4G_LAUNCH_CHECK("edge_interp_rows");
+  return S4G_OK;
+}
+
+extern "C" int s4g_rows_group_mean_bf16(const void* in, long long R, int C, void* out, void* stream) {
+  S4G_CHECK_ARG(in && out, "rows_group_mean: null pointer");
+  S4G_CHECK_ARG(R >= 0 && C > 0 && C % 8 == 0 && R * (C / 8) < (1ll << 31), "rows_group_mean: bad shape (C %% 8 == 0)");
+  S4G_CHECK_ARG(((uintptr_t)in & 15) == 0 && ((uintptr_t)out & 15) == 0, "rows_group_mean: rows must be 16-byte aligned");
+  if (R == 0) return S4G_OK;
+  const long long pieces = R * (C / 8);
+  const unsigned grid = (unsigned)std::min<long long>((pieces + 255) / 256, 148 * 16);
+  s4g::rows_group_mean_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const uint4*>(in), (int)R, C / 8,
+                                                                       reinterpret_cast<uint4*>(out));
+  S4G_LAUNCH_CHECK("rows_group_mean");
+  return S4G_OK;
+}
 
 extern "C" int s4g_gather_rows_bf16(const void* src, const int* index, int B, int N, int M, int C, void* out,
                                     void* stream) {

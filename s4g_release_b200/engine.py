@@ -321,19 +321,22 @@ class FusedPointNet2:
         self.fp_pre, self.fp_chains = [], []
         skip_c = [0] + [layers[-1][0].shape[0] for layers in self.sa]
         for i, layers in enumerate(self.fp):
-            broadcast = i == 0 and self.global_level
-            if (self.fp_linear_split and not broadcast and skip_c[-2 - i] == 0 and len(layers) > 1
-                    and layers[0][0].shape[0] <= 512):
-                w0, b0 = layers[0]
-                self.fp_pre.append(self._make_chain([(w0, b0, False)], IN_ROWS, 0, OUT_ROWS))
-                self.fp_chains.append(self._row_chains(layers[1:]))
-            else:
-                self.fp_pre.append(None)
-                self.fp_chains.append(self._row_chains(layers))
+            pre, chains = self._fp_chain(i, layers, skip_c[-2 - i])
+            self.fp_pre.append(pre)
+            self.fp_chains.append(chains)
         self.head_chains = []
         for k, (layers, w, b) in enumerate(self.heads):
             self.head_chains.append(self._make_chain([(lw, lb, True) for lw, lb in layers] + [(w, b, False)], IN_ROWS, 0,
                                                      OUT_LOGITS, sigmoid=self._HEAD_SIGMOID[k]))
+
+    def _fp_chain(self, i, layers, skip_c):
+        """Propagation level i's chains over a skip feature of skip_c channels (0: none) -> (the first layer on the
+        sparse rows, or None; the row chains)."""
+        broadcast = i == 0 and self.global_level
+        if self.fp_linear_split and not broadcast and skip_c == 0 and len(layers) > 1 and layers[0][0].shape[0] <= 512:
+            w0, b0 = layers[0]
+            return self._make_chain([(w0, b0, False)], IN_ROWS, 0, OUT_ROWS), self._row_chains(layers[1:])
+        return None, self._row_chains(layers)
 
     def _sa_chain(self, i, layers, feat_c):
         """The gathered max-pool chain of sampled level i over a feature table of feat_c channels."""
@@ -476,6 +479,12 @@ class FusedPointNet2:
         return torch.cat(out, 0)
 
     def _fp_torch(self, dense_xyz, sparse_xyz, dense_cl, sparse_cl, layers):
+        _, interp = self._interp_torch(dense_xyz, sparse_xyz, sparse_cl)
+        x = interp if dense_cl is None else torch.cat([interp, dense_cl], dim=-1)
+        return self._mlp(x, layers)
+
+    def _interp_torch(self, dense_xyz, sparse_xyz, sparse_cl):
+        """FeatureInterpolator's 3-NN interpolation: -> (the neighbours' features (B, Nq, 3, C), interpolated (B, Nq, C))."""
         idx, d2 = self.three_nn(dense_xyz, sparse_xyz)
         inv = 1.0 / torch.clamp(d2, min=1e-10)
         w = inv / inv.sum(dim=2, keepdim=True)
@@ -486,8 +495,7 @@ class FusedPointNet2:
         interp = g[:, :, 0] * w[:, :, 0:1]
         interp = torch.addcmul(interp, g[:, :, 1], w[:, :, 1:2])
         interp = torch.addcmul(interp, g[:, :, 2], w[:, :, 2:3])
-        x = interp if dense_cl is None else torch.cat([interp, dense_cl], dim=-1)
-        return self._mlp(x, layers)
+        return g, interp
 
     # ---------------------------------------------------------------- fused-path helpers
     @staticmethod
@@ -651,19 +659,26 @@ class FusedPointNet2:
                     w.record_stream(main)
                 else:
                     idx3, w = self.three_nn_weights(dense_xyz, sparse_xyz)
-            if self.fp_pre[i] is not None:
-                with _sec(timer, "fp%d.mlp" % i):
-                    pre = self.fp_pre[i].run_rows(sparse)  # first conv + shift on the sparse rows, no ReLU
-                with _sec(timer, "fp%d.interp_concat" % i):
-                    x = self.interp_concat(pre, idx3, w, None, B, sparse_xyz.shape[2], dense_xyz.shape[2], relu=True)
-            else:
-                with _sec(timer, "fp%d.interp_concat" % i):
-                    x = self.interp_concat(sparse, idx3, w, dense, B, sparse_xyz.shape[2], dense_xyz.shape[2])
-            with _sec(timer, "fp%d.mlp" % i):
-                for ch in chains:
-                    x = ch.run_rows(x)
-            sparse_xyz, sparse = dense_xyz, x
+            sparse = self._fp_level(i, sparse, dense, dense_xyz, idx3, w, sparse_xyz.shape[2], timer)
+            sparse_xyz = dense_xyz
         return lv_xyz[0], sparse, lv_feat
+
+    def _fp_level(self, i, sparse, dense, dense_xyz, idx3, w, Nk, timer):
+        """Interpolating propagation level i on the tcgen05 trunk: sparse bf16 [B*Nk, C2], skip bf16 [B*Nq, C1] (or None),
+        the dense cloud (B,3,Nq), the 3-NN indices / weights -> bf16 [B*Nq, C']."""
+        B, Nq = dense_xyz.shape[0], dense_xyz.shape[2]
+        if self.fp_pre[i] is not None:
+            with _sec(timer, "fp%d.mlp" % i):
+                pre = self.fp_pre[i].run_rows(sparse)  # first conv + shift on the sparse rows, no ReLU
+            with _sec(timer, "fp%d.interp_concat" % i):
+                x = self.interp_concat(pre, idx3, w, None, B, Nk, Nq, relu=True)
+        else:
+            with _sec(timer, "fp%d.interp_concat" % i):
+                x = self.interp_concat(sparse, idx3, w, dense, B, Nk, Nq)
+        with _sec(timer, "fp%d.mlp" % i):
+            for ch in self.fp_chains[i]:
+                x = ch.run_rows(x)
+        return x
 
     def _head_stage(self, xyz, sparse, timer=None, host_out=None):
         """PN2_CLS's four per-point heads on the trunk's features -> {score, frame_R, frame_t, movable_logits (after the
@@ -738,9 +753,14 @@ class FusedPointNet2:
                 x = sparse.expand(-1, dense_xyz.shape[2], -1)
                 sparse = self._mlp(x if dense is None else torch.cat([x, dense], dim=-1), layers)
             else:
-                sparse = self._fp_torch(dense_xyz, sparse_xyz, dense, sparse, layers)
+                sparse = self._fp_reference(i, dense_xyz, sparse_xyz, dense, sparse, layers)
             sparse_xyz = dense_xyz
         return lv_xyz[0], sparse, lv_feat
+
+    def _fp_reference(self, i, dense_xyz, sparse_xyz, dense, sparse, layers):
+        """Interpolating propagation level i on the torch / tf32 backends: (B, Nk, C2), skip (B, Nq, C1) or None ->
+        (B, Nq, C')."""
+        return self._fp_torch(dense_xyz, sparse_xyz, dense, sparse, layers)
 
     def _run(self, points, return_trace, timer, head_stage):
         """The trunk on this engine's backend, then ``head_stage(cloud, per-point features)``."""
@@ -916,3 +936,119 @@ class FusedEdgePointNet2Down(FusedPointNet2):
             return super()._sa_reference(i, xyz, feat, new_xyz, nbr, idx, layers)
         ctr_feat = torch.gather(feat, 1, idx.long().unsqueeze(-1).expand(-1, -1, feat.shape[-1]))
         return self._sa_torch(xyz, feat, new_xyz, nbr, layers, ctr_feat=ctr_feat)
+
+
+class FusedEdgePointNet2DownUp(FusedEdgePointNet2Down):
+    """EDGEPN2DU (models/EdgePointNet2DownUp.py): EDGEPN2D's encoder (edge set-abstraction levels, global level), a
+    decoder whose interpolating levels are edge levels (EdgeFPModule), and two heads (scene_score_logits, frame_R; no
+    sigmoid).  An edge propagation level's first layer sees EdgeFeatureInterpolator's rows [interp_q | n_k - interp_q | d_q]
+    for each dense point q and each of its 3 nearest sparse points k (2 C2 + C1 channels), and the level ends with the mean
+    over k.  With the folded weight split by those column groups, W' = [W_i | W_n | W_d], and interp_q = sum_j w_qj S_j,
+        y0[q,k] = sum_j w_qj U[idx_qj] + V[idx_qk] + T_q + b',   U = (W_i - W_n) S,  V = W_n S,  T = W_d d,
+    which needs no assumption on the weights' sum.  So on the tcgen05 trunk an edge propagation level is: one row chain
+    over the sparse rows with the stacked weight [W_i - W_n ; W_n] (zero shift, no ReLU) -> bf16 [U | V]; T by a one-layer
+    row chain (W_d, zero shift, no ReLU) over the skip rows, or, at the finest level, whose skip is the cloud itself, in
+    fp32 inside the row kernel; ``edge_interp_rows`` -> relu(y0) bf16 [B*Nq*3, cout0]; the row chains of the later layers
+    over those rows; ``rows_group_mean`` -> [B*Nq, C'].  The (B, 2 C2 + C1, Nq, 3) edge tensor never exists.  The torch /
+    tf32 backends build the edge rows literally with the unsplit weights and take the mean: an independent check of the
+    split.  The broadcast level (num_fp_neighbours = 0) is the sibling's."""
+
+    _HEAD_SIGMOID = (False, False)
+
+    def __init__(self, model, *args, **kwargs):
+        from .network_models.models.pointnet2_utils.modules import EdgeFPModule
+        # per propagation level: an edge level (EdgeFPModule that interpolates)
+        self.edge_fp = [isinstance(m, EdgeFPModule) and m.interpolator is not None for m in model.fp_modules]
+        self._edge_fp = {}  # edge propagation level -> ([U | V] chain, T chain or None, shift b', W_d of the cloud or None)
+        super().__init__(model, *args, **kwargs)
+
+    @staticmethod
+    def _head_modules(model):
+        return ((model.mlp_seg, model.seg_logit), (model.mlp_frame, model.frame_logit))
+
+    @staticmethod
+    def split_edge_fp_layer(w, c2):
+        """Folded first-layer weight of an edge propagation level, [cout, 2 c2 + c1] with columns [interpolated |
+        neighbour - interpolated | skip] -> ([W_i - W_n ; W_n] [2 cout, c2], W_d [cout, c1]), in the input's precision
+        (split before any bf16 cast)."""
+        assert w.dim() == 2 and w.shape[1] > 2 * c2, "edge propagation layer expects 2 x %d + skip input channels" % c2
+        wi, wn, wd = w[:, :c2], w[:, c2:2 * c2], w[:, 2 * c2:]
+        return torch.cat([wi - wn, wn], dim=0).contiguous(), wd.contiguous()
+
+    def _fp_chain(self, i, layers, skip_c):
+        if not self.edge_fp[i]:
+            return super()._fp_chain(i, layers, skip_c)
+        (w0, b0), rest = layers[0], layers[1:]
+        c1 = skip_c or 3  # no skip feature below the finest level: there it is the cloud (EdgePointNet2DownUp.forward)
+        w_uv, w_d = self.split_edge_fp_layer(w0, (w0.shape[1] - c1) // 2)
+        cout = w0.shape[0]
+        uv = self._make_chain([(w_uv, b0.new_zeros(2 * cout), False)], IN_ROWS, 0, OUT_ROWS)
+        if skip_c:
+            term, w_xyz = self._make_chain([(w_d, b0.new_zeros(cout), False)], IN_ROWS, 0, OUT_ROWS), None
+        else:
+            term, w_xyz = None, w_d.to(self.device)
+        self._edge_fp[i] = (uv, term, b0.to(self.device).contiguous(), w_xyz)
+        return None, self._row_chains(rest) if rest else []
+
+    @staticmethod
+    def edge_interp_rows(uv, idx, w, t_rows, xyz, w_xyz, shift, B, Nk, Nq):
+        """uv bf16 [B*Nk, 2C] rows [U | V]; 3-NN int32 idx / fp32 w (B,Nq,3); skip: t_rows bf16 [B*Nq, C] or the cloud
+        xyz (B,3,Nq) fp32 with w_xyz fp32 [C, 3]; shift fp32 [C] -> bf16 [B*Nq*3, C], relu of the first layer per (q, k)."""
+        C = shift.shape[0]
+        out = torch.empty((B * Nq * 3, C), dtype=torch.bfloat16, device=uv.device)
+        check(lib.s4g_edge_interp_rows_bf16(ptr(uv), ptr(idx), ptr(w), ptr(t_rows) if t_rows is not None else None,
+                                            ptr(xyz) if xyz is not None else None,
+                                            ptr(w_xyz) if w_xyz is not None else None, ptr(shift), B, Nk, Nq, C, ptr(out),
+                                            stream_ptr(uv.device)), "edge_interp_rows")
+        return out
+
+    @staticmethod
+    def rows_group_mean(rows):
+        """bf16 [3R, C] -> [R, C]: the mean of each 3 consecutive rows, ((r0 + r1) + r2) / 3 in fp32, rounded once."""
+        R, C = rows.shape[0] // 3, rows.shape[1]
+        out = torch.empty((R, C), dtype=torch.bfloat16, device=rows.device)
+        check(lib.s4g_rows_group_mean_bf16(ptr(rows), R, C, ptr(out), stream_ptr(rows.device)), "rows_group_mean")
+        return out
+
+    def _fp_level(self, i, sparse, dense, dense_xyz, idx3, w, Nk, timer):
+        if not self.edge_fp[i]:
+            return super()._fp_level(i, sparse, dense, dense_xyz, idx3, w, Nk, timer)
+        uv_chain, term_chain, shift, w_xyz = self._edge_fp[i]
+        B, Nq = dense_xyz.shape[0], dense_xyz.shape[2]
+        with _sec(timer, "fp%d.uv" % i):
+            uv = uv_chain.run_rows(sparse)
+        t_rows = None
+        if term_chain is not None:
+            with _sec(timer, "fp%d.term" % i):
+                t_rows = term_chain.run_rows(dense)
+        with _sec(timer, "fp%d.edge_rows" % i):
+            x = self.edge_interp_rows(uv, idx3, w, t_rows, dense_xyz if t_rows is None else None, w_xyz, shift, B, Nk, Nq)
+        with _sec(timer, "fp%d.mlp" % i):
+            for ch in self.fp_chains[i]:
+                x = ch.run_rows(x)
+        with _sec(timer, "fp%d.mean" % i):
+            return self.rows_group_mean(x)
+
+    def _fp_reference(self, i, dense_xyz, sparse_xyz, dense, sparse, layers):
+        if not self.edge_fp[i]:
+            return super()._fp_reference(i, dense_xyz, sparse_xyz, dense, sparse, layers)
+        g, interp = self._interp_torch(dense_xyz, sparse_xyz, sparse)  # (B, Nq, 3, C2), (B, Nq, C2)
+        skip = dense if dense is not None else dense_xyz.transpose(1, 2)
+        centre = interp.unsqueeze(2).expand_as(g)
+        x = torch.cat([centre, g - centre, skip.unsqueeze(2).expand(-1, -1, g.shape[2], -1)], dim=-1)
+        return self._mlp(x, layers).mean(dim=2)
+
+    def _downup_head_stage(self, xyz, sparse, timer):
+        """-> {scene_score_logits (B, score_classes, N), frame_R (B, 9, N)} fp32 logits."""
+        n = xyz.shape[2]
+        if self.mlp_backend != "tcgen05":
+            outs = [self._head_reference(sparse, k) for k in range(2)]
+        else:
+            with _sec(timer, "heads.mlp"):
+                outs = [ch.run_rows(sparse, n_points=n) for ch in self.head_chains]
+        return {"scene_score_logits": outs[0], "frame_R": outs[1]}
+
+    @torch.no_grad()
+    def forward(self, points, return_trace=False, timer=None):
+        """points (B,3,N) fp32 CUDA -> {scene_score_logits, frame_R}, as EdgePointNet2DownUp.forward."""
+        return self._run(points, return_trace, timer, lambda xyz, sparse: self._downup_head_stage(xyz, sparse, timer))

@@ -11,6 +11,12 @@ from .pointnet2_utils.modules import EdgeSAModule, PointnetFPModule
 PointNet2Loss, PointNet2Metric = _pn2.PointNet2Loss, _pn2.PointNet2Metric
 
 
+def edge_levels_fusable(c):
+    """Every edge set-abstraction level (sampled, with input features) of the configuration dict ``c`` is at least two
+    layers deep: the centroid term joins the first layer's epilogue, and a one-layer level's first layer is its max-pool."""
+    return all(len(ch) > 1 for i, ch in enumerate(c["sa_channels"]) if i > 0 and c["num_centroids"][i] != 0)
+
+
 class EdgePointNet2Down(_pn2.PointNet2):
     _SA_MODULE = EdgeSAModule
     _FP_MODULE = PointnetFPModule
@@ -20,10 +26,7 @@ class EdgePointNet2Down(_pn2.PointNet2):
         """Whether the fused engine has a plan for this configuration: the PN2 sibling's rules (PointNet2_tcls.PointNet2.
         fusable, ``allow_global`` as there) and every edge level (sampled, with input features) at least two layers deep
         — the centroid term joins the first layer's epilogue, and a one-layer level's first layer is its max-pool."""
-        if not super().fusable(allow_global):
-            return False
-        c = self.config
-        return all(len(ch) > 1 for i, ch in enumerate(c["sa_channels"]) if i > 0 and c["num_centroids"][i] != 0)
+        return super().fusable(allow_global) and edge_levels_fusable(self.config)
 
     def forward(self, data_batch, fused=None):
         """``fused``: None / False = the module path; True = the fused engine, for every configuration

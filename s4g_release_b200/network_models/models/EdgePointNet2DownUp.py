@@ -8,19 +8,26 @@ be instantiated there, and the forward it would inherit reads heads that this co
 the module surface: the same constructor (state_dict keys ``sa_modules.*``, ``fp_modules.*``, ``mlp_seg.*``,
 ``seg_logit.*``, ``mlp_frame.*``, ``frame_logit.*``), and a forward for the two heads it has — OUR definition, since the
 reference has no runnable one: the coordinates are the finest level's skip feature; returns ``scene_score_logits``
-(B, score_classes, N) and ``frame_R`` (B, 9, N)."""
+(B, score_classes, N) and ``frame_R`` (B, 9, N).
+
+The fused engine (engine.FusedEdgePointNet2DownUp) is opt-in, ``forward(..., fused=True)``: EDGEPN2D's encoder, and
+edge propagation levels whose first layer is split into a sparse-row part and a per-point part, so the edge rows are
+never built.  Otherwise the model runs on the module path (sm_100a operators + torch autograd), as does its training."""
 import torch.nn as nn
 
 from ..nn_utils.mlp import SharedMLP
 from . import PointNet2 as _pn2
+from .EdgePointNet2Down import edge_levels_fusable
+from .PointNet2_tcls import FusedEngineCache, _widths_ok, trunk_fusable
 from .pointnet2_utils.modules import EdgeFPModule, EdgeSAModule
 
 PointNet2Loss, PointNet2Metric = _pn2.PointNet2Loss, _pn2.PointNet2Metric
 
 
-class EdgePointNet2DownUp(nn.Module):
+class EdgePointNet2DownUp(FusedEngineCache, nn.Module):
     _SA_MODULE = EdgeSAModule
     _FP_MODULE = EdgeFPModule
+    _ENGINE = "FusedEdgePointNet2DownUp"
 
     def __init__(self,
                  score_classes,
@@ -36,6 +43,10 @@ class EdgePointNet2DownUp(nn.Module):
         n_sa, n_fp = len(num_centroids), len(fp_channels)
         assert len(radius) == n_sa and len(num_neighbours) == n_sa and len(sa_channels) == n_sa
         assert n_sa == n_fp and len(num_fp_neighbours) == n_fp
+        self.config = dict(score_classes=score_classes, num_centroids=tuple(num_centroids), radius=tuple(radius),
+                           num_neighbours=tuple(num_neighbours), sa_channels=tuple(map(tuple, sa_channels)),
+                           fp_channels=tuple(map(tuple, fp_channels)), num_fp_neighbours=tuple(num_fp_neighbours),
+                           seg_channels=tuple(seg_channels), dropout_prob=dropout_prob)
         self.sa_modules = nn.ModuleList()
         c = 0
         for i in range(n_sa):
@@ -55,9 +66,33 @@ class EdgePointNet2DownUp(nn.Module):
         self.seg_logit = nn.Conv1d(seg_channels[-1], score_classes, 1, bias=True)
         self.mlp_frame = SharedMLP(c, seg_channels, ndim=1)
         self.frame_logit = nn.Conv1d(seg_channels[-1], 9, 1, bias=True)
+        self._engine = None
+        self._engine_key = None
 
-    def forward(self, data_batch):
+    def fusable(self, allow_global=False):
+        """Whether the fused engine has a plan for this configuration: the trunk rules of ``trunk_fusable``
+        (``allow_global`` as there), EDGEPN2D's rule for edge set-abstraction levels (``edge_levels_fusable``), an edge
+        propagation level's first layer at most 512 wide (its stacked [U | V] pre-activations, 2 x that width, are one row
+        chain's output), and head widths that are multiples of 16, <= 512, with at most 16 score classes."""
+        c = self.config
+        if not (trunk_fusable(c, allow_global) and edge_levels_fusable(c)):
+            return False
+        if any(ch[0] > 512 for ch, k in zip(c["fp_channels"], c["num_fp_neighbours"]) if k != 0):
+            return False
+        return _widths_ok(c["seg_channels"]) and max(c["seg_channels"]) <= 512 and c["score_classes"] <= 16
+
+    def forward(self, data_batch, fused=None):
+        """``fused``: None / False = the module path; True = the fused engine, for every configuration
+        ``fusable(allow_global=True)`` accepts (others raise RuntimeError before any GPU work)."""
         points = data_batch["scene_points"]
+        if not fused:
+            return self.forward_modules(points)
+        if not self.fusable(allow_global=True):
+            raise RuntimeError("the fused engine has no plan for this configuration (see EdgePointNet2DownUp.fusable); "
+                               "call with fused=False for the module path")
+        return self.fused_engine().forward(points)
+
+    def forward_modules(self, points):
         xyz, feature = points, None
         level_xyz, level_feature = [xyz], [points]
         for sa in self.sa_modules:
